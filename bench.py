@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c1|c3|c4|c5|c5l4]
                     [--no-others] [--no-sustained] [--no-e2e] [--no-cpu-baseline] [--ess-iters I]
+                    [--dump-outputs DIR]
 
 Headline workload at every N: BASELINE config 2 -- 100-D correlated Gaussian (dense precision
 Lambda = A A^T / D + I), ensemble of 2^20 particles, L = 50 leapfrog steps per HMC iteration, float32 state,
@@ -22,6 +23,10 @@ cpu_baseline     : the NumPy float64 oracle port on the host cores (bounded samp
 cpu_baseline_ref : the UNMODIFIED reference under the jax.numpy stand-in at config 1 (and at configs 2 and 5 with a
             reduced ensemble), timed in the build container (it is Python and cannot travel to the GPU box;
             profiles/r02_ref_standin_c1.json, r02_ref_standin_reduced.json).
+
+--dump-outputs DIR writes what the headline leg's last timed step handed its caller to DIR/<name>.npy (see
+dump_outputs).  Every input is generated from fixed seeds, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -423,6 +428,39 @@ def fused_get_samples(E, leg, dev):
             "one launch, samples and momenta (D, P, S) written by the kernel"}
 
 
+DUMP_Q_BYTES = 32 << 20
+
+
+def dump_outputs(leg, out_dir, group):
+    """Writes what the leg's last timed call handed its caller to out_dir/<name>.npy (rank 0 writes):
+      q.npy  the positions HMC.step / HMC.run updated in place, float32 (D, n): the columns of a fixed, seeded sample of
+             n particles in ascending particle order, n the whole ensemble or as many as fit DUMP_Q_BYTES (the full
+             config-2 ensemble is 400 MB);
+      acceptRate, meanAcceptProb, meanH, stepSize, numSteps (one value per iteration), mean, var (D): what HMC.run
+             returned, float64 -- the adaptive legs (config 5) only."""
+    import torch
+    import torch.distributed as dist
+
+    q_all = leg.ens.q
+    n = min(leg.P, DUMP_Q_BYTES // (leg.D * q_all.element_size()))
+    cols = np.sort(np.random.RandomState(SEED).choice(leg.P, n, replace=False))
+    mine = cols[(cols >= leg.p_lo) & (cols < leg.p_lo + leg.Pl)] - leg.p_lo
+    q = q_all[:, torch.from_numpy(mine).to(q_all.device)].cpu().numpy()
+    if leg.world > 1:
+        parts = [None] * leg.world
+        dist.all_gather_object(parts, q, group=group)
+        q = np.concatenate(parts, axis=1)
+    if leg.rank != 0:
+        return
+    out = {"q": q}
+    if leg.run_out is not None:
+        for k in ("acceptRate", "meanAcceptProb", "meanH", "stepSize", "numSteps", "mean", "var"):
+            out[k] = np.asarray(leg.run_out[k], dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -437,7 +475,13 @@ def main():
     ap.add_argument("--no-sustained", action="store_true")
     ap.add_argument("--sustained-iters", type=int, default=0, help="0 = enough iterations for ~2.2 s (>= 700)")
     ap.add_argument("--ess-iters", type=int, default=150, help="iterations of the ESS/s phase (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline leg computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = CONFIGS[args.config]
 
@@ -489,6 +533,8 @@ def main():
     main_t = leg.timed(args.steps, args.warmup, group, barrier, ctx)
     value, ms_per_step = main_t["value"], main_t["ms_per_step"]
     main_adapt = leg.run_out
+    if args.dump_outputs:
+        dump_outputs(leg, args.dump_outputs, group)
     if os.environ.get("EHMC_ENS_DEBUG") and rank == 0:
         ctx.set_option("ens_debug_dump", max(0.0, float(os.environ["EHMC_ENS_DEBUG"]) - 24))
 

@@ -9,6 +9,7 @@ from __future__ import annotations
 
 import glob
 import os
+import shutil
 import subprocess
 import sys
 
@@ -21,6 +22,19 @@ NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC,-fvisibility=hidden", "-cudart", "static",
 ]
+
+
+def cuda_tool(name):
+    """Path of a CUDA toolkit program: on PATH, else under $CUDA_HOME (or $CUDA_PATH, or /usr/local/cuda)/bin,
+    which is where the toolkit lives when a login shell does not put it on PATH."""
+    found = shutil.which(name)
+    if found:
+        return found
+    home = os.environ.get("CUDA_HOME") or os.environ.get("CUDA_PATH") or "/usr/local/cuda"
+    path = os.path.join(home, "bin", name)
+    if not os.path.isfile(path):
+        raise FileNotFoundError(f"{name} is neither on PATH nor in {os.path.dirname(path)}: set CUDA_HOME")
+    return path
 
 
 def _sources():
@@ -50,7 +64,7 @@ def _newer(target, sources):
 
 def build_library(force=False, verbose=False):
     """Compile the .cu files under csrc/ that changed (parallel per file) and link one shared library."""
-    nvcc = os.environ.get("NVCC", "nvcc")
+    nvcc = os.environ.get("NVCC") or cuda_tool("nvcc")
     objdir = os.path.join(HERE, "build")
     os.makedirs(objdir, exist_ok=True)
     procs = []

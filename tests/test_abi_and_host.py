@@ -5,12 +5,14 @@ import ctypes
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
 import pytest
 
 import physicsbasedbayesianinference_b200 as E
 from physicsbasedbayesianinference_b200 import _lib
+from physicsbasedbayesianinference_b200.build import cuda_tool
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -43,7 +45,7 @@ def test_version_and_struct_layout():
 
 
 def test_library_contains_sm100a_sass_only():
-    out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    out = subprocess.run([cuda_tool("cuobjdump"), "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
     assert not re.search(r"sm_(?!100a)\d+", out)
 
@@ -142,12 +144,12 @@ def test_nbody_mode_constructor_prints_like_reference(capsys):
     assert integ.nBodyMode and integ.numSteps == 6
 
 
-def test_flat_module_shims():
+def test_flat_module_shims(tmp_path):
     code = ("import sys; sys.path.insert(0, %r); from ensemble import Ensemble; from integrator import Leapfrog, "
             "StormerVerlet; from HMC import HMC; from potential import harmonicPotentialND, noPotential; "
             "print(Ensemble(2, 3).q.shape, noPotential(0))") % os.path.join(
                 ROOT, "physicsbasedbayesianinference_b200", "flat")
-    out = subprocess.run(["python", "-c", code], capture_output=True, text=True, cwd="/tmp")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path)
     assert out.returncode == 0, out.stderr
     assert "(2, 3) 0" in out.stdout
 

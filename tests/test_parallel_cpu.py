@@ -1,6 +1,7 @@
 """CPU tests of the multi-rank host logic (gloo, world_size 2): particle sharding, the
 statistics all-reduce and the rank-identical step-size adaptation."""
 import os
+import socket
 
 import numpy as np
 import pytest
@@ -22,7 +23,7 @@ def test_shard_ranges_cover_exactly():
             assert max(sizes) - min(sizes) <= 1
 
 
-def _worker(rank, world, port, D, P, q):
+def _worker(rank, world, port, D, P, q, out_dir):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -44,17 +45,20 @@ def _worker(rank, world, port, D, P, q):
     hs = [ad.update(u["meanAcceptProb"]) for _ in range(3)]
     scales = torch.from_numpy(parallel.MassAdapter(D).scales(u["mean"].numpy(), u["var"].numpy(), P))
     torch.save(dict(stats=stats, hs=hs, mean=u["mean"], var=u["var"], acc=u["acceptRate"], scales=scales),
-               f"/tmp/ehmc_par_{port}_{rank}.pt")
+               os.path.join(out_dir, f"rank{rank}.pt"))
     dist.destroy_process_group()
 
 
-def test_stats_allreduce_and_adaptation_gloo_world2():
+def test_stats_allreduce_and_adaptation_gloo_world2(tmp_path):
     D, P, world = 5, 1001, 2
     rng = np.random.RandomState(0)
     q = rng.standard_normal((D, P))
-    port = 29500 + (os.getpid() % 2000)
-    mp.spawn(_worker, args=(world, port, D, P, q), nprocs=world, join=True)
-    r = [torch.load(f"/tmp/ehmc_par_{port}_{k}.pt") for k in range(world)]
+    sock = socket.socket()  # a port no other process on the machine holds
+    sock.bind(("127.0.0.1", 0))
+    port = sock.getsockname()[1]
+    sock.close()
+    mp.spawn(_worker, args=(world, port, D, P, q, str(tmp_path)), nprocs=world, join=True)
+    r = [torch.load(str(tmp_path / f"rank{k}.pt")) for k in range(world)]
     assert torch.equal(r[0]["stats"], r[1]["stats"])  # same sums on every rank
     assert r[0]["hs"] == r[1]["hs"]  # identical step sizes without a broadcast
     np.testing.assert_allclose(r[0]["mean"].numpy(), q.mean(1), rtol=1e-12, atol=1e-12)
