@@ -1,6 +1,6 @@
-// C-ABI of the ehmc engine (include/ehmc.h): argument validation, potential
-// packing, kernel dispatch, host-buffer staging.  No torch types, no exceptions.
-#include <cuda_fp16.h>
+// C-ABI of the ehmc engine (include/ehmc.h): argument validation, kernel dispatch, host-buffer staging.  The device
+// state of each potential family is built beside that family's launchers (build_* / pack_* in inst_*).  No torch
+// types, no exceptions.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -349,26 +349,16 @@ static int fetch_param(const DLTensor* t, const char* name, int ndim, std::vecto
   return EHMC_OK;
 }
 
-template <typename T>
-static int upload(const std::vector<double>& h, void** dptr) {
-  std::vector<T> t(h.size());
-  for (size_t i = 0; i < h.size(); ++i) t[i] = (T)h[i];
+int ehmc::upload_raw(const void* src, size_t bytes, void** dptr) {
   *dptr = nullptr;
-  if (h.empty()) return EHMC_OK;
-  CUDA_TRY(cudaMalloc(dptr, sizeof(T) * t.size()));
-  CUDA_TRY(cudaMemcpy(*dptr, t.data(), sizeof(T) * t.size(), cudaMemcpyHostToDevice));
-  return EHMC_OK;
-}
-
-static int upload_raw(const void* src, size_t bytes, void** dptr) {
-  *dptr = nullptr;
-  CUDA_TRY(cudaMalloc(dptr, bytes));
+  if (bytes == 0) return EHMC_OK;
+  if (cudaMalloc(dptr, bytes) != cudaSuccess) {
+    cudaGetLastError();
+    *dptr = nullptr;
+    return fail(EHMC_ERR_NOMEM, "cudaMalloc(%zu) failed", bytes);
+  }
   CUDA_TRY(cudaMemcpy(*dptr, src, bytes, cudaMemcpyHostToDevice));
   return EHMC_OK;
-}
-
-static int upload_bits(int bits, const std::vector<double>& h, void** dptr) {
-  return bits == 32 ? upload<float>(h, dptr) : upload<double>(h, dptr);
 }
 
 extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* const* params, int nparams,
@@ -385,39 +375,43 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
   p->family = family;
   p->bits = dtype_bits;
   p->scalars.assign(scalars, scalars + nscalars);
+  const bool f32 = dtype_bits == 32;
   int rc = EHMC_OK;
   View v;
+  std::vector<double> a, b;  // the float64 host copies of params[0], params[1]
   switch (family) {
     case EHMC_FAMILY_DIAG_GAUSSIAN: {
       if (nparams != 1) { rc = fail(EHMC_ERR_INVALID, "diag gaussian: params = {k[D]}"); break; }
-      rc = fetch_param(params[0], "k", 1, &p->hp0, &v);
+      rc = fetch_param(params[0], "k", 1, &a, &v);
       if (rc) break;
-      p->D = (int)p->hp0.size();
+      p->D = (int)a.size();
       if (p->D < 1) { rc = fail(EHMC_ERR_INVALID, "diag gaussian: empty k"); break; }
       if (p->D > 32 && p->D <= 128) {
         // route through the dense kernel with Lambda = diag(k)
         std::vector<double> lam((size_t)p->D * p->D, 0.0);
-        for (int d = 0; d < p->D; ++d) lam[(size_t)d * p->D + d] = p->hp0[d];
-        p->hp0.swap(lam);
-        p->hp1.assign(p->D, 0.0);
+        for (int d = 0; d < p->D; ++d) lam[(size_t)d * p->D + d] = a[d];
+        a.swap(lam);
+        b.assign(p->D, 0.0);
         p->family = EHMC_FAMILY_DENSE_GAUSSIAN;
       } else if (p->D > 128) {
         rc = fail(EHMC_ERR_UNSUPPORTED, "diag gaussian: D = %d > 128 not built", p->D);
+      } else {
+        p->diag_k.swap(a);
       }
       break;
     }
     case EHMC_FAMILY_DENSE_GAUSSIAN: {
       if (nparams < 1 || nparams > 2) { rc = fail(EHMC_ERR_INVALID, "dense gaussian: params = {Lambda[D,D], mu[D]?}"); break; }
-      rc = fetch_param(params[0], "Lambda", 2, &p->hp0, &v);
+      rc = fetch_param(params[0], "Lambda", 2, &a, &v);
       if (rc) break;
       if (v.shape[0] != v.shape[1] || v.shape[0] < 1) { rc = fail(EHMC_ERR_INVALID, "Lambda must be square"); break; }
       p->D = (int)v.shape[0];
       if (nparams == 2 && params[1] != nullptr) {
-        rc = fetch_param(params[1], "mu", 1, &p->hp1, &v);
+        rc = fetch_param(params[1], "mu", 1, &b, &v);
         if (rc) break;
-        if ((int)p->hp1.size() != p->D) { rc = fail(EHMC_ERR_INVALID, "mu must have D entries"); break; }
+        if ((int)b.size() != p->D) { rc = fail(EHMC_ERR_INVALID, "mu must have D entries"); break; }
       } else {
-        p->hp1.assign(p->D, 0.0);
+        b.assign(p->D, 0.0);
       }
       if (p->D > 128) rc = fail(EHMC_ERR_UNSUPPORTED, "dense gaussian: D = %d > 128 not built", p->D);
       break;
@@ -432,205 +426,51 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
     }
     case EHMC_FAMILY_COIN_TOSS: {
       if (nparams != 2) { rc = fail(EHMC_ERR_INVALID, "coin toss: params = {successes[D], trials[D]}"); break; }
-      rc = fetch_param(params[0], "successes", 1, &p->hp0, &v);
+      rc = fetch_param(params[0], "successes", 1, &p->coin_k, &v);
       if (rc) break;
-      rc = fetch_param(params[1], "trials", 1, &p->hp1, &v);
+      rc = fetch_param(params[1], "trials", 1, &p->coin_n, &v);
       if (rc) break;
-      p->D = (int)p->hp0.size();
+      p->D = (int)p->coin_k.size();
       if (p->D < 1 || p->D > 32) { rc = fail(EHMC_ERR_UNSUPPORTED, "coin toss: 1 <= D <= 32 (got %d)", p->D); break; }
-      if ((int)p->hp1.size() != p->D) { rc = fail(EHMC_ERR_INVALID, "coin toss: trials must have D entries"); break; }
+      if ((int)p->coin_n.size() != p->D) { rc = fail(EHMC_ERR_INVALID, "coin toss: trials must have D entries"); break; }
       for (int d = 0; d < p->D && rc == EHMC_OK; ++d)
-        if (!(p->hp0[d] >= 0 && p->hp1[d] >= p->hp0[d])) rc = fail(EHMC_ERR_INVALID, "coin toss: need 0 <= successes <= trials");
+        if (!(p->coin_k[d] >= 0 && p->coin_n[d] >= p->coin_k[d])) rc = fail(EHMC_ERR_INVALID, "coin toss: need 0 <= successes <= trials");
       break;
     }
     case EHMC_FAMILY_NBODY: {
       if (nparams != 1 || nscalars != 2) { rc = fail(EHMC_ERR_INVALID, "nbody: params = {bodyMass[B]}, scalars = {G, eps}"); break; }
-      rc = fetch_param(params[0], "bodyMass", 1, &p->hp0, &v);
+      rc = fetch_param(params[0], "bodyMass", 1, &a, &v);
       if (rc) break;
-      p->B = (int)p->hp0.size();
-      p->D = 3 * p->B;
-      if (p->B < 1) { rc = fail(EHMC_ERR_INVALID, "nbody: empty bodyMass"); break; }
-      if (p->B > 7000) { rc = fail(EHMC_ERR_UNSUPPORTED, "nbody: B = %d > 7000 bodies", p->B); break; }
+      const int B = (int)a.size();
+      p->D = 3 * B;
+      if (B < 1) { rc = fail(EHMC_ERR_INVALID, "nbody: empty bodyMass"); break; }
+      if (B > 7000) { rc = fail(EHMC_ERR_UNSUPPORTED, "nbody: B = %d > 7000 bodies", B); break; }
       if (!(scalars[1] >= 0)) { rc = fail(EHMC_ERR_INVALID, "nbody: eps must be >= 0"); break; }
-      rc = upload_bits(p->bits, p->hp0, &p->d0);
+      rc = f32 ? build_nbody<float>(p, a) : build_nbody<double>(p, a);
       break;
     }
     case EHMC_FAMILY_LOGISTIC: {
       if (nparams != 2 || nscalars < 1 || nscalars > 2) { rc = fail(EHMC_ERR_INVALID, "logistic: params = {X[N,D], y[N]}, scalars = {priorScale, precision?}"); break; }
-      rc = fetch_param(params[0], "X", 2, &p->hp0, &v);
+      rc = fetch_param(params[0], "X", 2, &a, &v);
       if (rc) break;
-      p->N = (int)v.shape[0];
+      p->logistic.n = (int)v.shape[0];
       p->D = (int)v.shape[1];
-      rc = fetch_param(params[1], "y", 1, &p->hp1, &v);
+      rc = fetch_param(params[1], "y", 1, &b, &v);
       if (rc) break;
-      if ((int)p->hp1.size() != p->N) { rc = fail(EHMC_ERR_INVALID, "logistic: y must have N entries"); break; }
+      if ((int)b.size() != p->logistic.n) { rc = fail(EHMC_ERR_INVALID, "logistic: y must have N entries"); break; }
       if (p->D < 1 || p->D > 256) { rc = fail(EHMC_ERR_UNSUPPORTED, "logistic: 1 <= D <= 256 (got %d)", p->D); break; }
       if (!(scalars[0] > 0)) { rc = fail(EHMC_ERR_INVALID, "logistic: priorScale must be > 0"); break; }
-      rc = upload_bits(p->bits, p->hp0, &p->d0);
-      if (rc == EHMC_OK) rc = upload_bits(p->bits, p->hp1, &p->d1);
-      p->use_tc = nscalars == 2 ? (int)scalars[1] : 0;
-      if (p->use_tc < 0 || p->use_tc > 3) { rc = fail(EHMC_ERR_INVALID, "logistic: precision selector must be 0 (CUDA cores), 1 (bf16), 2 (fp16 split) or 3 (auto)"); break; }
-      if (p->use_tc == 3 && p->bits != 32) p->use_tc = 0;  // auto: float64 state runs the exact kernel
-      if (rc == EHMC_OK && p->use_tc >= 2) {
-        // float32-accurate tensor-core path (k_logistic_tcs): X * 2^a as fp16 (hi, lo) pairs, half-chunk ring entries
-        // [DP/8][64][8] fp16 + 64 floats (2^10 y in the hi entry).  Guard (auto only): one power-of-two scale serves
-        // the whole matrix, so a column whose entries sit more than ~2^10 below max |X| has its lo parts in fp16's
-        // subnormal range; if any column's worst split error exceeds 2^-20 of the column's own max, auto selects the
-        // exact CUDA-core kernel instead.
-        if (p->bits != 32) { rc = fail(EHMC_ERR_INVALID, "logistic: the tensor-core path needs float32 state"); break; }
-        const int D = p->D, N = p->N, DP = (D + 15) / 16 * 16, NB = 64, NC = (N + NB - 1) / NB;
-        double amax = 0.0;
-        for (size_t i = 0; i < (size_t)N * D; ++i) amax = std::max(amax, std::fabs((double)(float)p->hp0[i]));
-        int ex = 0;
-        if (amax > 0 && std::isfinite(amax)) std::frexp(amax, &ex);  // amax = f * 2^ex, f in [0.5, 1)
-        const int sh = std::max(-100, std::min(100, 8 - ex));
-        const double xscale = std::ldexp(1.0, sh);
-        const size_t eb = (size_t)DP * NB * 2 + NB * 4;
-        std::vector<unsigned char> buf(eb * 2 * NC, 0);
-        std::vector<double> colmax(D, 0.0), colerr(D, 0.0);
-        for (int c = 0; c < NC; ++c) {
-          // ring order: entry 2c = Xl, entry 2c + 1 = Xh followed by 2^10 y (the small products run first)
-          __half* xl = reinterpret_cast<__half*>(buf.data() + eb * (2 * c));
-          __half* xh = reinterpret_cast<__half*>(buf.data() + eb * (2 * c + 1));
-          float* ky = reinterpret_cast<float*>(buf.data() + eb * (2 * c + 1) + (size_t)DP * NB * 2);
-          for (int r = 0; r < NB; ++r) {
-            const int n = c * NB + r;
-            ky[r] = 1024.f * (n < N ? (float)p->hp1[n] : 0.5f);
-            if (n >= N) continue;
-            for (int d = 0; d < D; ++d) {
-              const float x = (float)((double)(float)p->hp0[(size_t)n * D + d] * xscale);
-              const __half hi = __float2half_rn(x);
-              const __half lo = __float2half_rn(x - __half2float(hi));
-              const size_t o = ((size_t)(d / 8) * NB + r) * 8 + (d % 8);
-              xh[o] = hi;
-              xl[o] = lo;
-              colmax[d] = std::max(colmax[d], (double)std::fabs(x));
-              colerr[d] = std::max(colerr[d], std::fabs((double)x - (double)__half2float(hi) - (double)__half2float(lo)));
-            }
-          }
-        }
-        bool ok = std::isfinite(amax);
-        for (int d = 0; d < D && ok; ++d) ok = colerr[d] <= colmax[d] * 9.5367431640625e-7;  // 2^-20
-        if (p->use_tc == 3 && !ok) {
-          p->use_tc = 0;
-        } else {
-          p->use_tc = 2;
-          if (cudaMalloc(&p->d6, buf.size()) != cudaSuccess) { rc = fail(EHMC_ERR_NOMEM, "cudaMalloc(%zu) failed", buf.size()); break; }
-          if (cudaMemcpy(p->d6, buf.data(), buf.size(), cudaMemcpyHostToDevice) != cudaSuccess) { rc = fail(EHMC_ERR_CUDA, "upload of the packed X failed"); break; }
-          p->lt_nc = NC;
-          p->lt_dp = DP;
-          p->lt_npad = NC * NB - N;
-          p->lt_chunk_bytes = (unsigned)eb;
-          p->lts_x_iscale = (float)std::ldexp(1.0, -sh);
-        }
-      }
-      if (rc == EHMC_OK && p->use_tc == 1) {
-        if (p->bits != 32) { rc = fail(EHMC_ERR_INVALID, "logistic: the tensor-core path needs float32 state"); break; }
-        // bf16 chunks of 64 data rows in the canonical UMMA layout [DP/8][64][8] + y[64] (float); LT_NB
-        const int D = p->D, N = p->N, DP = (D + 15) / 16 * 16, NB = 64, NC = (N + NB - 1) / NB;
-        const size_t cb = (size_t)DP * NB * 2 + NB * 4 + NB * 2;  // X | y float | (1/2 - y) half
-        std::vector<unsigned char> buf(cb * NC, 0);
-        auto bf16 = [](float f) -> uint16_t {
-          uint32_t b;
-          memcpy(&b, &f, 4);
-          b += 0x7FFFu + ((b >> 16) & 1u);  // round to nearest even
-          return (uint16_t)(b >> 16);
-        };
-        for (int c = 0; c < NC; ++c) {
-          uint16_t* xs = reinterpret_cast<uint16_t*>(buf.data() + cb * c);
-          float* ys = reinterpret_cast<float*>(buf.data() + cb * c + (size_t)DP * NB * 2);
-          __half* cs = reinterpret_cast<__half*>(buf.data() + cb * c + (size_t)DP * NB * 2 + NB * 4);
-          for (int r = 0; r < NB; ++r) {
-            const int n = c * NB + r;
-            ys[r] = n < N ? (float)p->hp1[n] : 0.5f;
-            cs[r] = __float2half_rn(0.5f - ys[r]);
-            if (n >= N) continue;
-            for (int d = 0; d < D; ++d)
-              xs[((size_t)(d / 8) * NB + r) * 8 + (d % 8)] = bf16((float)p->hp0[(size_t)n * D + d]);
-          }
-        }
-        if (cudaMalloc(&p->d6, buf.size()) != cudaSuccess) { rc = fail(EHMC_ERR_NOMEM, "cudaMalloc(%zu) failed", buf.size()); break; }
-        if (cudaMemcpy(p->d6, buf.data(), buf.size(), cudaMemcpyHostToDevice) != cudaSuccess) { rc = fail(EHMC_ERR_CUDA, "upload of the packed X failed"); break; }
-        p->lt_nc = NC;
-        p->lt_dp = DP;
-        p->lt_npad = NC * NB - N;
-        p->lt_chunk_bytes = (unsigned)cb;
-      }
+      const int precision = nscalars == 2 ? (int)scalars[1] : 0;
+      if (precision < 0 || precision > 3) { rc = fail(EHMC_ERR_INVALID, "logistic: precision selector must be 0 (CUDA cores), 1 (bf16), 2 (fp16 split) or 3 (auto)"); break; }
+      if ((precision == 1 || precision == 2) && !f32) { rc = fail(EHMC_ERR_INVALID, "logistic: the tensor-core path needs float32 state"); break; }
+      rc = f32 ? build_logistic<float>(p, a, b, precision) : build_logistic<double>(p, a, b, precision);
       break;
     }
     default:
       rc = fail(EHMC_ERR_UNSUPPORTED, "potential family %d is not built into this library", family);
   }
-  if (rc == EHMC_OK && p->family == EHMC_FAMILY_DENSE_GAUSSIAN) {
-    const int D = p->D;
-    rc = upload_bits(p->bits, p->hp0, &p->d2);
-    if (rc == EHMC_OK && D > 16) {
-      const int TN = dense_tn(D);
-      const int TNP = p->bits == 32 ? dense_tnp<float>(TN) : dense_tnp<double>(TN);
-      p->TN = TN;
-      std::vector<double> Ls((size_t)D * K2_WARPS_HOST * TNP, 0.0), mu((size_t)K2_WARPS_HOST * TN, 0.0);
-      for (int k = 0; k < D; ++k)
-        for (int w = 0; w < K2_WARPS_HOST; ++w)
-          for (int j = 0; j < TN; ++j) {
-            const int i = w * TN + j;
-            if (i < D) Ls[((size_t)k * K2_WARPS_HOST + w) * TNP + j] = p->hp0[(size_t)i * D + k];
-          }
-      for (int d = 0; d < D; ++d) mu[d] = p->hp1[d];
-      rc = upload_bits(p->bits, Ls, &p->d0);
-      if (rc == EHMC_OK) rc = upload_bits(p->bits, mu, &p->d1);
-      if (rc == EHMC_OK && p->bits == 32 && D <= 128) {
-        // 3xFP16 tensor-core operands (k_dense_tc3): Lambda scaled by a power of two so that max |Lambda| lands in
-        // [2^13, 2^14), hi = rn16, lo = rn16(remainder); canonical K-major no-swizzle layout [KP/8][NP][8].
-        const int C8 = (D + 7) / 8, KP = (C8 + 1) / 2 * 16, NP = KP, KCH = KP / 8;
-        double amax = 0.0;
-        for (size_t i = 0; i < (size_t)D * D; ++i) amax = std::max(amax, std::fabs((double)(float)p->hp0[i]));
-        int ex = 0;
-        if (amax > 0 && std::isfinite(amax)) std::frexp(amax, &ex);  // amax = f * 2^ex, f in [0.5, 1)
-        const int sh = std::max(-100, std::min(100, 14 - ex));
-        const double lscale = std::ldexp(1.0, sh);
-        std::vector<__half> bhi((size_t)KCH * NP * 8, __float2half_rn(0.f)), blo(bhi.size(), __float2half_rn(0.f));
-        // Guard of the split (auto path only; dense_path = 4 overrides).  fp16 has 5 exponent bits: entries more
-        // than ~2^27 below max |Lambda| lose bits (hi subnormal, lo flushed).  What that does to the gradient is
-        // measured in the units the target itself sets: x_k ~ Lambda_kk^-1/2 and (grad U)_n ~ Lambda_nn^1/2, so the
-        // relative gradient error of row n is rss_k( dLambda_nk / sqrt(Lambda_nn Lambda_kk) ).  The same argument on
-        // the x side (one power-of-two scale per particle row, 2^7 headroom) bounds the spread of the coordinate
-        // scales: sqrt(max Lambda_kk / min Lambda_kk) <= 2^10.  Otherwise the exact CUDA-core kernel runs.
-        double dmin = INFINITY, dmax = 0.0;
-        for (int d = 0; d < D; ++d) {
-          dmin = std::min(dmin, p->hp0[(size_t)d * D + d]);
-          dmax = std::max(dmax, p->hp0[(size_t)d * D + d]);
-        }
-        bool ok = dmin > 0 && std::isfinite(dmax) && dmax <= dmin * 1048576.0;
-        double worst = 0.0;
-        for (int n = 0; n < D; ++n) {
-          double rss = 0.0;
-          for (int k = 0; k < D; ++k) {
-            const float x = (float)((double)(float)p->hp0[(size_t)n * D + k] * lscale);
-            const __half hi = __float2half_rn(x);
-            const __half lo = __float2half_rn(x - __half2float(hi));
-            const size_t o = ((size_t)(k / 8) * NP + n) * 8 + (k % 8);
-            bhi[o] = hi;
-            blo[o] = lo;
-            if (ok) {
-              const double err = ((double)x - (double)__half2float(hi) - (double)__half2float(lo)) / lscale;
-              rss += err * err / (p->hp0[(size_t)n * D + n] * p->hp0[(size_t)k * D + k]);
-            }
-          }
-          worst = std::max(worst, rss);
-        }
-        p->tc3_ok = (ok && std::sqrt(worst) <= 9.5367431640625e-7) ? 1 : 0;  // 2^-20
-        std::vector<float> mu3(128, 0.f);
-        for (int d = 0; d < D; ++d) mu3[d] = (float)p->hp1[d];
-        rc = upload_raw(bhi.data(), sizeof(__half) * bhi.size(), &p->d7);
-        if (rc == EHMC_OK) rc = upload_raw(blo.data(), sizeof(__half) * blo.size(), &p->d8);
-        if (rc == EHMC_OK) rc = upload_raw(mu3.data(), sizeof(float) * mu3.size(), &p->d9);
-        p->tc3_c8 = C8;
-        p->tc3_inv_lscale = (float)std::ldexp(1.0, -sh);
-      }
-    } else if (rc == EHMC_OK) {
-      rc = upload_bits(p->bits, p->hp1, &p->d1);
-    }
-  }
+  if (rc == EHMC_OK && p->family == EHMC_FAMILY_DENSE_GAUSSIAN)
+    rc = f32 ? build_dense<float>(p, a, b) : build_dense<double>(p, a, b);
   if (rc != EHMC_OK) {
     ehmc_potential_destroy(p);
     return rc;
@@ -643,36 +483,37 @@ extern "C" int ehmc_potential_destroy(ehmc_potential* p) {
   if (!p) return EHMC_OK;
   if (p->ctx) cudaSetDevice(p->ctx->device);
   if (p->ctx && p->ctx->ep_pot == p) p->ctx->ep_valid = false;  // a new potential may reuse this address
-  if (p->d0) cudaFree(p->d0);
-  if (p->d1) cudaFree(p->d1);
-  if (p->d2) cudaFree(p->d2);
-  if (p->d6) cudaFree(p->d6);
-  if (p->d7) cudaFree(p->d7);
-  if (p->d8) cudaFree(p->d8);
-  if (p->d9) cudaFree(p->d9);
+  const DenseState& d = p->dense;
+  for (void* buf : {d.lambda, d.mu, d.ls, d.tc3.hi, d.tc3.lo, d.tc3.mu, p->logistic.x, p->logistic.y,
+                    p->logistic.chunks.buf, p->nbody.body_mass})
+    if (buf) cudaFree(buf);
   delete p;
   return EHMC_OK;
 }
 
-// number of CTAs the trajectory kernel uses for P particles (statistics partials)
+// the float32 dense family runs on the tensor cores unless told otherwise
+static bool use_dense_tc(const ehmc_ctx* c, const ehmc_potential* p) {
+  if (!(p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->bits == 32) || c->dense_path == 1) return false;
+  return p->dense.tc3.c8 >= 3 && (p->dense.tc3.exact || c->dense_path == 4);  // 0 (auto), 4 (forced): 3xFP16 persistent kernel
+}
+
 // families whose trajectory kernel reports statistics per particle ([P][3]) and needs k_colstats
-static bool use_dense_tc(const ehmc_ctx* c, const ehmc_potential* p, int integ);
-static bool per_particle_stats(const ehmc_ctx* c, const ehmc_potential* p, int integ) {
+static bool per_particle_stats(const ehmc_ctx* c, const ehmc_potential* p) {
   if (p->family == EHMC_FAMILY_NBODY || p->family == EHMC_FAMILY_LOGISTIC) return true;
   // the 3xFP16 tensor-core dense kernel reports per-particle scalars too
-  return use_dense_tc(c, p, integ);
+  return use_dense_tc(c, p);
 }
 
-// the float32 dense family runs on the tensor cores unless told otherwise
-static bool use_dense_tc(const ehmc_ctx* c, const ehmc_potential* p, int integ) {
-  if (!(p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->bits == 32) || c->dense_path == 1) return false;
-  (void)integ;
-  return p->tc3_c8 >= 3 && (p->tc3_ok || c->dense_path == 4);  // 0 (auto), 4 (forced): 3xFP16 persistent kernel
+// families with a register-resident kernel (k_small): the only ones the fused multi-iteration runs cover
+static bool small_family(const ehmc_potential* p) {
+  return p->family == EHMC_FAMILY_DIAG_GAUSSIAN || p->family == EHMC_FAMILY_FUNNEL || p->family == EHMC_FAMILY_COIN_TOSS ||
+         (p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->D <= 16);
 }
 
+// number of CTAs the trajectory kernel uses for P particles (statistics partials)
 template <typename T>
-static long long traj_blocks(const ehmc_ctx* c, const ehmc_potential* p, long long P, int integ) {
-  if (per_particle_stats(c, p, integ)) return P;
+static long long traj_blocks(const ehmc_ctx* c, const ehmc_potential* p, long long P) {
+  if (per_particle_stats(c, p)) return P;
   if (p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->D > 16) {
     const int PT = dense_particles_per_cta<T>();
     return (P + PT - 1) / PT;
@@ -685,11 +526,11 @@ static int launch_traj(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& 
                        cudaStream_t st, int slot = 0) {
   c->last_rows = 0;
   if (A.P == 0) return EHMC_OK;
-  c->last_rows = traj_blocks<T>(c, p, A.P, integ);  // upper bound == exact for every kernel but the persistent k_small
+  c->last_rows = traj_blocks<T>(c, p, A.P);  // upper bound == exact for every kernel but the persistent k_small
   if (p->family == EHMC_FAMILY_NBODY) return launch_nbody<T>(c, p, A, integ, hmc, st);
   if (p->family == EHMC_FAMILY_LOGISTIC) return launch_logistic<T>(c, p, A, integ, hmc, st, slot);
   if constexpr (sizeof(T) == 4) {
-    if (use_dense_tc(c, p, integ)) return launch_dense_tc3(c, p, A, integ, hmc, st);
+    if (use_dense_tc(c, p)) return launch_dense_tc3(c, p, A, integ, hmc, st);
   }
   if (c->dense_path == 4 && p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->D > 16 && sizeof(T) == 4)
     return fail(EHMC_ERR_UNSUPPORTED, "dense_path = 4 (tensor cores) but this call is not eligible (D = %d, integrator %d)", p->D, integ);
@@ -738,11 +579,48 @@ static IterArgs<T> base_args(const CallViews& v, double h, double h2, int L) {
   return A;
 }
 
+// the IterArgs of an HMC entry point
+template <typename T>
+static IterArgs<T> hmc_args(const CallViews& v, const ehmc_hmc_args* a) {
+  IterArgs<T> A = base_args<T>(v, a->stepSize, a->stepSizeSq, a->numSteps);
+  A.flags = a->flags;
+  A.kB = a->boltzmann;
+  A.temp = a->temperature;
+  A.pscale = std::sqrt(a->boltzmann * a->temperature);
+  A.seed = a->seed;
+  A.iter = a->iteration;
+  A.offset = a->particleOffset;
+  A.dyn = static_cast<const DynArgs*>(a->dynamic);
+  return A;
+}
+
+enum class HmcEntry { iter, run, ensemble };
+
+// The checks of ehmc_hmc_args (and of the fused ensemble run's ehmc_adapt_args `ad`) the HMC entry points share, in
+// each entry point's own words.  `negative`: one of the call's own counts (iterations, offsets) is below 0.
+static int check_hmc_args(HmcEntry e, const char* fn, const ehmc_hmc_args* a, const ehmc_adapt_args* ad, bool negative) {
+  if (!a) return fail(EHMC_ERR_INVALID, "%s: args is NULL", fn);
+  if (e == HmcEntry::ensemble) {
+    if (a->struct_size != sizeof(ehmc_hmc_args) || ad->struct_size != sizeof(ehmc_adapt_args))
+      return fail(EHMC_ERR_INVALID, "%s: struct_size mismatch", fn);
+  } else if (a->struct_size != sizeof(ehmc_hmc_args)) {
+    return fail(EHMC_ERR_INVALID, "%s: args.struct_size %u != %zu", fn, a->struct_size, sizeof(ehmc_hmc_args));
+  }
+  if (a->numSteps < 0 || negative)
+    return fail(EHMC_ERR_INVALID, e == HmcEntry::iter ? "%s: numSteps < 0" : "%s: negative count", fn);
+  if (e == HmcEntry::ensemble && a->integrator != EHMC_LEAPFROG) return fail(EHMC_ERR_UNSUPPORTED, "%s: leapfrog only", fn);
+  if (a->integrator != EHMC_LEAPFROG && a->integrator != EHMC_STORMER_VERLET)
+    return fail(EHMC_ERR_INVALID, "%s: Invalid integration method selected.", fn);
+  // ehmc_hmc_iter checks args.dynamic against the potential
+  if (e != HmcEntry::iter && a->dynamic != nullptr) return fail(EHMC_ERR_UNSUPPORTED, "%s: args.dynamic is not supported here", fn);
+  return EHMC_OK;
+}
+
 // Device path of one iteration / integration.  Statistics go to stats_dev (device, 2D+3 doubles).
 template <typename T>
 static int run_device(ehmc_ctx* c, const ehmc_potential* pot, IterArgs<T> A, int integ, bool hmc, double* stats_dev,
                       cudaStream_t st) {
-  const bool pps = per_particle_stats(c, pot, integ);
+  const bool pps = per_particle_stats(c, pot);
   const int NS = 2 * A.D + 3;
   long long nblk = 0;
   if (stats_dev != nullptr) {
@@ -753,7 +631,7 @@ static int run_device(ehmc_ctx* c, const ehmc_potential* pot, IterArgs<T> A, int
       if (A.P >= 16LL * A.D) TRY(c->partials.ensure(sizeof(double) * (size_t)nblk * NS));
       A.partials = static_cast<double*>(c->pstats.ptr);
     } else {
-      nblk = traj_blocks<T>(c, pot, A.P, integ);
+      nblk = traj_blocks<T>(c, pot, A.P);
       TRY(c->partials.ensure(sizeof(double) * (size_t)std::max(1LL, nblk) * NS));
       A.partials = static_cast<double*>(c->partials.ptr);
     }
@@ -807,8 +685,8 @@ static int run_host(ehmc_ctx* c, const ehmc_potential* pot, const CallViews& v, 
   const size_t slab_bytes = slab_elems * sizeof(T) + (size_t)chunk + 64;
   for (int i = 0; i < N_STAGE; ++i) TRY(c->stage[i].ensure(slab_bytes));
   long long blocks_total = 0;  // upper bound of the statistics rows (exact count: rows_done below)
-  for (long long k = 0; k < nchunks; ++k) blocks_total += traj_blocks<T>(c, pot, std::min(chunk, P - k * chunk), integ);
-  const bool pps = per_particle_stats(c, pot, integ);
+  for (long long k = 0; k < nchunks; ++k) blocks_total += traj_blocks<T>(c, pot, std::min(chunk, P - k * chunk));
+  const bool pps = per_particle_stats(c, pot);
   if (v.has_stats) {
     // fused families: one row of NS sums per CTA.  per-particle families: [P][3] rows in pstats plus
     // one row of coordinate sums per chunk (k_colstats) in partials.
@@ -944,12 +822,7 @@ extern "C" int ehmc_hmc_iter(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor*
   const char* fn = "ehmc_hmc_iter";
   CallViews v;
   TRY(common_checks(ctx, pot, q, mass, &v, fn));
-  if (!a) return fail(EHMC_ERR_INVALID, "%s: args is NULL", fn);
-  if (a->struct_size != sizeof(ehmc_hmc_args))
-    return fail(EHMC_ERR_INVALID, "%s: args.struct_size %u != %zu", fn, a->struct_size, sizeof(ehmc_hmc_args));
-  if (a->numSteps < 0) return fail(EHMC_ERR_INVALID, "%s: numSteps < 0", fn);
-  if (a->integrator != EHMC_LEAPFROG && a->integrator != EHMC_STORMER_VERLET)
-    return fail(EHMC_ERR_INVALID, "%s: Invalid integration method selected.", fn);
+  TRY(check_hmc_args(HmcEntry::iter, fn, a, nullptr, false));
   if (p_out) {
     TRY(parse_float(p_out, "p_out", 2, v.bits, &v.p));
     v.has_p = true;
@@ -979,33 +852,19 @@ extern "C" int ehmc_hmc_iter(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor*
   TRY(check_same_place(v));
   TRY(enter_device(ctx));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  auto fill = [&](auto& A) {
-    A.flags = a->flags;
-    A.kB = a->boltzmann;
-    A.temp = a->temperature;
-    A.pscale = std::sqrt(a->boltzmann * a->temperature);
-    A.seed = a->seed;
-    A.iter = a->iteration;
-    A.offset = a->particleOffset;
-    A.dyn = static_cast<const DynArgs*>(a->dynamic);
-  };
   if (a->dynamic != nullptr) {
     // only kernels that resolve the block themselves; everything else would silently use the host values
-    const bool small = pot->family == EHMC_FAMILY_DIAG_GAUSSIAN || pot->family == EHMC_FAMILY_FUNNEL ||
-                       pot->family == EHMC_FAMILY_COIN_TOSS || (pot->family == EHMC_FAMILY_DENSE_GAUSSIAN && pot->D <= 16);
-    const bool tc3 = v.bits == 32 && use_dense_tc(ctx, pot, a->integrator);
-    if (v.q.host || !(small || tc3))
+    const bool tc3 = v.bits == 32 && use_dense_tc(ctx, pot);
+    if (v.q.host || !(small_family(pot) || tc3))
       return fail(EHMC_ERR_UNSUPPORTED, "%s: args.dynamic needs device tensors and a small-D or float32 dense (tensor-core) potential", fn);
   }
   if (v.bits == 32) {
-    IterArgs<float> A = base_args<float>(v, a->stepSize, a->stepSizeSq, a->numSteps);
-    fill(A);
+    IterArgs<float> A = hmc_args<float>(v, a);
     if (v.q.host) return run_host<float>(ctx, pot, v, A, a->integrator, true);
     return run_device<float>(ctx, pot, A, a->integrator, true,
                              v.has_stats ? reinterpret_cast<double*>(v.stats.data) : nullptr, st);
   }
-  IterArgs<double> A = base_args<double>(v, a->stepSize, a->stepSizeSq, a->numSteps);
-  fill(A);
+  IterArgs<double> A = hmc_args<double>(v, a);
   if (v.q.host) return run_host<double>(ctx, pot, v, A, a->integrator, true);
   return run_device<double>(ctx, pot, A, a->integrator, true,
                             v.has_stats ? reinterpret_cast<double*>(v.stats.data) : nullptr, st);
@@ -1017,14 +876,7 @@ extern "C" int ehmc_hmc_iter(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor*
 template <typename T>
 static int hmc_run_typed(ehmc_ctx* ctx, const ehmc_potential* pot, const CallViews& v, const ehmc_hmc_args* a, int nIter,
                          const View* vs, const View* vm, long long s0, long long S, int* accepted, cudaStream_t st) {
-  IterArgs<T> A = base_args<T>(v, a->stepSize, a->stepSizeSq, a->numSteps);
-  A.flags = a->flags;
-  A.kB = a->boltzmann;
-  A.temp = a->temperature;
-  A.pscale = std::sqrt(a->boltzmann * a->temperature);
-  A.seed = a->seed;
-  A.iter = a->iteration;
-  A.offset = a->particleOffset;
+  IterArgs<T> A = hmc_args<T>(v, a);
   RunArgs<T> R;
   R.samples = vs ? reinterpret_cast<T*>(vs->data) : nullptr;
   R.momenta = vm ? reinterpret_cast<T*>(vm->data) : nullptr;
@@ -1044,16 +896,8 @@ extern "C" int ehmc_hmc_run(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* 
   const char* fn = "ehmc_hmc_run";
   CallViews v;
   TRY(common_checks(ctx, pot, q, mass, &v, fn));
-  if (!a) return fail(EHMC_ERR_INVALID, "%s: args is NULL", fn);
-  if (a->struct_size != sizeof(ehmc_hmc_args))
-    return fail(EHMC_ERR_INVALID, "%s: args.struct_size %u != %zu", fn, a->struct_size, sizeof(ehmc_hmc_args));
-  if (a->numSteps < 0 || numIterations < 0 || sampleOffset < 0) return fail(EHMC_ERR_INVALID, "%s: negative count", fn);
-  if (a->integrator != EHMC_LEAPFROG && a->integrator != EHMC_STORMER_VERLET)
-    return fail(EHMC_ERR_INVALID, "%s: Invalid integration method selected.", fn);
-  if (a->dynamic != nullptr) return fail(EHMC_ERR_UNSUPPORTED, "%s: args.dynamic is not supported here", fn);
-  const bool small = pot->family == EHMC_FAMILY_DIAG_GAUSSIAN || pot->family == EHMC_FAMILY_FUNNEL ||
-                     pot->family == EHMC_FAMILY_COIN_TOSS || (pot->family == EHMC_FAMILY_DENSE_GAUSSIAN && pot->D <= 16);
-  if (v.q.host || !small)
+  TRY(check_hmc_args(HmcEntry::run, fn, a, nullptr, numIterations < 0 || sampleOffset < 0));
+  if (v.q.host || !small_family(pot))
     return fail(EHMC_ERR_UNSUPPORTED, "%s: device tensors and a small-D potential family are required", fn);
   View vs, vm, va;
   long long S = 0;
@@ -1097,15 +941,8 @@ extern "C" int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, D
   CallViews v;
   TRY(common_checks(ctx, pot, q, mass, &v, fn));
   if (!a || !ad || !state) return fail(EHMC_ERR_INVALID, "%s: args, adapt and state are required", fn);
-  if (a->struct_size != sizeof(ehmc_hmc_args) || ad->struct_size != sizeof(ehmc_adapt_args))
-    return fail(EHMC_ERR_INVALID, "%s: struct_size mismatch", fn);
-  if (a->numSteps < 0 || numIterations < 0 || traceParticles < 0 || traceOffset < 0)
-    return fail(EHMC_ERR_INVALID, "%s: negative count", fn);
-  if (a->integrator != EHMC_LEAPFROG) return fail(EHMC_ERR_UNSUPPORTED, "%s: leapfrog only", fn);
-  if (a->dynamic != nullptr) return fail(EHMC_ERR_UNSUPPORTED, "%s: args.dynamic is not supported here", fn);
-  const bool small = pot->family == EHMC_FAMILY_DIAG_GAUSSIAN || pot->family == EHMC_FAMILY_FUNNEL ||
-                     pot->family == EHMC_FAMILY_COIN_TOSS || (pot->family == EHMC_FAMILY_DENSE_GAUSSIAN && pot->D <= 16);
-  if (v.q.host || !small)
+  TRY(check_hmc_args(HmcEntry::ensemble, fn, a, ad, numIterations < 0 || traceParticles < 0 || traceOffset < 0));
+  if (v.q.host || !small_family(pot))
     return fail(EHMC_ERR_UNSUPPORTED, "%s: device tensors and a small-D potential family are required", fn);
   if (!(ad->numParticlesTotal > 0) || !(ad->minStep > 0) || !(ad->maxStep >= ad->minStep))
     return fail(EHMC_ERR_INVALID, "%s: bad adaptation scalars", fn);
@@ -1143,14 +980,7 @@ extern "C" int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, D
   for (int i = 0; i < n_adapt; ++i) gains[i] = ad->gain0 / std::pow(st_host[2] + 1.0 + i, ad->kappa);
   auto run = [&](auto tag) -> int {
     typedef decltype(tag) T;
-    IterArgs<T> A = base_args<T>(v, a->stepSize, a->stepSizeSq, a->numSteps);
-    A.flags = a->flags;
-    A.kB = a->boltzmann;
-    A.temp = a->temperature;
-    A.pscale = std::sqrt(a->boltzmann * a->temperature);
-    A.seed = a->seed;
-    A.iter = a->iteration;
-    A.offset = a->particleOffset;
+    IterArgs<T> A = hmc_args<T>(v, a);
     EnsRunArgs<T> R;
     memset(&R, 0, sizeof(R));
     R.nIter = numIterations;
@@ -1261,8 +1091,9 @@ static int eval_device(ehmc_ctx* c, const ehmc_potential* p, const T* q, long lo
                        long long g_ld, cudaStream_t st) {
   if (P == 0) return EHMC_OK;
   if (p->family == EHMC_FAMILY_DENSE_GAUSSIAN) {
-    const T* mu = static_cast<const T*>(p->d1);
-    k_eval_dense<T><<<(unsigned)((P + 127) / 128), 128, 0, st>>>(q, q_ld, P, p->D, static_cast<const T*>(p->d2), mu, e, g, g_ld);
+    const T* lambda = static_cast<const T*>(p->dense.lambda);
+    const T* mu = static_cast<const T*>(p->dense.mu);
+    k_eval_dense<T><<<(unsigned)((P + 127) / 128), 128, 0, st>>>(q, q_ld, P, p->D, lambda, mu, e, g, g_ld);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return EHMC_OK;

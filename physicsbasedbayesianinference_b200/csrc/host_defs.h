@@ -77,31 +77,56 @@ struct ehmc_ctx {
   int tc_debug = 0;               // profiling knobs of the tensor-core kernels (see DenseTcArgs::dbg)
 };
 
+// Per-family state of a potential: what that family's launchers and eval read.  Device arrays hold the dtype of the
+// potential (float / double) unless noted.
+struct DenseState {                 // dense Gaussian (and the diagonal family for 32 < D <= 128)
+  void* lambda = nullptr;           // Lambda [D][D] row-major (k_eval_dense)
+  void* mu = nullptr;               // mu [D]; D > 16: zero padded to 8 TN
+  void* ls = nullptr;               // D > 16: Lambda transposed and padded for k_dense [D][8][TNP]
+  int tn = 0;                       // D > 16: rows of Lambda per warp of k_dense
+  std::vector<double> h_lambda, h_mu;  // D <= 16: host copies (make_dense_small)
+  struct {                          // float32, D > 16: 3xFP16 tensor-core operands (pack_dense_tc3)
+    void* hi = nullptr;             // fp16 [KP/8][NP][8] rn16(scale * Lambda)
+    void* lo = nullptr;             // fp16 [KP/8][NP][8] rn16(scale * Lambda - hi)
+    void* mu = nullptr;             // float [128], zero padded
+    int c8 = 0;                     // ceil(D / 8) (0 = not packed)
+    bool exact = false;             // the (hi, lo) split represents Lambda to float32 accuracy (the auto guard)
+    float inv_scale = 1.f;          // 1 / scale (power of two)
+  } tc3;
+};
+
+// gradient kernel of the logistic family: the values of the precision selector (scalars[1]) but auto (3)
+enum LogisticKernel { LOGISTIC_EXACT = 0, LOGISTIC_BF16 = 1, LOGISTIC_FP16X3 = 2 };
+
+struct LogisticState {
+  int n = 0;                        // data rows
+  LogisticKernel kernel = LOGISTIC_EXACT;  // resolved from the selector (auto decides here, once)
+  void* x = nullptr;                // exact kernel: X [N][D]
+  void* y = nullptr;                // exact kernel: y [N]
+  struct {                          // tensor-core kernels: X and y in 64-row chunks (pack_logistic_tc)
+    void* buf = nullptr;            // bf16: NC chunks; fp16 split: 2 NC ring entries (lo, hi)
+    int nc = 0, dp = 0, npad = 0;   // chunks, D rounded up to 16, zero rows appended to the last chunk
+    unsigned bytes = 0;             // one chunk / ring entry
+    float x_iscale = 1.f;           // fp16 split: 1 / (power-of-two scale of X)
+  } chunks;
+};
+
+struct NBodyState {
+  void* body_mass = nullptr;        // [B]
+  int b = 0;                        // bodies per particle
+};
+
 struct ehmc_potential {
   ehmc_ctx* ctx = nullptr;
   int family = 0;
   int D = 0;
   int bits = 32;
-  std::vector<double> hp0, hp1;  // host copies of the parameters (double)
   std::vector<double> scalars;
-  void* d0 = nullptr;  // dense: packed Ls ; nbody: body masses ; logistic: X
-  void* d1 = nullptr;  // dense: mu (padded) ; logistic: y
-  void* d2 = nullptr;  // dense: plain Lambda row-major (eval kernel)
-  int TN = 0;          // dense tile selection
-  void* d6 = nullptr;  // logistic tensor-core path: packed bf16 X chunks + y
-  int lt_nc = 0, lt_dp = 0, lt_npad = 0;
-  unsigned lt_chunk_bytes = 0;
-  void* d7 = nullptr;  // dense float32 3xFP16 tensor-core path: Lambda_hi fp16 [KP/8][NP][8]
-  void* d8 = nullptr;  //                                       Lambda_lo
-  void* d9 = nullptr;  //                                       mu [128]
-  int tc3_c8 = 0;      // ceil(D / 8) (0 = not eligible)
-  int tc3_ok = 0;      // 1: the (hi, lo) fp16 split represents Lambda to float32 accuracy (no entry flushes)
-  float tc3_inv_lscale = 1.f;
-  int use_tc = 0;      // logistic (scalars[1]): 0 = CUDA cores (exact), 1 = bf16 tensor-core gradient,
-                       // 2 = float32-accurate tensor-core gradient (3-pass fp16 split)
-  float lts_x_iscale = 1.f;  // 1 / (power-of-two scale of the packed fp16 X)
-  int B = 0;           // nbody: bodies per particle
-  int N = 0;           // logistic: data rows
+  std::vector<double> diag_k;                    // diagonal Gaussian, D <= 32 (make_diag)
+  std::vector<double> coin_k, coin_n;            // coin toss: successes, trials (make_coin)
+  DenseState dense;
+  LogisticState logistic;
+  NBodyState nbody;
 };
 
 // peer-memory mailboxes of the fused ensemble run (comm.cu)
@@ -117,11 +142,31 @@ struct ehmc_comm {
   unsigned long long seq = 0;                    // iterations reduced so far (identical on all ranks)
 };
 
-// ---- launchers (explicitly instantiated for float / double in inst_*.cu) ----------
+// ---- potential builders and launchers (explicitly instantiated for float / double in inst_*.cu) ----------
 namespace ehmc {
 
 constexpr int K1_THREADS_HOST = 128;
 constexpr int K2_WARPS_HOST = 8;
+
+// new device array holding `bytes` host bytes (*dptr = nullptr, nothing allocated, for 0 bytes)
+int upload_raw(const void* src, size_t bytes, void** dptr);
+// new device array of T holding h converted entry by entry
+template <typename T>
+int upload(const std::vector<double>& h, void** dptr) {
+  const std::vector<T> t(h.begin(), h.end());
+  return upload_raw(t.data(), sizeof(T) * t.size(), dptr);
+}
+
+// Builders: the device state of a potential whose parameters ehmc_potential_create has checked (host, float64).
+// On failure the buffers allocated so far stay in the state for ehmc_potential_destroy.
+template <typename T>
+int build_dense(ehmc_potential* p, std::vector<double>& lambda, std::vector<double>& mu);  // takes the vectors at D <= 16
+int pack_dense_tc3(ehmc_potential* p, const std::vector<double>& lambda, const std::vector<double>& mu);
+template <typename T>
+int build_logistic(ehmc_potential* p, const std::vector<double>& X, const std::vector<double>& y, int precision);
+int pack_logistic_tc(ehmc_potential* p, const std::vector<double>& X, const std::vector<double>& y, int precision);
+template <typename T>
+int build_nbody(ehmc_potential* p, const std::vector<double>& body_mass);
 
 // fused trajectory kernels, D <= 32 register-resident families
 template <typename T>

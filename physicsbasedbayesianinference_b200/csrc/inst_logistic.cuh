@@ -10,9 +10,9 @@ namespace ehmc {
 template <typename T>
 static LogisticArgs<T> logistic_args(const ehmc_potential* p) {
   LogisticArgs<T> pa;
-  pa.X = static_cast<const T*>(p->d0);
-  pa.y = static_cast<const T*>(p->d1);
-  pa.N = p->N;
+  pa.X = static_cast<const T*>(p->logistic.x);
+  pa.y = static_cast<const T*>(p->logistic.y);
+  pa.N = p->logistic.n;
   pa.D = p->D;
   pa.inv_s2 = (T)(1.0 / (p->scalars[0] * p->scalars[0]));
   return pa;
@@ -22,8 +22,9 @@ template <typename T>
 static int logistic_grad(ehmc_ctx* c, const ehmc_potential* p, const T* theta, long long t_ld, long long P, T* g,
                          long long g_ld, T* e, double* e64, cudaStream_t st) {
   if constexpr (sizeof(T) == 4) {
-    if (p->use_tc == 2 && p->d6 != nullptr) return logistic_grad_tcs(c, p, theta, t_ld, P, g, g_ld, e, e64, st);
-    if (p->use_tc == 1 && p->d6 != nullptr) return logistic_grad_tc(c, p, theta, t_ld, P, g, g_ld, e, e64, st);
+    const LogisticState& s = p->logistic;
+    if (s.kernel == LOGISTIC_FP16X3 && s.chunks.buf) return logistic_grad_tcs(c, p, theta, t_ld, P, g, g_ld, e, e64, st);
+    if (s.kernel == LOGISTIC_BF16 && s.chunks.buf) return logistic_grad_tc(c, p, theta, t_ld, P, g, g_ld, e, e64, st);
   }
   constexpr int PT = LogiTile<T>::PT;
   const int D = p->D, DS = (D + 3) & ~3;
@@ -35,6 +36,20 @@ static int logistic_grad(ehmc_ctx* c, const ehmc_potential* p, const T* theta, l
   c->launches++;
   CUDA_TRY(cudaGetLastError());
   return EHMC_OK;
+}
+
+// precision: the selector ehmc_potential_create checked (1 and 2 need float32 state; auto falls back to the exact
+// kernel for float64 state or where the fp16 split of X loses accuracy).  X and y go to the device as they are only
+// for the exact kernel.
+template <typename T>
+int build_logistic(ehmc_potential* p, const std::vector<double>& X, const std::vector<double>& y, int precision) {
+  LogisticState& s = p->logistic;
+  if constexpr (sizeof(T) == 4) {
+    if (precision != LOGISTIC_EXACT) TRY(pack_logistic_tc(p, X, y, precision));
+  }
+  if (s.kernel != LOGISTIC_EXACT) return EHMC_OK;
+  TRY(upload<T>(X, &s.x));
+  return upload<T>(y, &s.y);
 }
 
 template <typename T>

@@ -14,8 +14,8 @@ static int nbody_threads(int B, int ti) {
 template <typename T>
 static NBodyArgs<T> nbody_args(const ehmc_potential* p) {
   NBodyArgs<T> pa;
-  pa.bmass = static_cast<const T*>(p->d0);
-  pa.B = p->B;
+  pa.bmass = static_cast<const T*>(p->nbody.body_mass);
+  pa.B = p->nbody.b;
   pa.G = (T)p->scalars[0];
   pa.eps2 = (T)(p->scalars[1] * p->scalars[1]);
   pa.fcache = nullptr;
@@ -27,7 +27,7 @@ static NBodyArgs<T> nbody_args(const ehmc_potential* p) {
 template <typename T, int TI>
 static int launch_nbody_ti(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, bool hmc,
                            cudaStream_t st) {
-  const int B = p->B, nt = nbody_threads(B, TI);
+  const int B = p->nbody.b, nt = nbody_threads(B, TI);
   if (nt * TI < B) return fail(EHMC_ERR_UNSUPPORTED, "nbody: B = %d > %d bodies", B, 1024 * TI);
   const size_t sm = (size_t)B * BodyRec<T>::VECS * 4 * sizeof(T) + 40 * sizeof(T);
   if (sm > 227 * 1024) return fail(EHMC_ERR_UNSUPPORTED, "nbody: B = %d needs %zu B shared memory", B, sm);
@@ -69,15 +69,15 @@ static int launch_nbody_ti(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<
 template <typename T>
 int launch_nbody(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, bool hmc, cudaStream_t st) {
   // 4 bodies per thread (twice the warps per SM) while that covers B, else 8
-  const int ti = c->nbody_ti ? c->nbody_ti : (p->B <= 4096 ? 4 : 8);
-  if (ti == 4 && p->B <= 4096) return launch_nbody_ti<T, 4>(c, p, A, integ, hmc, st);
+  const int ti = c->nbody_ti ? c->nbody_ti : (p->nbody.b <= 4096 ? 4 : 8);
+  if (ti == 4 && p->nbody.b <= 4096) return launch_nbody_ti<T, 4>(c, p, A, integ, hmc, st);
   return launch_nbody_ti<T, 8>(c, p, A, integ, hmc, st);
 }
 
 template <typename T>
 int eval_nbody(ehmc_ctx* c, const ehmc_potential* p, const T* q, long long q_ld, long long P, T* e, T* g,
                long long g_ld, cudaStream_t st) {
-  const int B = p->B;
+  const int B = p->nbody.b;
   int nt = 32;
   while (nt < B && nt < 256) nt <<= 1;
   const size_t sm = (size_t)B * 4 * sizeof(T) + 40 * sizeof(T);
@@ -89,6 +89,12 @@ int eval_nbody(ehmc_ctx* c, const ehmc_potential* p, const T* q, long long q_ld,
   c->launches++;
   CUDA_TRY(cudaGetLastError());
   return EHMC_OK;
+}
+
+template <typename T>
+int build_nbody(ehmc_potential* p, const std::vector<double>& body_mass) {
+  p->nbody.b = (int)body_mass.size();
+  return upload<T>(body_mass, &p->nbody.body_mass);
 }
 
 template <typename T>

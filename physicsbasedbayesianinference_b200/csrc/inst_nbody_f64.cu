@@ -4,4 +4,5 @@ template int launch_nbody<double>(ehmc_ctx*, const ehmc_potential*, const IterAr
 template int eval_nbody<double>(ehmc_ctx*, const ehmc_potential*, const double*, long long, long long, double*, double*, long long,
                              cudaStream_t);
 template int colstats<double>(ehmc_ctx*, const double*, long long, long long, int, double*, cudaStream_t);
+template int build_nbody<double>(ehmc_potential*, const std::vector<double>&);
 }  // namespace ehmc

@@ -12,15 +12,15 @@ namespace ehmc {
 template <typename T, int DT>
 static DiagPot<T, DT> make_diag(const ehmc_potential* p) {
   DiagPot<T, DT> f;
-  for (int d = 0; d < DT; ++d) f.k[d] = d < p->D ? (T)p->hp0[d] : T(0);
+  for (int d = 0; d < DT; ++d) f.k[d] = d < p->D ? (T)p->diag_k[d] : T(0);
   return f;
 }
 template <typename T, int DT>
 static DenseSmallPot<T, DT> make_dense_small(const ehmc_potential* p) {
   DenseSmallPot<T, DT> f;
   for (int i = 0; i < DT; ++i) {
-    f.mu[i] = i < p->D ? (T)p->hp1[i] : T(0);
-    for (int j = 0; j < DT; ++j) f.lam[i * DT + j] = (i < p->D && j < p->D) ? (T)p->hp0[(size_t)i * p->D + j] : T(0);
+    f.mu[i] = i < p->D ? (T)p->dense.h_mu[i] : T(0);
+    for (int j = 0; j < DT; ++j) f.lam[i * DT + j] = (i < p->D && j < p->D) ? (T)p->dense.h_lambda[(size_t)i * p->D + j] : T(0);
   }
   return f;
 }
@@ -55,8 +55,8 @@ template <typename T, int DT>
 static CoinPot<T, DT> make_coin(const ehmc_potential* p) {
   CoinPot<T, DT> f;
   for (int d = 0; d < DT; ++d) {
-    f.k[d] = d < p->D ? (T)p->hp0[d] : T(0);
-    f.nk[d] = d < p->D ? (T)(p->hp1[d] - p->hp0[d]) : T(0);
+    f.k[d] = d < p->D ? (T)p->coin_k[d] : T(0);
+    f.nk[d] = d < p->D ? (T)(p->coin_n[d] - p->coin_k[d]) : T(0);
   }
   return f;
 }

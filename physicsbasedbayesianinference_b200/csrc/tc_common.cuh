@@ -5,6 +5,10 @@
 
 #include <cuda_fp16.h>
 
+#include <algorithm>
+#include <cmath>
+#include <vector>
+
 #include "common.cuh"
 
 namespace ehmc {
@@ -266,5 +270,28 @@ __device__ __forceinline__ uint32_t h16_saturated(uint32_t w) {
   const uint32_t a = w & 0x7fff7fffu;
   return (uint32_t)((a & 0xffffu) >= 0x7bffu) | (uint32_t)((a >> 16) >= 0x7bffu);
 }
+
+// ---- host: fp16 (hi, lo) split of a constant operand (Lambda of k_dense_tc3, X of k_logistic_tcs) ----------------
+// One power-of-two scale serves the whole matrix: max |v| (v rounded to float32) lands in [2^(target-1), 2^target).
+struct Fp16Split {
+  double amax = 0.0;  // max |float32(v)|
+  int shift = 0;      // scale = 2^shift, clamped to [2^-100, 2^100]
+  double scale = 1.0;
+  Fp16Split(const std::vector<double>& v, int target) {
+    for (double e : v) amax = std::max(amax, std::fabs((double)(float)e));
+    int ex = 0;
+    if (amax > 0 && std::isfinite(amax)) std::frexp(amax, &ex);  // amax = f * 2^ex, f in [0.5, 1)
+    shift = std::max(-100, std::min(100, target - ex));
+    scale = std::ldexp(1.0, shift);
+  }
+  // x = float32(float32(v) * scale) as hi = rn16(x), lo = rn16(x - hi); returns x, *rem = x - hi - lo (exact)
+  float operator()(double v, __half* hi, __half* lo, double* rem) const {
+    const float x = (float)((double)(float)v * scale);
+    *hi = __float2half_rn(x);
+    *lo = __float2half_rn(x - __half2float(*hi));
+    *rem = (double)x - (double)__half2float(*hi) - (double)__half2float(*lo);
+    return x;
+  }
+};
 
 }  // namespace ehmc
