@@ -350,6 +350,80 @@ def hmc_iter_diag_mass(q, z, u, mass, mass_diag, temperature, step_size, n_steps
     return np.where(reject[None, :], q, x), ~reject, old_h, new_h
 
 
+def ensemble_stats(q_kept, accept, old_h, new_h):
+    """The 2D+3 ensemble statistics of one iteration (build-defined; the reference has none): the vector
+    ehmc_hmc_iter returns and parallel.unpack_stats reads (physicsbasedbayesianinference_b200/parallel.py,
+    csrc/k_small.cuh WarpStats), as plain float64 sums over the particles:
+        [0] n_accept, [1] sum min(1, exp(oldH - newH)) (src/HMC.py:168), [2] sum H of the kept state (newH where the
+        proposal was accepted, oldH where it was not, src/HMC.py:173-176), [3 .. 3+D) sum q_d, [3+D .. 3+2D) sum q_d^2
+        of the kept positions q_kept (D, P).
+    Non-finite energies are not handled here (the kernels count a NaN ratio as acceptance probability 1)."""
+    q_kept = np.asarray(q_kept, dtype=np.float64)
+    accept = np.asarray(accept, dtype=bool)
+    old_h = np.asarray(old_h, dtype=np.float64)
+    new_h = np.asarray(new_h, dtype=np.float64)
+    with np.errstate(over="ignore"):
+        acc_prob = np.minimum(1.0, np.exp(old_h - new_h))
+    kept_h = np.where(accept, new_h, old_h)
+    return np.concatenate([[float(np.sum(accept)), np.sum(acc_prob), np.sum(kept_h)], np.sum(q_kept, axis=1),
+                           np.sum(q_kept * q_kept, axis=1)])
+
+
+def adaptive_run(q0, mass, pot, num_iterations, temperature, step_size, n_steps, seed, *, iteration0=0,
+                 particle_offset=0, adapt_iterations=None, target=0.8, lag=1, gain0=1.5, kappa=0.5, min_step=1e-6,
+                 max_step=1e3, max_move=0.7, bug_compat=False, boltzmann=BOLTZMANN):
+    """HMC.run(adapt=True, keepNumSteps=True) of one float64 ensemble, replayed iteration by iteration
+    (build-defined; the reference has no adaptation):
+    * iteration k draws z, u from philox_stream(seed, iteration0 + k, particle ids, D, float64) and runs hmc_iter
+      (src/HMC.py:154-179) with the step size of iteration k and a fixed number of leapfrog steps;
+    * its statistics (ensemble_stats) give acceptRate = n_accept / P, meanAcceptProb, meanH;
+    * the Robbins-Monro rule of parallel.StepSizeAdapter, restated: for k < adapt_iterations,
+          j += 1;  log h += clip(gain0 / j^kappa * (meanAcceptProb - target), -max_move, max_move),
+          log h clipped to [log min_step, log max_step],  h = exp(log h)
+      and the lag schedule of HMC.run(adaptLag=lag): the statistics of iteration k set the step size of iteration
+      k + 1 + lag (iterations 0 .. lag keep the incoming step size, later ones the newest update).
+    Returns dict(stepSize[S], acceptRate[S], meanAcceptProb[S], meanH[S], q (D, P) after the run, trace (D, P, S),
+    mean[D], var[D] (moments pooled over the iterations), finalStepSize: the newest step size, what HMC.run leaves in
+    HMC.stepSize)."""
+    q = np.array(q0, dtype=np.float64, copy=True)
+    mass = np.asarray(mass, dtype=np.float64)
+    D, P = q.shape
+    S = int(num_iterations)
+    n_adapt = S if adapt_iterations is None else min(S, int(adapt_iterations))
+    ids = np.arange(P, dtype=np.uint64) + np.uint64(particle_offset)
+    log_h = np.log(step_size)
+    lo, hi = np.log(min_step), np.log(max_step)
+    sched = [float(step_size)] * (S + 1 + lag)  # step size of every iteration
+    h_new = float(step_size)
+    j = 0
+    out = dict(stepSize=[], acceptRate=[], meanAcceptProb=[], meanH=[])
+    trace = np.empty((D, P, S))
+    sums = np.zeros(2 * D)
+    for k in range(S):
+        h = sched[k]
+        z, u = philox_stream(seed, iteration0 + k, ids, D, np.float64)
+        q, _, acc, old_h, new_h = hmc_iter(q, z, u, mass, temperature, h, n_steps, pot, boltzmann=boltzmann,
+                                           bug_compat=bug_compat)
+        st = ensemble_stats(q, acc, old_h, new_h)
+        out["stepSize"].append(h)
+        out["acceptRate"].append(st[0] / P)
+        out["meanAcceptProb"].append(st[1] / P)
+        out["meanH"].append(st[2] / P)
+        sums += st[3:]
+        trace[:, :, k] = q
+        if k < n_adapt:
+            acc_prob = st[1] / P if np.isfinite(st[1]) else 0.0
+            j += 1
+            log_h = min(max(log_h + min(max(gain0 / j**kappa * (acc_prob - target), -max_move), max_move), lo), hi)
+            h_new = float(np.exp(log_h))
+            for t in range(k + 1 + lag, S + 1 + lag):
+                sched[t] = h_new
+    n = max(S, 1) * P
+    mean = sums[:D] / n
+    out.update(q=q, trace=trace, mean=mean, var=sums[D:] / n - mean * mean, finalStepSize=h_new)
+    return out
+
+
 def get_samples(num_dims, num_particles, mass, pot, num_samples, temperature, q_std,
                 simul_time, step_size, integrator="Leapfrog", record=None):
     """HMC.getSamples, src/HMC.py:123-183, drawing from NumPy's GLOBAL legacy
