@@ -108,7 +108,18 @@ typedef enum {
    * U = -sum_d [ k_d ln q_d + (n_d - k_d) ln(1 - q_d) ],  dU/dq_d = -k_d/q_d + (n_d - k_d)/(1 - q_d)
    * (references/NotesOnParticleBasedHMC.pdf eq. 22).  Outside (0, 1) U is NaN, as ln of a negative
    * number is in the reference.  params: successes k[D], trials n[D].  scalars: none.  D <= 32. */
-  EHMC_FAMILY_COIN_TOSS = 6
+  EHMC_FAMILY_COIN_TOSS = 6,
+  /* Normal-normal hierarchical model (eight schools): y_j ~ N(theta_j, sigma_j^2) with sigma_j known,
+   * theta_j ~ N(mu, tau^2), mu ~ N(muLoc, muScale^2), tau ~ HalfCauchy(tauScale), j = 0 .. J-1, 1 <= J <= 30,
+   * in NumPyro's unconstrained coordinates, D = J + 2:  q[0] = mu, q[1] = eta = ln tau, q[2+j] = theta_j
+   * (centered = 1) or thetaTilde_j with theta_j = mu + e^eta thetaTilde_j (centered = 0).  U is minus the log
+   * density with the Jacobian of eta, additive constants dropped:
+   *   (mu - muLoc)^2 / (2 muScale^2) + softplus(2 eta - 2 ln tauScale) - eta + 0.5 sum_j (y_j - theta_j)^2 / sigma_j^2
+   *   centred:      + J eta + 0.5 e^{-2 eta} sum_j (theta_j - mu)^2
+   *   non-centred:  + 0.5 sum_j thetaTilde_j^2
+   * params: y[J], sigma[J] [, scale[D]]: with scale, the same potential in rescaled coordinates, U'(q) = U(scale q)
+   * (diagonal mass matrix, HMC.run(adaptMass=True)).  scalars: {muLoc, muScale, tauScale, centered}. */
+  EHMC_FAMILY_HIERARCHICAL_NORMAL = 7
 } ehmc_family;
 
 typedef enum {
@@ -271,7 +282,8 @@ EHMC_API int ehmc_hmc_iter(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q
  *                sampleOffset .. sampleOffset + numIterations - 1 are written
  *   momenta_out  [D*P, S] optional
  *   accepted_out [P] int32 optional: accepted proposals per particle
- * Device tensors and the small-D families only (diagonal / small dense Gaussian, funnel, coin toss);
+ * Device tensors and the small-D families only (diagonal / small dense Gaussian, funnel, coin toss, hierarchical
+ * normal);
  * EHMC_ERR_UNSUPPORTED otherwise -- call ehmc_hmc_iter per iteration then. */
 EHMC_API int ehmc_hmc_run(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
                  const ehmc_hmc_args* args, int numIterations, DLTensor* samples_out, DLTensor* momenta_out,
@@ -313,7 +325,8 @@ typedef struct {
  *   moments  float64[2D] device, optional, accumulated: sum q_d, sum q_d^2 over particles and iterations
  *   trace    [D*traceParticles, S] device, optional: kept positions of the first traceParticles local particles,
  *            iteration k in slot traceOffset + k
- * Small-D families, device tensors, leapfrog; every rank of `comm` (NULL: single GPU) must make the same call. */
+ * Small-D families (diagonal / small dense Gaussian, funnel, coin toss, hierarchical normal), device tensors,
+ * leapfrog; every rank of `comm` (NULL: single GPU) must make the same call. */
 EHMC_API int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
                           const ehmc_hmc_args* args, int numIterations, const ehmc_adapt_args* adapt, ehmc_comm* comm,
                           DLTensor* state, DLTensor* history, DLTensor* moments, DLTensor* trace,

@@ -217,7 +217,8 @@ class HMC:
     def _fused_loop_ok(self):
         """Families whose getSamples loop runs as one launch (ehmc_hmc_run)."""
         pot = self.potential
-        return pot.family in (_lib.FAMILY_DIAG_GAUSSIAN, _lib.FAMILY_FUNNEL, _lib.FAMILY_COIN_TOSS) and \
+        return pot.family in (_lib.FAMILY_DIAG_GAUSSIAN, _lib.FAMILY_FUNNEL, _lib.FAMILY_COIN_TOSS,
+                              _lib.FAMILY_HIERARCHICAL_NORMAL) and \
             pot.numDimensions <= 32 or (pot.family == _lib.FAMILY_DENSE_GAUSSIAN and pot.numDimensions <= 16)
 
     # ------------------------------------------------------------------------------------

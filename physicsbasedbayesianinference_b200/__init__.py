@@ -22,6 +22,7 @@ from .potential import (  # noqa: F401
     FunnelPotential,
     GaussianPotential,
     HarmonicPotential,
+    HierarchicalNormalPotential,
     LogisticPotential,
     NBodyPotential,
     Potential,

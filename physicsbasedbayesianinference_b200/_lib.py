@@ -23,6 +23,7 @@ FAMILY_FUNNEL = 3
 FAMILY_NBODY = 4
 FAMILY_LOGISTIC = 5
 FAMILY_COIN_TOSS = 6
+FAMILY_HIERARCHICAL_NORMAL = 7
 LEAPFROG = 0
 STORMER_VERLET = 1
 FLAG_BUGCOMPAT_MOMENTUM = 1

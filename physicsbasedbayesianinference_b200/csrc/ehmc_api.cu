@@ -466,6 +466,48 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
       rc = f32 ? build_logistic<float>(p, a, b, precision) : build_logistic<double>(p, a, b, precision);
       break;
     }
+    case EHMC_FAMILY_HIERARCHICAL_NORMAL: {
+      if ((nparams != 2 && nparams != 3) || nscalars != 4) {
+        rc = fail(EHMC_ERR_INVALID, "hierarchical normal: params = {y[J], sigma[J] [, scale[J+2]]}, scalars = {muLoc, muScale, tauScale, centered}");
+        break;
+      }
+      HierarchicalState& h = p->hier;
+      rc = fetch_param(params[0], "y", 1, &h.y, &v);
+      if (rc) break;
+      rc = fetch_param(params[1], "sigma", 1, &b, &v);
+      if (rc) break;
+      const int J = (int)h.y.size();
+      p->D = J + 2;
+      if (J < 1) { rc = fail(EHMC_ERR_INVALID, "hierarchical normal: empty y"); break; }
+      if (J > 30) { rc = fail(EHMC_ERR_UNSUPPORTED, "hierarchical normal: 1 <= J <= 30 groups (got %d)", J); break; }
+      if ((int)b.size() != J) { rc = fail(EHMC_ERR_INVALID, "hierarchical normal: sigma must have J entries"); break; }
+      h.w.resize(J);
+      for (int j = 0; j < J && rc == EHMC_OK; ++j) {
+        if (!std::isfinite(h.y[j])) rc = fail(EHMC_ERR_INVALID, "hierarchical normal: y must be finite");
+        else if (!(b[j] > 0 && std::isfinite(b[j]))) rc = fail(EHMC_ERR_INVALID, "hierarchical normal: sigma must be > 0");
+        else h.w[j] = 1.0 / (b[j] * b[j]);
+      }
+      if (rc) break;
+      if (nparams == 3 && params[2] != nullptr) {
+        rc = fetch_param(params[2], "scale", 1, &h.scale, &v);
+        if (rc) break;
+        if ((int)h.scale.size() != p->D) { rc = fail(EHMC_ERR_INVALID, "hierarchical normal: scale must have J + 2 entries"); break; }
+        for (double x : h.scale)
+          if (!(x > 0 && std::isfinite(x))) rc = fail(EHMC_ERR_INVALID, "hierarchical normal: scales must be > 0");
+        if (rc) break;
+      } else {
+        h.scale.assign(p->D, 1.0);
+      }
+      h.muLoc = scalars[0];
+      h.muScale = scalars[1];
+      h.tauScale = scalars[2];
+      if (!std::isfinite(h.muLoc)) rc = fail(EHMC_ERR_INVALID, "hierarchical normal: muLoc must be finite");
+      else if (!(h.muScale > 0 && std::isfinite(h.muScale))) rc = fail(EHMC_ERR_INVALID, "hierarchical normal: muScale must be > 0");
+      else if (!(h.tauScale > 0 && std::isfinite(h.tauScale))) rc = fail(EHMC_ERR_INVALID, "hierarchical normal: tauScale must be > 0");
+      else if (scalars[3] != 0.0 && scalars[3] != 1.0) rc = fail(EHMC_ERR_INVALID, "hierarchical normal: centered must be 0 or 1");
+      h.centered = scalars[3] == 1.0;
+      break;
+    }
     default:
       rc = fail(EHMC_ERR_UNSUPPORTED, "potential family %d is not built into this library", family);
   }
@@ -507,7 +549,7 @@ static bool per_particle_stats(const ehmc_ctx* c, const ehmc_potential* p) {
 // families with a register-resident kernel (k_small): the only ones the fused multi-iteration runs cover
 static bool small_family(const ehmc_potential* p) {
   return p->family == EHMC_FAMILY_DIAG_GAUSSIAN || p->family == EHMC_FAMILY_FUNNEL || p->family == EHMC_FAMILY_COIN_TOSS ||
-         (p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->D <= 16);
+         p->family == EHMC_FAMILY_HIERARCHICAL_NORMAL || (p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->D <= 16);
 }
 
 // number of CTAs the trajectory kernel uses for P particles (statistics partials)

@@ -116,6 +116,13 @@ struct NBodyState {
   int b = 0;                        // bodies per particle
 };
 
+struct HierarchicalState {          // hierarchical normal model (make_hier), float64 host tables
+  std::vector<double> y, w;         // y [J], w = 1 / sigma^2 [J]
+  std::vector<double> scale;        // coordinate scale [J + 2] (ones without rescaling)
+  double muLoc = 0.0, muScale = 1.0, tauScale = 1.0;
+  bool centered = false;
+};
+
 struct ehmc_potential {
   ehmc_ctx* ctx = nullptr;
   int family = 0;
@@ -127,6 +134,7 @@ struct ehmc_potential {
   DenseState dense;
   LogisticState logistic;
   NBodyState nbody;
+  HierarchicalState hier;
 };
 
 // peer-memory mailboxes of the fused ensemble run (comm.cu)

@@ -61,6 +61,29 @@ static CoinPot<T, DT> make_coin(const ehmc_potential* p) {
   return f;
 }
 
+// the hierarchical normal model; centred or not is part of the functor's type (HierPot)
+template <typename T, int DT, bool CENTERED>
+static HierPot<T, DT, CENTERED> make_hier(const ehmc_potential* p) {
+  const HierarchicalState& h = p->hier;
+  HierPot<T, DT, CENTERED> f;
+  for (int d = 0; d < DT; ++d) {
+    const bool theta = d >= 2 && d < p->D;
+    f.s[d] = d < p->D ? (T)h.scale[d] : T(0);
+    f.m[d] = theta ? T(1) : T(0);
+    f.w[d] = theta ? (T)h.w[d - 2] : T(0);
+    f.y[d] = theta ? (T)h.y[d - 2] : T(0);
+    f.nwy[d] = theta ? (T)(-h.w[d - 2] * h.y[d - 2]) : T(0);
+  }
+  f.muLoc = (T)h.muLoc;
+  f.invMuS2 = (T)(1.0 / (h.muScale * h.muScale));
+  f.lnTau2 = (T)(2.0 * std::log(h.tauScale));
+  f.invTau2 = (T)(1.0 / (h.tauScale * h.tauScale));
+  f.J = (T)(p->D - 2);
+  f.scaled = false;
+  for (int d = 2; d < p->D; ++d) f.scaled = f.scaled || h.scale[d] != 1.0;
+  return f;
+}
+
 template <typename T, int DT, class Pot>
 static int launch_small_pot(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, int integ, bool hmc, cudaStream_t st) {
   static_assert(K1_THREADS == K1_THREADS_HOST, "K1 block size");
@@ -103,6 +126,11 @@ static int launch_small_dt(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<
     case EHMC_FAMILY_DENSE_GAUSSIAN:
       if constexpr (DT <= 16) return launch_small_pot<T, DT>(c, A, make_dense_small<T, DT>(p), integ, hmc, st);
       break;
+    case EHMC_FAMILY_HIERARCHICAL_NORMAL:  // D = J + 2 >= 3
+      if constexpr (DT >= 4)
+        return p->hier.centered ? launch_small_pot<T, DT>(c, A, make_hier<T, DT, true>(p), integ, hmc, st)
+                                : launch_small_pot<T, DT>(c, A, make_hier<T, DT, false>(p), integ, hmc, st);
+      break;
     default:
       break;
   }
@@ -143,6 +171,11 @@ static int run_small_dt(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>&
     case EHMC_FAMILY_DENSE_GAUSSIAN:
       if constexpr (DT <= 16) return run_small_pot<T, DT>(c, A, make_dense_small<T, DT>(p), integ, R, st);
       break;
+    case EHMC_FAMILY_HIERARCHICAL_NORMAL:
+      if constexpr (DT >= 4)
+        return p->hier.centered ? run_small_pot<T, DT>(c, A, make_hier<T, DT, true>(p), integ, R, st)
+                                : run_small_pot<T, DT>(c, A, make_hier<T, DT, false>(p), integ, R, st);
+      break;
     default: break;
   }
   return fail(EHMC_ERR_UNSUPPORTED, "family %d has no fused multi-iteration kernel for D = %d", p->family, p->D);
@@ -174,6 +207,15 @@ static int eval_small_dt(ehmc_ctx* c, const ehmc_potential* p, const T* q, long 
     case EHMC_FAMILY_COIN_TOSS:
       k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_coin<T, DT>(p));
       break;
+    case EHMC_FAMILY_HIERARCHICAL_NORMAL:
+      if constexpr (DT >= 4) {
+        if (p->hier.centered)
+          k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_hier<T, DT, true>(p));
+        else
+          k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_hier<T, DT, false>(p));
+        break;
+      }
+      return fail(EHMC_ERR_UNSUPPORTED, "eval: family %d", p->family);
     default:
       return fail(EHMC_ERR_UNSUPPORTED, "eval: family %d", p->family);
   }

@@ -111,6 +111,11 @@ static int ens_dt(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, co
     case EHMC_FAMILY_DENSE_GAUSSIAN:
       if constexpr (DT <= 16) return ens_pot<T, DT>(c, A, make_dense_small<T, DT>(p), R, st);
       break;
+    case EHMC_FAMILY_HIERARCHICAL_NORMAL:
+      if constexpr (DT >= 4)
+        return p->hier.centered ? ens_pot<T, DT>(c, A, make_hier<T, DT, true>(p), R, st)
+                                : ens_pot<T, DT>(c, A, make_hier<T, DT, false>(p), R, st);
+      break;
     default: break;
   }
   return fail(EHMC_ERR_UNSUPPORTED, "family %d has no fused ensemble-run kernel for D = %d", p->family, p->D);

@@ -11,7 +11,8 @@ from __future__ import annotations
 
 import numpy as np
 
-from .potential import CoinTossPotential, FunnelPotential, GaussianPotential, HarmonicPotential, LogisticPotential
+from .potential import (CoinTossPotential, FunnelPotential, GaussianPotential, HarmonicPotential,
+                        HierarchicalNormalPotential, LogisticPotential)
 
 
 def potentialFromSpec(spec):
@@ -19,7 +20,8 @@ def potentialFromSpec(spec):
 
     families: "normal_iid" (scale per dim), "mvn" (mean, cov | precision),
     "funnel" (numDimensions, sigmaV), "coin_toss" (observations | successes, trials),
-    "logistic_regression" (X, y, priorScale)."""
+    "logistic_regression" (X, y, priorScale),
+    "hierarchical_normal" (y, sigma, muLoc, muScale, tauScale, centered)."""
     fam = spec.get("family")
     if fam == "normal_iid":
         scale = np.atleast_1d(np.asarray(spec["scale"], dtype=np.float64))
@@ -37,8 +39,13 @@ def potentialFromSpec(spec):
     if fam == "logistic_regression":
         return LogisticPotential(spec["X"], spec["y"], float(spec.get("priorScale", 1.0)),
                                  precision=spec.get("precision", "fp32"))
+    if fam == "hierarchical_normal":  # eight schools: HierarchicalNormalPotential.eightSchools()
+        return HierarchicalNormalPotential(spec["y"], spec["sigma"], float(spec.get("muLoc", 0.0)),
+                                           float(spec.get("muScale", 5.0)), float(spec.get("tauScale", 5.0)),
+                                           spec.get("centered", False))
     raise NotImplementedError(
-        f"model family {fam!r} has no fused CUDA kernel; supported: normal_iid, mvn, funnel, coin_toss, logistic_regression")
+        f"model family {fam!r} has no fused CUDA kernel; supported: normal_iid, mvn, funnel, coin_toss, "
+        "logistic_regression, hierarchical_normal")
 
 
 def logisticSpecFromLinearLogits(logits_of, numDimensions, y, priorScale, rtol=1e-6):

@@ -200,6 +200,90 @@ class CoinTossPotential(Potential):
         return [self.successes, self.trials]
 
 
+class HierarchicalNormalPotential(Potential):
+    """The normal-normal hierarchical model (NumPyro's eight-schools example):
+
+        mu ~ N(muLoc, muScale^2),  tau ~ HalfCauchy(tauScale),  theta_j ~ N(mu, tau^2),  y_j ~ N(theta_j, sigma_j^2)
+
+    with J groups and known sigma_j, sampled in NumPyro's unconstrained coordinates (D = J + 2):
+    q[0] = mu, q[1] = eta = ln tau, q[2 + j] = theta_j (centered=True) or thetaTilde_j with
+    theta_j = mu + tau thetaTilde_j (centered=False, the non-centred form that has no funnel in (eta, theta)).
+    U(q) is minus the log posterior density, Jacobian of eta included, additive constants dropped.
+
+    scale: the same potential in rescaled coordinates, U'(q) = U(scale * q) -- what mass adaptation produces
+    (Potential.rescaled)."""
+
+    family = _lib.FAMILY_HIERARCHICAL_NORMAL
+
+    EIGHT_SCHOOLS_Y = (28.0, 8.0, -3.0, 7.0, -1.0, 1.0, 18.0, 12.0)
+    EIGHT_SCHOOLS_SIGMA = (15.0, 10.0, 16.0, 11.0, 9.0, 11.0, 10.0, 18.0)
+
+    def __init__(self, y, sigma, muLoc=0.0, muScale=5.0, tauScale=5.0, centered=False, scale=None):
+        self.y = np.atleast_1d(np.asarray(y, dtype=np.float64)).copy()
+        self.sigma = np.atleast_1d(np.asarray(sigma, dtype=np.float64)).copy()
+        if self.y.ndim != 1 or self.sigma.shape != self.y.shape:
+            raise ValueError("y and sigma must be 1-D with one entry per group")
+        J = self.y.shape[0]
+        if not 1 <= J <= 30:
+            raise ValueError(f"the hierarchical normal kernels take 1 <= J <= 30 groups (got {J})")
+        if not np.all(np.isfinite(self.y)):
+            raise ValueError("y must be finite")
+        if not np.all((self.sigma > 0) & np.isfinite(self.sigma)):
+            raise ValueError("sigma must be > 0")
+        self.muLoc, self.muScale, self.tauScale = float(muLoc), float(muScale), float(tauScale)
+        if not np.isfinite(self.muLoc):
+            raise ValueError("muLoc must be finite")
+        if not (self.muScale > 0 and np.isfinite(self.muScale) and self.tauScale > 0 and np.isfinite(self.tauScale)):
+            raise ValueError("muScale and tauScale must be > 0")
+        if centered not in (True, False, 0, 1):
+            raise ValueError("centered must be True or False")
+        self.centered = bool(centered)
+        self.scale = None if scale is None else np.asarray(scale, dtype=np.float64).copy()
+        if self.scale is not None and (self.scale.shape != (J + 2,) or not np.all((self.scale > 0) & np.isfinite(self.scale))):
+            raise ValueError("scale must hold J + 2 entries > 0")
+        super().__init__(J + 2)
+
+    @classmethod
+    def eightSchools(cls, centered=False):
+        """The eight-schools data and priors of NumPyro's example (muLoc 0, muScale 5, tauScale 5)."""
+        return cls(cls.EIGHT_SCHOOLS_Y, cls.EIGHT_SCHOOLS_SIGMA, 0.0, 5.0, 5.0, centered)
+
+    def _params(self):
+        return [self.y, self.sigma] + ([] if self.scale is None else [self.scale])
+
+    def _scalars(self):
+        return [self.muLoc, self.muScale, self.tauScale, 1.0 if self.centered else 0.0]
+
+    def rescaled(self, scales):
+        s = np.asarray(scales, dtype=np.float64)
+        base = np.ones(self.numDimensions) if self.scale is None else self.scale
+        return HierarchicalNormalPotential(self.y, self.sigma, self.muLoc, self.muScale, self.tauScale, self.centered,
+                                           scale=base * s)
+
+    def modelParameters(self, q):
+        """dict(mu, tau, theta) of positions q in this descriptor's coordinates: q is a NumPy array or a torch
+        tensor of shape (D,), (D, P) or (D, P, S); mu and tau have q's shape without the first axis, theta has
+        (J,) + that shape."""
+        s = np.ones(self.numDimensions) if self.scale is None else self.scale
+        if hasattr(q, "is_cuda"):  # torch
+            import torch
+
+            exp = torch.exp
+            sv = torch.as_tensor(s, dtype=q.dtype, device=q.device)
+        else:
+            q = np.asarray(q, dtype=np.float64)
+            exp = np.exp
+            sv = s
+        if q.shape[0] != self.numDimensions:
+            raise ValueError(f"q must have {self.numDimensions} rows (mu, eta, J group effects)")
+        st = sv[2:].reshape((-1,) + (1,) * (q.ndim - 1))
+        mu = sv[0] * q[0]
+        tau = exp(sv[1] * q[1])
+        x = st * q[2:]
+        theta = x if self.centered else mu + tau * x
+        return dict(mu=mu, tau=tau, theta=theta)
+
+
 class NBodyPotential(Potential):
     """Every ensemble particle is a whole B-body system; coordinates are flattened
     component-major, d = c*B + b (the reference's own convention, src/potential.py:83-84).
