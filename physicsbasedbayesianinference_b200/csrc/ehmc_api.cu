@@ -374,7 +374,6 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
   p->ctx = ctx;
   p->family = family;
   p->bits = dtype_bits;
-  p->scalars.assign(scalars, scalars + nscalars);
   const bool f32 = dtype_bits == 32;
   int rc = EHMC_OK;
   View v;
@@ -396,7 +395,7 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
       } else if (p->D > 128) {
         rc = fail(EHMC_ERR_UNSUPPORTED, "diag gaussian: D = %d > 128 not built", p->D);
       } else {
-        p->diag_k.swap(a);
+        p->diag.k.swap(a);
       }
       break;
     }
@@ -420,21 +419,28 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
       if (nscalars != 2 && nscalars != 4) { rc = fail(EHMC_ERR_INVALID, "funnel: scalars = {D, sigma_v [, scaleV, scaleX]}"); break; }
       p->D = (int)scalars[0];
       if (p->D < 2 || p->D > 32) { rc = fail(EHMC_ERR_UNSUPPORTED, "funnel: 2 <= D <= 32 (got %d)", p->D); break; }
-      if (!(scalars[1] > 0)) rc = fail(EHMC_ERR_INVALID, "funnel: sigma_v must be > 0");
-      else if (nscalars == 4 && !(scalars[2] > 0 && scalars[3] > 0)) rc = fail(EHMC_ERR_INVALID, "funnel: scales must be > 0");
+      FunnelState& s = p->funnel;
+      s.sigmaV = scalars[1];
+      if (nscalars == 4) {
+        s.scaleV = scalars[2];
+        s.scaleX = scalars[3];
+      }
+      if (!(s.sigmaV > 0)) rc = fail(EHMC_ERR_INVALID, "funnel: sigma_v must be > 0");
+      else if (!(s.scaleV > 0 && s.scaleX > 0)) rc = fail(EHMC_ERR_INVALID, "funnel: scales must be > 0");
       break;
     }
     case EHMC_FAMILY_COIN_TOSS: {
       if (nparams != 2) { rc = fail(EHMC_ERR_INVALID, "coin toss: params = {successes[D], trials[D]}"); break; }
-      rc = fetch_param(params[0], "successes", 1, &p->coin_k, &v);
+      CoinState& s = p->coin;
+      rc = fetch_param(params[0], "successes", 1, &s.k, &v);
       if (rc) break;
-      rc = fetch_param(params[1], "trials", 1, &p->coin_n, &v);
+      rc = fetch_param(params[1], "trials", 1, &s.n, &v);
       if (rc) break;
-      p->D = (int)p->coin_k.size();
+      p->D = (int)s.k.size();
       if (p->D < 1 || p->D > 32) { rc = fail(EHMC_ERR_UNSUPPORTED, "coin toss: 1 <= D <= 32 (got %d)", p->D); break; }
-      if ((int)p->coin_n.size() != p->D) { rc = fail(EHMC_ERR_INVALID, "coin toss: trials must have D entries"); break; }
+      if ((int)s.n.size() != p->D) { rc = fail(EHMC_ERR_INVALID, "coin toss: trials must have D entries"); break; }
       for (int d = 0; d < p->D && rc == EHMC_OK; ++d)
-        if (!(p->coin_k[d] >= 0 && p->coin_n[d] >= p->coin_k[d])) rc = fail(EHMC_ERR_INVALID, "coin toss: need 0 <= successes <= trials");
+        if (!(s.k[d] >= 0 && s.n[d] >= s.k[d])) rc = fail(EHMC_ERR_INVALID, "coin toss: need 0 <= successes <= trials");
       break;
     }
     case EHMC_FAMILY_NBODY: {
@@ -445,7 +451,9 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
       p->D = 3 * B;
       if (B < 1) { rc = fail(EHMC_ERR_INVALID, "nbody: empty bodyMass"); break; }
       if (B > 7000) { rc = fail(EHMC_ERR_UNSUPPORTED, "nbody: B = %d > 7000 bodies", B); break; }
-      if (!(scalars[1] >= 0)) { rc = fail(EHMC_ERR_INVALID, "nbody: eps must be >= 0"); break; }
+      p->nbody.G = scalars[0];
+      p->nbody.eps = scalars[1];
+      if (!(p->nbody.eps >= 0)) { rc = fail(EHMC_ERR_INVALID, "nbody: eps must be >= 0"); break; }
       rc = f32 ? build_nbody<float>(p, a) : build_nbody<double>(p, a);
       break;
     }
@@ -459,7 +467,8 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
       if (rc) break;
       if ((int)b.size() != p->logistic.n) { rc = fail(EHMC_ERR_INVALID, "logistic: y must have N entries"); break; }
       if (p->D < 1 || p->D > 256) { rc = fail(EHMC_ERR_UNSUPPORTED, "logistic: 1 <= D <= 256 (got %d)", p->D); break; }
-      if (!(scalars[0] > 0)) { rc = fail(EHMC_ERR_INVALID, "logistic: priorScale must be > 0"); break; }
+      p->logistic.priorScale = scalars[0];
+      if (!(p->logistic.priorScale > 0)) { rc = fail(EHMC_ERR_INVALID, "logistic: priorScale must be > 0"); break; }
       const int precision = nscalars == 2 ? (int)scalars[1] : 0;
       if (precision < 0 || precision > 3) { rc = fail(EHMC_ERR_INVALID, "logistic: precision selector must be 0 (CUDA cores), 1 (bf16), 2 (fp16 split) or 3 (auto)"); break; }
       if ((precision == 1 || precision == 2) && !f32) { rc = fail(EHMC_ERR_INVALID, "logistic: the tensor-core path needs float32 state"); break; }
@@ -544,12 +553,6 @@ static bool per_particle_stats(const ehmc_ctx* c, const ehmc_potential* p) {
   if (p->family == EHMC_FAMILY_NBODY || p->family == EHMC_FAMILY_LOGISTIC) return true;
   // the 3xFP16 tensor-core dense kernel reports per-particle scalars too
   return use_dense_tc(c, p);
-}
-
-// families with a register-resident kernel (k_small): the only ones the fused multi-iteration runs cover
-static bool small_family(const ehmc_potential* p) {
-  return p->family == EHMC_FAMILY_DIAG_GAUSSIAN || p->family == EHMC_FAMILY_FUNNEL || p->family == EHMC_FAMILY_COIN_TOSS ||
-         p->family == EHMC_FAMILY_HIERARCHICAL_NORMAL || (p->family == EHMC_FAMILY_DENSE_GAUSSIAN && p->D <= 16);
 }
 
 // number of CTAs the trajectory kernel uses for P particles (statistics partials)
@@ -897,7 +900,7 @@ extern "C" int ehmc_hmc_iter(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor*
   if (a->dynamic != nullptr) {
     // only kernels that resolve the block themselves; everything else would silently use the host values
     const bool tc3 = v.bits == 32 && use_dense_tc(ctx, pot);
-    if (v.q.host || !(small_family(pot) || tc3))
+    if (v.q.host || !(has_small_kernel(pot) || tc3))
       return fail(EHMC_ERR_UNSUPPORTED, "%s: args.dynamic needs device tensors and a small-D or float32 dense (tensor-core) potential", fn);
   }
   if (v.bits == 32) {
@@ -939,7 +942,7 @@ extern "C" int ehmc_hmc_run(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* 
   CallViews v;
   TRY(common_checks(ctx, pot, q, mass, &v, fn));
   TRY(check_hmc_args(HmcEntry::run, fn, a, nullptr, numIterations < 0 || sampleOffset < 0));
-  if (v.q.host || !small_family(pot))
+  if (v.q.host || !has_small_kernel(pot))
     return fail(EHMC_ERR_UNSUPPORTED, "%s: device tensors and a small-D potential family are required", fn);
   View vs, vm, va;
   long long S = 0;
@@ -984,7 +987,7 @@ extern "C" int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, D
   TRY(common_checks(ctx, pot, q, mass, &v, fn));
   if (!a || !ad || !state) return fail(EHMC_ERR_INVALID, "%s: args, adapt and state are required", fn);
   TRY(check_hmc_args(HmcEntry::ensemble, fn, a, ad, numIterations < 0 || traceParticles < 0 || traceOffset < 0));
-  if (v.q.host || !small_family(pot))
+  if (v.q.host || !has_small_kernel(pot))
     return fail(EHMC_ERR_UNSUPPORTED, "%s: device tensors and a small-D potential family are required", fn);
   if (!(ad->numParticlesTotal > 0) || !(ad->minStep > 0) || !(ad->maxStep >= ad->minStep))
     return fail(EHMC_ERR_INVALID, "%s: bad adaptation scalars", fn);

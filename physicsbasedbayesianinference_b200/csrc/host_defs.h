@@ -95,11 +95,12 @@ struct DenseState {                 // dense Gaussian (and the diagonal family f
   } tc3;
 };
 
-// gradient kernel of the logistic family: the values of the precision selector (scalars[1]) but auto (3)
+// gradient kernel of the logistic family: the values of the precision selector (its second scalar) but auto (3)
 enum LogisticKernel { LOGISTIC_EXACT = 0, LOGISTIC_BF16 = 1, LOGISTIC_FP16X3 = 2 };
 
 struct LogisticState {
   int n = 0;                        // data rows
+  double priorScale = 1.0;          // s of the Gaussian prior N(0, s^2 I) on the coefficients
   LogisticKernel kernel = LOGISTIC_EXACT;  // resolved from the selector (auto decides here, once)
   void* x = nullptr;                // exact kernel: X [N][D]
   void* y = nullptr;                // exact kernel: y [N]
@@ -114,6 +115,19 @@ struct LogisticState {
 struct NBodyState {
   void* body_mass = nullptr;        // [B]
   int b = 0;                        // bodies per particle
+  double G = 0.0, eps = 0.0;        // gravitational constant, softening length (eps = 0: the unsoftened kernel)
+};
+
+struct DiagState {                  // diagonal Gaussian, D <= 32 (make_diag)
+  std::vector<double> k;
+};
+
+struct CoinState {                  // coin toss (make_coin)
+  std::vector<double> k, n;         // successes, trials
+};
+
+struct FunnelState {                // the funnel of v = scaleV q[0], x_k = scaleX q[k] (make_funnel)
+  double sigmaV = 1.0, scaleV = 1.0, scaleX = 1.0;
 };
 
 struct HierarchicalState {          // hierarchical normal model (make_hier), float64 host tables
@@ -128,9 +142,9 @@ struct ehmc_potential {
   int family = 0;
   int D = 0;
   int bits = 32;
-  std::vector<double> scalars;
-  std::vector<double> diag_k;                    // diagonal Gaussian, D <= 32 (make_diag)
-  std::vector<double> coin_k, coin_n;            // coin toss: successes, trials (make_coin)
+  DiagState diag;
+  CoinState coin;
+  FunnelState funnel;
   DenseState dense;
   LogisticState logistic;
   NBodyState nbody;
@@ -176,6 +190,9 @@ int pack_logistic_tc(ehmc_potential* p, const std::vector<double>& X, const std:
 template <typename T>
 int build_nbody(ehmc_potential* p, const std::vector<double>& body_mass);
 
+// whether p has a register-resident kernel (with_small_pot, inst_small.cuh): the only potentials the fused
+// multi-iteration runs cover
+bool has_small_kernel(const ehmc_potential* p);
 // fused trajectory kernels, D <= 32 register-resident families
 template <typename T>
 int launch_small(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, bool hmc, cudaStream_t st);

@@ -14,7 +14,7 @@ static LogisticArgs<T> logistic_args(const ehmc_potential* p) {
   pa.y = static_cast<const T*>(p->logistic.y);
   pa.N = p->logistic.n;
   pa.D = p->D;
-  pa.inv_s2 = (T)(1.0 / (p->scalars[0] * p->scalars[0]));
+  pa.inv_s2 = (T)(1.0 / (p->logistic.priorScale * p->logistic.priorScale));
   return pa;
 }
 

@@ -114,7 +114,7 @@ int logistic_grad_tc(ehmc_ctx* c, const ehmc_potential* p, const float* theta, l
   pa.D = p->D;
   pa.n_pad = s.chunks.npad;
   pa.chunk_bytes = s.chunks.bytes;
-  pa.inv_s2 = (float)(1.0 / (p->scalars[0] * p->scalars[0]));
+  pa.inv_s2 = (float)(1.0 / (s.priorScale * s.priorScale));
   const size_t fixed = 2 * LT_M * 8 + (2 * LT_MAX_STAGES + 5) * 8 + 16;
   pa.stages = (int)std::min<size_t>(LT_MAX_STAGES, (227 * 1024 - fixed) / pa.chunk_bytes);
   if (pa.stages < 2) return fail(EHMC_ERR_UNSUPPORTED, "logistic tensor-core kernel: chunk of %u B does not fit twice", pa.chunk_bytes);
@@ -134,7 +134,7 @@ int logistic_grad_tcs(ehmc_ctx* c, const ehmc_potential* p, const float* theta, 
   pa.D = p->D;
   pa.n_pad = s.chunks.npad;
   pa.entry_bytes = s.chunks.bytes;
-  pa.inv_s2 = (float)(1.0 / (p->scalars[0] * p->scalars[0]));
+  pa.inv_s2 = (float)(1.0 / (s.priorScale * s.priorScale));
   pa.x_iscale = s.chunks.x_iscale;
   const size_t fixed = (size_t)pa.DP * LT_M * 2 + (2 * LT_MAX_STAGES + 6) * 8 + 16;  // Theta_lo + barriers + TMEM slot
   pa.stages = (int)std::min<size_t>(LT_MAX_STAGES, (227 * 1024 - fixed) / pa.entry_bytes);

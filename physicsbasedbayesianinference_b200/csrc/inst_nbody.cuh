@@ -16,8 +16,8 @@ static NBodyArgs<T> nbody_args(const ehmc_potential* p) {
   NBodyArgs<T> pa;
   pa.bmass = static_cast<const T*>(p->nbody.body_mass);
   pa.B = p->nbody.b;
-  pa.G = (T)p->scalars[0];
-  pa.eps2 = (T)(p->scalars[1] * p->scalars[1]);
+  pa.G = (T)p->nbody.G;
+  pa.eps2 = (T)(p->nbody.eps * p->nbody.eps);
   pa.fcache = nullptr;
   pa.ucache = nullptr;
   pa.cache_read = 0;
@@ -44,7 +44,7 @@ static int launch_nbody_ti(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<
     pa.cache_read = hit ? 1 : 0;
   }
   c->ep_valid = false;
-  const bool eps0 = p->scalars[1] == 0.0;
+  const bool eps0 = p->nbody.eps == 0.0;
   void (*k)(const IterArgs<T>, const NBodyArgs<T>, const int, const int);
   if (nt <= 128)
     k = eps0 ? k_nbody<T, true, 128, TI> : k_nbody<T, false, 128, TI>;
@@ -83,7 +83,7 @@ int eval_nbody(ehmc_ctx* c, const ehmc_potential* p, const T* q, long long q_ld,
   const size_t sm = (size_t)B * 4 * sizeof(T) + 40 * sizeof(T);
   if (sm > 227 * 1024) return fail(EHMC_ERR_UNSUPPORTED, "nbody: B = %d needs %zu B shared memory", B, sm);
   const NBodyArgs<T> pa = nbody_args<T>(p);
-  auto k = p->scalars[1] == 0.0 ? k_nbody_eval<T, true> : k_nbody_eval<T, false>;
+  auto k = p->nbody.eps == 0.0 ? k_nbody_eval<T, true> : k_nbody_eval<T, false>;
   CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
   k<<<(unsigned)P, nt, sm, st>>>(q, q_ld, e, g, g_ld, pa);
   c->launches++;

@@ -2,6 +2,7 @@
 #pragma once
 
 #include <algorithm>
+#include <type_traits>
 
 #include "host_defs.h"
 #include "k_misc.cuh"
@@ -12,7 +13,7 @@ namespace ehmc {
 template <typename T, int DT>
 static DiagPot<T, DT> make_diag(const ehmc_potential* p) {
   DiagPot<T, DT> f;
-  for (int d = 0; d < DT; ++d) f.k[d] = d < p->D ? (T)p->diag_k[d] : T(0);
+  for (int d = 0; d < DT; ++d) f.k[d] = d < p->D ? (T)p->diag.k[d] : T(0);
   return f;
 }
 template <typename T, int DT>
@@ -26,13 +27,12 @@ static DenseSmallPot<T, DT> make_dense_small(const ehmc_potential* p) {
 }
 template <typename T, int DT>
 static FunnelPot<T, DT> make_funnel(const ehmc_potential* p) {
+  const FunnelState& s = p->funnel;
   FunnelPot<T, DT> f;
-  // scalars {D, sigma_v [, scaleV, scaleX]}: the funnel of v = scaleV q[0], x_k = scaleX q[k]
-  const double a = p->scalars.size() >= 4 ? p->scalars[2] : 1.0, cx = p->scalars.size() >= 4 ? p->scalars[3] : 1.0;
-  f.inv_s2 = (T)(a * a / (p->scalars[1] * p->scalars[1]));
-  f.half_dm1 = (T)(0.5 * a * (p->D - 1));
-  f.a = (T)a;
-  f.lnb = (T)(2.0 * std::log(cx));
+  f.inv_s2 = (T)(s.scaleV * s.scaleV / (s.sigmaV * s.sigmaV));
+  f.half_dm1 = (T)(0.5 * s.scaleV * (p->D - 1));
+  f.a = (T)s.scaleV;
+  f.lnb = (T)(2.0 * std::log(s.scaleX));
   return f;
 }
 
@@ -53,10 +53,11 @@ static int small_grid(ehmc_ctx* c, K kernel, size_t sm, long long P, unsigned* g
 
 template <typename T, int DT>
 static CoinPot<T, DT> make_coin(const ehmc_potential* p) {
+  const CoinState& s = p->coin;
   CoinPot<T, DT> f;
   for (int d = 0; d < DT; ++d) {
-    f.k[d] = d < p->D ? (T)p->coin_k[d] : T(0);
-    f.nk[d] = d < p->D ? (T)(p->coin_n[d] - p->coin_k[d]) : T(0);
+    f.k[d] = d < p->D ? (T)s.k[d] : T(0);
+    f.nk[d] = d < p->D ? (T)(s.n[d] - s.k[d]) : T(0);
   }
   return f;
 }
@@ -84,157 +85,105 @@ static HierPot<T, DT, CENTERED> make_hier(const ehmc_potential* p) {
   return f;
 }
 
-template <typename T, int DT, class Pot>
-static int launch_small_pot(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, int integ, bool hmc, cudaStream_t st) {
-  static_assert(K1_THREADS == K1_THREADS_HOST, "K1 block size");
-  // statistics: per-warp value tiles + per-warp rows (WarpStats, k_small.cuh)
-  const size_t sm = A.partials != nullptr ? WarpStats<T, DT>::kSmemBytes : 0;
-  unsigned grid = 1;
-  auto go = [&](auto kernel) -> int {
-    TRY(small_grid(c, kernel, sm, A.P, &grid));
-    kernel<<<grid, K1_THREADS, sm, st>>>(A, pot);
-    return EHMC_OK;
+// The register-resident functor of p at its kernel width DT, the least of 2, 4, 8, 10, 16, 32 that holds p->D, handed
+// to f(std::integral_constant<int, DT>(), pot).  The dense family has one up to DT = 16 (above, k_dense), the
+// hierarchical model from DT = 4 (D = J + 2 >= 3).  Without one: EHMC_ERR_UNSUPPORTED, with the message "family F has
+// no <what> for D = N" unless `what` is null.
+template <typename T, class F>
+static int with_small_pot(const ehmc_potential* p, const char* what, F&& f) {
+  auto none = [&]() -> int {
+    return what ? fail(EHMC_ERR_UNSUPPORTED, "family %d has no %s for D = %d", p->family, what, p->D) : EHMC_ERR_UNSUPPORTED;
   };
-  const bool exact = A.D == DT;  // no padded dimensions: the kernel without the per-dimension bounds tests
-  if (hmc) {
-    if (integ == INTEG_LEAPFROG)
-      TRY(exact ? go(k_small<T, DT, Pot, INTEG_LEAPFROG, true, true>) : go(k_small<T, DT, Pot, INTEG_LEAPFROG, true, false>));
-    else
-      TRY(exact ? go(k_small<T, DT, Pot, INTEG_STORMER, true, true>) : go(k_small<T, DT, Pot, INTEG_STORMER, true, false>));
-  } else {
-    if (integ == INTEG_LEAPFROG)
-      TRY(exact ? go(k_small<T, DT, Pot, INTEG_LEAPFROG, false, true>) : go(k_small<T, DT, Pot, INTEG_LEAPFROG, false, false>));
-    else
-      TRY(exact ? go(k_small<T, DT, Pot, INTEG_STORMER, false, true>) : go(k_small<T, DT, Pot, INTEG_STORMER, false, false>));
-  }
-  c->launches++;
-  c->last_rows = grid;  // statistics partials: one row per CTA actually launched
-  CUDA_TRY(cudaGetLastError());
-  return EHMC_OK;
-}
-
-template <typename T, int DT>
-static int launch_small_dt(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, bool hmc,
-                           cudaStream_t st) {
-  switch (p->family) {
-    case EHMC_FAMILY_DIAG_GAUSSIAN:
-      return launch_small_pot<T, DT>(c, A, make_diag<T, DT>(p), integ, hmc, st);
-    case EHMC_FAMILY_FUNNEL:
-      return launch_small_pot<T, DT>(c, A, make_funnel<T, DT>(p), integ, hmc, st);
-    case EHMC_FAMILY_COIN_TOSS:
-      return launch_small_pot<T, DT>(c, A, make_coin<T, DT>(p), integ, hmc, st);
-    case EHMC_FAMILY_DENSE_GAUSSIAN:
-      if constexpr (DT <= 16) return launch_small_pot<T, DT>(c, A, make_dense_small<T, DT>(p), integ, hmc, st);
-      break;
-    case EHMC_FAMILY_HIERARCHICAL_NORMAL:  // D = J + 2 >= 3
-      if constexpr (DT >= 4)
-        return p->hier.centered ? launch_small_pot<T, DT>(c, A, make_hier<T, DT, true>(p), integ, hmc, st)
-                                : launch_small_pot<T, DT>(c, A, make_hier<T, DT, false>(p), integ, hmc, st);
-      break;
-    default:
-      break;
-  }
-  return fail(EHMC_ERR_UNSUPPORTED, "family %d has no small-D kernel for D = %d", p->family, p->D);
+  auto at = [&](auto dt) -> int {
+    constexpr int DT = decltype(dt)::value;
+    switch (p->family) {
+      case EHMC_FAMILY_DIAG_GAUSSIAN: return f(dt, make_diag<T, DT>(p));
+      case EHMC_FAMILY_FUNNEL: return f(dt, make_funnel<T, DT>(p));
+      case EHMC_FAMILY_COIN_TOSS: return f(dt, make_coin<T, DT>(p));
+      case EHMC_FAMILY_DENSE_GAUSSIAN:
+        if constexpr (DT <= 16) return f(dt, make_dense_small<T, DT>(p));
+        break;
+      case EHMC_FAMILY_HIERARCHICAL_NORMAL:
+        if constexpr (DT >= 4) return p->hier.centered ? f(dt, make_hier<T, DT, true>(p)) : f(dt, make_hier<T, DT, false>(p));
+        break;
+      default: break;
+    }
+    return none();
+  };
+  const int D = p->D;
+  if (D <= 2) return at(std::integral_constant<int, 2>());
+  if (D <= 4) return at(std::integral_constant<int, 4>());
+  if (D <= 8) return at(std::integral_constant<int, 8>());
+  if (D <= 10) return at(std::integral_constant<int, 10>());
+  if (D <= 16) return at(std::integral_constant<int, 16>());
+  if (D <= 32) return at(std::integral_constant<int, 32>());
+  return none();
 }
 
 template <typename T>
 int launch_small(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, bool hmc, cudaStream_t st) {
-  const int D = p->D;
-  if (D <= 2) return launch_small_dt<T, 2>(c, p, A, integ, hmc, st);
-  if (D <= 4) return launch_small_dt<T, 4>(c, p, A, integ, hmc, st);
-  if (D <= 8) return launch_small_dt<T, 8>(c, p, A, integ, hmc, st);
-  if (D <= 10) return launch_small_dt<T, 10>(c, p, A, integ, hmc, st);
-  if (D <= 16) return launch_small_dt<T, 16>(c, p, A, integ, hmc, st);
-  if (D <= 32) return launch_small_dt<T, 32>(c, p, A, integ, hmc, st);
-  return fail(EHMC_ERR_UNSUPPORTED, "small-D kernel: D = %d > 32", D);
-}
-
-template <typename T, int DT, class Pot>
-static int run_small_pot(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, int integ, const RunArgs<T>& R, cudaStream_t st) {
-  const unsigned grid = (unsigned)std::max<long long>(1, (A.P + K1_THREADS - 1) / K1_THREADS);
-  if (integ == INTEG_LEAPFROG)
-    k_small_run<T, DT, Pot, INTEG_LEAPFROG><<<grid, K1_THREADS, 0, st>>>(A, pot, R);
-  else
-    k_small_run<T, DT, Pot, INTEG_STORMER><<<grid, K1_THREADS, 0, st>>>(A, pot, R);
-  c->launches++;
-  CUDA_TRY(cudaGetLastError());
-  return EHMC_OK;
-}
-
-template <typename T, int DT>
-static int run_small_dt(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, const RunArgs<T>& R,
-                        cudaStream_t st) {
-  switch (p->family) {
-    case EHMC_FAMILY_DIAG_GAUSSIAN: return run_small_pot<T, DT>(c, A, make_diag<T, DT>(p), integ, R, st);
-    case EHMC_FAMILY_FUNNEL: return run_small_pot<T, DT>(c, A, make_funnel<T, DT>(p), integ, R, st);
-    case EHMC_FAMILY_COIN_TOSS: return run_small_pot<T, DT>(c, A, make_coin<T, DT>(p), integ, R, st);
-    case EHMC_FAMILY_DENSE_GAUSSIAN:
-      if constexpr (DT <= 16) return run_small_pot<T, DT>(c, A, make_dense_small<T, DT>(p), integ, R, st);
-      break;
-    case EHMC_FAMILY_HIERARCHICAL_NORMAL:
-      if constexpr (DT >= 4)
-        return p->hier.centered ? run_small_pot<T, DT>(c, A, make_hier<T, DT, true>(p), integ, R, st)
-                                : run_small_pot<T, DT>(c, A, make_hier<T, DT, false>(p), integ, R, st);
-      break;
-    default: break;
-  }
-  return fail(EHMC_ERR_UNSUPPORTED, "family %d has no fused multi-iteration kernel for D = %d", p->family, p->D);
+  static_assert(K1_THREADS == K1_THREADS_HOST, "K1 block size");
+  return with_small_pot<T>(p, "small-D kernel", [&](auto dt, const auto& pot) -> int {
+    constexpr int DT = decltype(dt)::value;
+    using Pot = std::decay_t<decltype(pot)>;
+    // statistics: per-warp value tiles + per-warp rows (WarpStats, k_small.cuh)
+    const size_t sm = A.partials != nullptr ? WarpStats<T, DT>::kSmemBytes : 0;
+    unsigned grid = 1;
+    auto go = [&](auto kernel) -> int {
+      TRY(small_grid(c, kernel, sm, A.P, &grid));
+      kernel<<<grid, K1_THREADS, sm, st>>>(A, pot);
+      return EHMC_OK;
+    };
+    const bool exact = A.D == DT;  // no padded dimensions: the kernel without the per-dimension bounds tests
+    if (hmc) {
+      if (integ == INTEG_LEAPFROG)
+        TRY(exact ? go(k_small<T, DT, Pot, INTEG_LEAPFROG, true, true>) : go(k_small<T, DT, Pot, INTEG_LEAPFROG, true, false>));
+      else
+        TRY(exact ? go(k_small<T, DT, Pot, INTEG_STORMER, true, true>) : go(k_small<T, DT, Pot, INTEG_STORMER, true, false>));
+    } else {
+      if (integ == INTEG_LEAPFROG)
+        TRY(exact ? go(k_small<T, DT, Pot, INTEG_LEAPFROG, false, true>) : go(k_small<T, DT, Pot, INTEG_LEAPFROG, false, false>));
+      else
+        TRY(exact ? go(k_small<T, DT, Pot, INTEG_STORMER, false, true>) : go(k_small<T, DT, Pot, INTEG_STORMER, false, false>));
+    }
+    c->launches++;
+    c->last_rows = grid;  // statistics partials: one row per CTA actually launched
+    CUDA_TRY(cudaGetLastError());
+    return EHMC_OK;
+  });
 }
 
 template <typename T>
 int run_small(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, const RunArgs<T>& R, cudaStream_t st) {
-  const int D = p->D;
-  if (D <= 2) return run_small_dt<T, 2>(c, p, A, integ, R, st);
-  if (D <= 4) return run_small_dt<T, 4>(c, p, A, integ, R, st);
-  if (D <= 8) return run_small_dt<T, 8>(c, p, A, integ, R, st);
-  if (D <= 10) return run_small_dt<T, 10>(c, p, A, integ, R, st);
-  if (D <= 16) return run_small_dt<T, 16>(c, p, A, integ, R, st);
-  if (D <= 32) return run_small_dt<T, 32>(c, p, A, integ, R, st);
-  return fail(EHMC_ERR_UNSUPPORTED, "small-D kernel: D = %d > 32", D);
-}
-
-template <typename T, int DT>
-static int eval_small_dt(ehmc_ctx* c, const ehmc_potential* p, const T* q, long long q_ld, long long P, T* e, T* g,
-                         long long g_ld, cudaStream_t st) {
-  const unsigned grid = (unsigned)((P + 127) / 128);
-  switch (p->family) {
-    case EHMC_FAMILY_DIAG_GAUSSIAN:
-      k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_diag<T, DT>(p));
-      break;
-    case EHMC_FAMILY_FUNNEL:
-      k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_funnel<T, DT>(p));
-      break;
-    case EHMC_FAMILY_COIN_TOSS:
-      k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_coin<T, DT>(p));
-      break;
-    case EHMC_FAMILY_HIERARCHICAL_NORMAL:
-      if constexpr (DT >= 4) {
-        if (p->hier.centered)
-          k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_hier<T, DT, true>(p));
-        else
-          k_eval_small<T, DT><<<grid, 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, make_hier<T, DT, false>(p));
-        break;
-      }
-      return fail(EHMC_ERR_UNSUPPORTED, "eval: family %d", p->family);
-    default:
-      return fail(EHMC_ERR_UNSUPPORTED, "eval: family %d", p->family);
-  }
-  c->launches++;
-  CUDA_TRY(cudaGetLastError());
-  return EHMC_OK;
+  return with_small_pot<T>(p, "fused multi-iteration kernel", [&](auto dt, const auto& pot) -> int {
+    constexpr int DT = decltype(dt)::value;
+    using Pot = std::decay_t<decltype(pot)>;
+    const unsigned grid = (unsigned)std::max<long long>(1, (A.P + K1_THREADS - 1) / K1_THREADS);
+    if (integ == INTEG_LEAPFROG)
+      k_small_run<T, DT, Pot, INTEG_LEAPFROG><<<grid, K1_THREADS, 0, st>>>(A, pot, R);
+    else
+      k_small_run<T, DT, Pot, INTEG_STORMER><<<grid, K1_THREADS, 0, st>>>(A, pot, R);
+    c->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return EHMC_OK;
+  });
 }
 
 template <typename T>
 int eval_small(ehmc_ctx* c, const ehmc_potential* p, const T* q, long long q_ld, long long P, T* e, T* g,
                long long g_ld, cudaStream_t st) {
-  const int D = p->D;
-  if (D <= 2) return eval_small_dt<T, 2>(c, p, q, q_ld, P, e, g, g_ld, st);
-  if (D <= 4) return eval_small_dt<T, 4>(c, p, q, q_ld, P, e, g, g_ld, st);
-  if (D <= 8) return eval_small_dt<T, 8>(c, p, q, q_ld, P, e, g, g_ld, st);
-  if (D <= 10) return eval_small_dt<T, 10>(c, p, q, q_ld, P, e, g, g_ld, st);
-  if (D <= 16) return eval_small_dt<T, 16>(c, p, q, q_ld, P, e, g, g_ld, st);
-  if (D <= 32) return eval_small_dt<T, 32>(c, p, q, q_ld, P, e, g, g_ld, st);
-  return fail(EHMC_ERR_UNSUPPORTED, "eval: D = %d", D);
+  return with_small_pot<T>(p, "eval kernel", [&](auto dt, const auto& pot) -> int {
+    constexpr int DT = decltype(dt)::value;
+    // dense potentials are evaluated by k_eval_dense at every D (eval_device): k_eval_small has no dense instance
+    if constexpr (std::is_same_v<std::decay_t<decltype(pot)>, DenseSmallPot<T, DT>>) {
+      return fail(EHMC_ERR_UNSUPPORTED, "eval: dense potentials are evaluated by k_eval_dense");
+    } else {
+      k_eval_small<T, DT><<<(unsigned)((P + 127) / 128), 128, 0, st>>>(q, q_ld, P, p->D, e, g, g_ld, pot);
+      c->launches++;
+      CUDA_TRY(cudaGetLastError());
+      return EHMC_OK;
+    }
+  });
 }
 
 }  // namespace ehmc

@@ -97,40 +97,13 @@ static int ens_launch(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, EnsRunA
   return EHMC_OK;
 }
 
-template <typename T, int DT, class Pot>
-static int ens_pot(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, const EnsRunArgs<T>& R, cudaStream_t st) {
-  return A.D == DT ? ens_launch<T, DT, Pot, true>(c, A, pot, R, st) : ens_launch<T, DT, Pot, false>(c, A, pot, R, st);
-}
-
-template <typename T, int DT>
-static int ens_dt(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, const EnsRunArgs<T>& R, cudaStream_t st) {
-  switch (p->family) {
-    case EHMC_FAMILY_DIAG_GAUSSIAN: return ens_pot<T, DT>(c, A, make_diag<T, DT>(p), R, st);
-    case EHMC_FAMILY_FUNNEL: return ens_pot<T, DT>(c, A, make_funnel<T, DT>(p), R, st);
-    case EHMC_FAMILY_COIN_TOSS: return ens_pot<T, DT>(c, A, make_coin<T, DT>(p), R, st);
-    case EHMC_FAMILY_DENSE_GAUSSIAN:
-      if constexpr (DT <= 16) return ens_pot<T, DT>(c, A, make_dense_small<T, DT>(p), R, st);
-      break;
-    case EHMC_FAMILY_HIERARCHICAL_NORMAL:
-      if constexpr (DT >= 4)
-        return p->hier.centered ? ens_pot<T, DT>(c, A, make_hier<T, DT, true>(p), R, st)
-                                : ens_pot<T, DT>(c, A, make_hier<T, DT, false>(p), R, st);
-      break;
-    default: break;
-  }
-  return fail(EHMC_ERR_UNSUPPORTED, "family %d has no fused ensemble-run kernel for D = %d", p->family, p->D);
-}
-
 template <typename T>
 int run_small_ens(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, const EnsRunArgs<T>& R, cudaStream_t st) {
-  const int D = p->D;
-  if (D <= 2) return ens_dt<T, 2>(c, p, A, R, st);
-  if (D <= 4) return ens_dt<T, 4>(c, p, A, R, st);
-  if (D <= 8) return ens_dt<T, 8>(c, p, A, R, st);
-  if (D <= 10) return ens_dt<T, 10>(c, p, A, R, st);
-  if (D <= 16) return ens_dt<T, 16>(c, p, A, R, st);
-  if (D <= 32) return ens_dt<T, 32>(c, p, A, R, st);
-  return fail(EHMC_ERR_UNSUPPORTED, "small-D kernel: D = %d > 32", D);
+  return with_small_pot<T>(p, "fused ensemble-run kernel", [&](auto dt, const auto& pot) -> int {
+    constexpr int DT = decltype(dt)::value;
+    using Pot = std::decay_t<decltype(pot)>;
+    return A.D == DT ? ens_launch<T, DT, Pot, true>(c, A, pot, R, st) : ens_launch<T, DT, Pot, false>(c, A, pot, R, st);
+  });
 }
 
 }  // namespace ehmc
