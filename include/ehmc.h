@@ -332,6 +332,33 @@ EHMC_API int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, DLT
                           DLTensor* state, DLTensor* history, DLTensor* moments, DLTensor* trace,
                           int64_t traceParticles, int64_t traceOffset, void* stream);
 
+/* ---- per-chain moments for convergence diagnostics (nested R-hat) ------------------------------------------------ */
+/* Welford's streaming update of every chain's mean and sum of squared deviations m2 with its n-th draw, in the dtype
+ * of q:  n = 1: mean = q, m2 = 0 (nothing is read: the buffers need no initialisation);  n > 1: d = q - mean,
+ * mean += d (1/n), m2 += d (q - mean).  The within-chain variance of N draws is m2 / (N - 1).
+ *   q        [D,P] device
+ *   mean, m2 [D,P] device, same dtype as q, the same row stride as each other; in/out
+ * One elementwise kernel on `stream`. */
+EHMC_API int ehmc_chain_moments_update(ehmc_ctx* ctx, const DLTensor* q, DLTensor* mean, DLTensor* m2, int64_t n,
+                                       void* stream);
+
+/* Optional per-chain moments of ehmc_hmc_run_ensemble_chains: iteration k >= windowStart of the call enters mean / m2
+ * as draw n = k - windowStart + 1, with the update of ehmc_chain_moments_update (identical bits). */
+typedef struct {
+  uint32_t struct_size;  /* sizeof(ehmc_chain_args) */
+  DLTensor* mean;        /* [D,P] device, dtype of q */
+  DLTensor* m2;          /* [D,P] device, dtype of q, row stride of mean */
+  int64_t windowStart;   /* >= 0 */
+} ehmc_chain_args;
+
+/* ehmc_hmc_run_ensemble with per-chain moments accumulated inside the same launch (chains = NULL: none; the
+ * trajectories, statistics and step sizes do not depend on it). */
+EHMC_API int ehmc_hmc_run_ensemble_chains(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
+                                          const ehmc_hmc_args* args, int numIterations, const ehmc_adapt_args* adapt,
+                                          ehmc_comm* comm, DLTensor* state, DLTensor* history, DLTensor* moments,
+                                          DLTensor* trace, int64_t traceParticles, int64_t traceOffset,
+                                          const ehmc_chain_args* chains, void* stream);
+
 /* Consumes the (all-reduced) statistics of the iteration that just ran with the block `dynamic`:
  *   history[dynamic.row] = {acceptRate, meanAcceptProb, meanH, stepSize used}  (optional, float64 [S,4])
  *   moments[0:D] += sum q_d, moments[D:2D] += sum q_d^2                        (optional, float64 [2D])

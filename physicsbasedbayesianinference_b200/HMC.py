@@ -224,7 +224,7 @@ class HMC:
     # ------------------------------------------------------------------------------------
     def run(self, numIterations, temperature, *, adapt=False, targetAccept=0.8, adaptIterations=None,
             traceParticles=0, group=None, collectStats=True, keepNumSteps=False, deviceAdapt=False, graph=False,
-            fused=None, adaptLag=1, adaptMass=False, massWindows=3):
+            fused=None, adaptLag=1, adaptMass=False, massWindows=3, chainDiagnostics=False, superchainSize=1):
         """Production loop for device ensembles (build-defined; scales where getSamples'
         (D, P, S) arrays cannot, SURVEY.md section 7 hard part 7).
 
@@ -271,11 +271,25 @@ class HMC:
         mean, var (those of the last phase: after the warm-up if the call goes beyond it) and trace.  See
         _run_mass_adapt.
 
+        chainDiagnostics=True accumulates every chain's mean and within-chain variance over the sampling window on the
+        GPU (Welford, inside the fused launch or one elementwise kernel per iteration of the host loop) and returns
+        nested R-hat over ALL chains of all ranks (diagnostics.py), chains k M .. k M + M - 1 of the global ensemble
+        forming superchain k (M = superchainSize; start them with Ensemble.setPosition(qStd, superchainSize=M)).  The
+        window is the iterations whose step size is final: adaptIterations + adaptLag .. with adapt=True (the
+        non-warm-up phase with adaptMass), the whole call otherwise.  Positions, traces, step sizes and statistics are
+        the same bits with and without it.  Not with deviceAdapt=True.
+
         Returns dict(acceptRate[S], meanAcceptProb[S], meanH[S], stepSize[S], mean[D], var[D],
-        trace (D, traceParticles, S) or None).
+        trace (D, traceParticles, S) or None); with chainDiagnostics also rhat[D], rhatBetween[D] (B^), rhatWithin[D]
+        (W^) as float64 CPU tensors, chainMean and chainVar (D, P local) device tensors in the ensemble's dtype (the
+        original coordinates) and rhatDraws (N, the window's length) -- all None when the window is empty.
         """
         if adaptLag not in (1, 2, 3, 4):
             raise ValueError("adaptLag must be 1, 2, 3 or 4")
+        if chainDiagnostics and not self._inRun:
+            phased = adaptMass or getattr(self, "massScale", None) is not None
+            self._check_chain_diagnostics(numIterations, adapt, adaptIterations, adaptLag, phased, deviceAdapt, group,
+                                          superchainSize)
         if not self._inRun:
             # everything below runs with _inRun set: non-finite acceptance ratios are rejected unless the driver was
             # built with an explicit rejectNonFinite=False (see __init__)
@@ -285,7 +299,8 @@ class HMC:
                                 adaptIterations=adaptIterations, traceParticles=traceParticles, group=group,
                                 collectStats=collectStats, keepNumSteps=keepNumSteps, deviceAdapt=deviceAdapt,
                                 graph=graph, fused=fused, adaptLag=adaptLag, adaptMass=adaptMass,
-                                massWindows=massWindows)
+                                massWindows=massWindows, chainDiagnostics=chainDiagnostics,
+                                superchainSize=superchainSize)
             finally:
                 self._inRun = False
         if adaptMass or getattr(self, "massScale", None) is not None:
@@ -295,7 +310,8 @@ class HMC:
                                         adapt=adapt, targetAccept=targetAccept, adaptIterations=adaptIterations,
                                         traceParticles=traceParticles, group=group, collectStats=collectStats,
                                         keepNumSteps=keepNumSteps, deviceAdapt=deviceAdapt, graph=graph, fused=fused,
-                                        adaptLag=adaptLag)
+                                        adaptLag=adaptLag, chainDiagnostics=chainDiagnostics,
+                                        superchainSize=superchainSize)
         if deviceAdapt and adaptLag != 1:
             raise ValueError("deviceAdapt=True implements adaptLag=1 only")
         if fused is None:
@@ -303,7 +319,7 @@ class HMC:
                      and self._fused_loop_ok() and (keepNumSteps or not adapt) and numIterations > 0)
         if fused:
             return self._run_fused(numIterations, temperature, adapt, targetAccept, adaptIterations, traceParticles,
-                                   group, adaptLag)
+                                   group, adaptLag, chainDiagnostics, superchainSize)
         if deviceAdapt:
             return self._run_device_adapt(numIterations, temperature, adapt, targetAccept, adaptIterations,
                                           traceParticles, group, graph)
@@ -345,6 +361,9 @@ class HMC:
         nstat = 0
         trace = (torch.empty((D, traceParticles, numIterations), dtype=ens.dtype, device=dev)
                  if traceParticles else None)
+        w0 = self._chain_window(numIterations, adapt, adaptIterations, adaptLag) if chainDiagnostics else numIterations
+        chains = self._chain_buffers(numIterations - w0)
+        ctx = _lib.Context.get(dev.index)
         self.integrator.q = ens.q
         pending = []  # slots whose statistics are in flight, oldest first (at most adaptLag of them)
 
@@ -374,6 +393,8 @@ class HMC:
             self.step(temperature, stats=stats[slot] if collectStats else None, reuseEndpoint=it > 0)
             if trace is not None:
                 trace[:, :, it] = ens.q[:, :traceParticles]
+            if chains is not None and it >= w0:
+                _lib.chain_moments_update(ctx, ens.q, chains[0], chains[1], it - w0 + 1, _lib.current_stream_ptr(ens.q))
             if collectStats:
                 side.wait_stream(main)
                 with torch.cuda.stream(side):
@@ -391,11 +412,65 @@ class HMC:
         n = max(nstat, 1) * Ptot
         mean = sum1 / n
         out.update(mean=mean, var=sum2 / n - mean * mean, trace=trace, worldSize=world)
+        if chainDiagnostics:
+            out.update(self._chain_result(chains, numIterations - w0, superchainSize,
+                                          (group if group is not None else reducer.dist.group.WORLD)
+                                          if reducer.enabled else None))
         return out
+
+    # ------------------------------------------------------------------------------------
+    def _chain_window(self, n, adapt, adaptIterations, adaptLag, phased=False):
+        """First iteration of a run() call whose positions enter the chain diagnostics: the first one whose step size
+        is final (the statistics of iteration k set the step size of iteration k + 1 + adaptLag); with mass
+        adaptation (phased) the first one after the warm-up phases."""
+        nAdapt = 0 if not adapt else (n if adaptIterations is None else min(n, int(adaptIterations)))
+        if nAdapt == 0:
+            return 0
+        return nAdapt if phased else min(n, nAdapt + adaptLag)
+
+    def _check_chain_diagnostics(self, n, adapt, adaptIterations, adaptLag, phased, deviceAdapt, group, M):
+        """run(chainDiagnostics=True)'s refusals, raised before any device work."""
+        if deviceAdapt:
+            raise ValueError("chainDiagnostics=True needs deviceAdapt=False (a graph replay would bake in the draw count)")
+        ens = self.ensemble
+        M = int(M)
+        if M < 1 or ens.numParticles % M or ens.particleOffset % M:
+            raise ValueError(f"superchainSize {M} must be >= 1 and divide numParticles ({ens.numParticles}) and "
+                             f"particleOffset ({ens.particleOffset}): a superchain must not straddle two shards")
+        N = int(n) - self._chain_window(int(n), adapt, adaptIterations, adaptLag, phased)
+        if N == 1 and M == 1:
+            raise ValueError("nested R-hat needs superchainSize > 1 or a window of more than one iteration")
+        import torch.distributed as dist
+
+        single = not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1
+        if single and ens.numParticles // M < 2:
+            raise ValueError(f"nested R-hat needs at least 2 superchains, got {ens.numParticles // M}")
+
+    def _chain_buffers(self, N):
+        """(mean, m2) accumulators [D, P] of the chain diagnostics (no initialisation: draw 1 writes them), or None."""
+        if N <= 0:
+            return None
+        import torch
+
+        ens = self.ensemble
+        return tuple(torch.empty((ens.numDimensions, ens.numParticles), dtype=ens.dtype, device=ens.device)
+                     for _ in range(2))
+
+    def _chain_result(self, chains, N, M, group):
+        """The result keys of run(chainDiagnostics=True) from the accumulators of N draws (group: combine the ranks)."""
+        if chains is None:
+            return dict(rhat=None, rhatBetween=None, rhatWithin=None, chainMean=None, chainVar=None, rhatDraws=None)
+        from .diagnostics import nested_rhat_from_moments
+
+        mean, m2 = chains
+        var = m2 / (N - 1) if N > 1 else m2.zero_()
+        rhat, between, within = nested_rhat_from_moments(mean, var, N, M, group=group)
+        return dict(rhat=rhat.cpu(), rhatBetween=between.cpu(), rhatWithin=within.cpu(), chainMean=mean, chainVar=var,
+                    rhatDraws=N)
 
 
     def _run_mass_adapt(self, numIterations, temperature, *, adaptMass, massWindows, adapt, adaptIterations,
-                        traceParticles, **kw):
+                        traceParticles, chainDiagnostics=False, superchainSize=1, **kw):
         """run() in rescaled coordinates (see run(adaptMass=True)).
 
         The call is cut into phases -- parallel.mass_windows during the warm-up, one phase for the rest -- and every
@@ -431,16 +506,24 @@ class HMC:
         ens.q.div_(st)  # into the rescaled coordinates
         out = dict(acceptRate=[], meanAcceptProb=[], meanH=[], stepSize=[], numSteps=[], massScale=[])
         traces = []
+        chainOut = dict(rhat=None, rhatBetween=None, rhatWithin=None, chainMean=None, chainVar=None, rhatDraws=None)
         r = None
         try:
             for k, updateMass, adaptive in phases:
+                # the chain diagnostics' window is the phase after the warm-up (its step size and mass are final)
                 r = self.run(k, temperature, adapt=adaptive, adaptIterations=k if adaptive else 0,
-                             traceParticles=traceParticles, **kw)
+                             traceParticles=traceParticles, chainDiagnostics=chainDiagnostics and not adaptive,
+                             superchainSize=superchainSize, **kw)
                 for key in ("acceptRate", "meanAcceptProb", "meanH", "stepSize", "numSteps"):
                     out[key].extend(r[key])
                 out["massScale"].extend([scale.copy()] * k)
                 if r["trace"] is not None:
                     traces.append(r["trace"] * st[:, :, None])  # original coordinates
+                if r.get("chainMean") is not None:  # original coordinates; R-hat itself is scale invariant
+                    sc2 = torch.from_numpy(scale * scale)
+                    chainOut = dict(rhat=r["rhat"], rhatBetween=r["rhatBetween"] * sc2, rhatWithin=r["rhatWithin"] * sc2,
+                                    chainMean=r["chainMean"] * st, chainVar=r["chainVar"] * (st * st),
+                                    rhatDraws=r["rhatDraws"])
                 if updateMass:
                     cnt = float(k) * float(r.get("numParticlesTotal", ens.numParticles * r.get("worldSize", 1)))
                     s_new = base.projectScales(adapter.scales(r["mean"].numpy(), r["var"].numpy(), cnt))
@@ -456,10 +539,12 @@ class HMC:
             out.update(mean=r["mean"] * sc, var=r["var"] * sc * sc, worldSize=r.get("worldSize", 1),
                        fused=r.get("fused", False))
         out["trace"] = torch.cat(traces, dim=2) if traces else None
+        if chainDiagnostics:
+            out.update(chainOut)
         return out
 
     def _run_fused(self, numIterations, temperature, adapt, targetAccept, adaptIterations, traceParticles, group,
-                   adaptLag=1):
+                   adaptLag=1, chainDiagnostics=False, superchainSize=1):
         """HMC.run as ONE launch: see run(fused=True) and csrc/k_small_ens.cuh."""
         import math
 
@@ -497,6 +582,8 @@ class HMC:
         mom = torch.zeros(2 * D, dtype=torch.float64, device=dev)
         ntrace = int(traceParticles)
         trace = torch.empty((D, ntrace, n), dtype=ens.dtype, device=dev) if ntrace else None
+        w0 = self._chain_window(n, adapt, adaptIterations, adaptLag) if chainDiagnostics else n
+        chains = self._chain_buffers(n - w0)
         self.integrator.q = ens.q
         numSteps = self.integrator.numSteps
         q = ens.q
@@ -505,7 +592,8 @@ class HMC:
                               _lib.make_adapt_args(Ptot, adaptRows, target=targetAccept, lag=adaptLag), state, comm=comm,
                               history=hist,
                               moments=mom, trace=None if trace is None else trace.view(D * ntrace, n),
-                              trace_particles=ntrace, stream=_lib.current_stream_ptr(q))
+                              trace_particles=ntrace, stream=_lib.current_stream_ptr(q),
+                              chains=None if chains is None else (chains[0], chains[1], w0))
         self.iteration += n
         st = state.cpu().numpy()  # synchronises
         self.stepSize = float(st[0])
@@ -515,9 +603,15 @@ class HMC:
         m = mom.cpu().numpy()
         cnt = float(max(n, 1)) * Ptot
         mean = torch.from_numpy(m[:D] / cnt)
-        return dict(acceptRate=list(h[:, 0]), meanAcceptProb=list(h[:, 1]), meanH=list(h[:, 2]), stepSize=list(h[:, 3]),
-                    numSteps=[numSteps] * n, mean=mean, var=torch.from_numpy(m[D:] / cnt) - mean * mean,
-                    trace=trace, worldSize=world, fused=True)
+        out = dict(acceptRate=list(h[:, 0]), meanAcceptProb=list(h[:, 1]), meanH=list(h[:, 2]), stepSize=list(h[:, 3]),
+                   numSteps=[numSteps] * n, mean=mean, var=torch.from_numpy(m[D:] / cnt) - mean * mean,
+                   trace=trace, worldSize=world, fused=True)
+        if chainDiagnostics:
+            ranks = None
+            if comm is not None:
+                ranks = group if group is not None else dist.group.WORLD
+            out.update(self._chain_result(chains, n - w0, superchainSize, ranks))
+        return out
 
     def _run_device_adapt(self, numIterations, temperature, adapt, targetAccept, adaptIterations, traceParticles,
                           group, graph, graphIterations=10):

@@ -38,6 +38,7 @@ SYMBOLS = (
     "ehmc_potential_eval", "ehmc_set_position", "ehmc_set_momentum", "ehmc_philox_fill", "ehmc_leapfrog",
     "ehmc_stormer_verlet", "ehmc_integrate_nbody_mode", "ehmc_hmc_iter", "ehmc_hmc_run", "ehmc_adapt_step",
     "ehmc_comm_create", "ehmc_comm_handle", "ehmc_comm_connect", "ehmc_comm_destroy", "ehmc_hmc_run_ensemble",
+    "ehmc_chain_moments_update", "ehmc_hmc_run_ensemble_chains",
 )
 COMM_HANDLE_BYTES = 64
 COMM_MAX_RANKS = 16
@@ -98,6 +99,17 @@ class AdaptArgs(ctypes.Structure):
     ]
 
 
+class ChainArgs(ctypes.Structure):
+    """struct ehmc_chain_args (include/ehmc.h)."""
+
+    _fields_ = [
+        ("struct_size", ctypes.c_uint32),
+        ("mean", ctypes.c_void_p),
+        ("m2", ctypes.c_void_p),
+        ("windowStart", ctypes.c_int64),
+    ]
+
+
 _lib = None
 _lib_lock = threading.Lock()
 
@@ -143,6 +155,10 @@ def load():
             "ehmc_comm_destroy": [vp],
             "ehmc_hmc_run_ensemble": [vp, vp, vp, vp, ctypes.POINTER(HmcArgs), ci, ctypes.POINTER(AdaptArgs), vp, vp, vp,
                                       vp, vp, ctypes.c_int64, ctypes.c_int64, vp],
+            "ehmc_hmc_run_ensemble_chains": [vp, vp, vp, vp, ctypes.POINTER(HmcArgs), ci, ctypes.POINTER(AdaptArgs), vp,
+                                             vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int64, ctypes.POINTER(ChainArgs),
+                                             vp],
+            "ehmc_chain_moments_update": [vp, vp, vp, vp, ctypes.c_int64, vp],
         }
         for name, args in sigs.items():
             fn = getattr(lib, name)
@@ -418,12 +434,27 @@ def make_adapt_args(num_particles_total, adapt_iterations, target=0.8, gain0=1.5
 
 
 def hmc_run_ensemble(ctx, pot, q, mass, args, num_iterations, adapt, state, comm=None, history=None, moments=None,
-                     trace=None, trace_particles=0, trace_offset=0, stream=None):
+                     trace=None, trace_particles=0, trace_offset=0, stream=None, chains=None):
+    """chains: None, or (mean, m2, window_start): per-chain moments of iterations window_start .. of the call
+    (ehmc_hmc_run_ensemble_chains)."""
     vq, vm, vs = dl(q), dl(mass), dl(state)
     vh, vmo, vt = dl(history), dl(moments), dl(trace)
-    check(ctx.lib.ehmc_hmc_run_ensemble(ctx.handle, pot.handle, vq.ptr, vm.ptr, ctypes.byref(args), int(num_iterations),
-                                        ctypes.byref(adapt), None if comm is None else comm.handle, vs.ptr, _p(vh),
-                                        _p(vmo), _p(vt), int(trace_particles), int(trace_offset), stream))
+    cargs = ()
+    if chains is not None:
+        mean, m2, window_start = chains
+        vcm, vc2 = dl(mean), dl(m2)
+        ca = ChainArgs(ctypes.sizeof(ChainArgs), vcm.ptr, vc2.ptr, int(window_start))
+        cargs = (ctypes.byref(ca),)
+    fn = ctx.lib.ehmc_hmc_run_ensemble if chains is None else ctx.lib.ehmc_hmc_run_ensemble_chains
+    check(fn(ctx.handle, pot.handle, vq.ptr, vm.ptr, ctypes.byref(args), int(num_iterations), ctypes.byref(adapt),
+             None if comm is None else comm.handle, vs.ptr, _p(vh), _p(vmo), _p(vt), int(trace_particles),
+             int(trace_offset), *cargs, stream))
+
+
+def chain_moments_update(ctx, q, mean, m2, n, stream=None):
+    """Welford update of the per-chain mean / m2 [D, P] with the n-th draw q [D, P] (ehmc_chain_moments_update)."""
+    vq, vm, v2 = dl(q), dl(mean), dl(m2)
+    check(ctx.lib.ehmc_chain_moments_update(ctx.handle, vq.ptr, vm.ptr, v2.ptr, int(n), stream))
 
 
 def philox_fill(ctx, z=None, u=None, seed=0, iteration=0, particle_offset=0, stream=None):

@@ -343,6 +343,42 @@ __device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) {
   return d;
 }
 
+// ---------------------------------------------------------------------------
+// Per-chain moments (nested R-hat, diagnostics.py): Welford's streaming update of one chain's mean and sum of squared
+// deviations m2 with its n-th draw q; rn = 1/n rounded to T, computed on the host (an IEEE reciprocal on the device is
+// a slow-path subroutine call, and a call changes the register allocation of the whole trajectory kernel).  n = 1
+// writes (q, 0) and reads nothing, so the buffers need no initialisation.  Every operation is an explicitly rounded
+// intrinsic: the fused run (k_small_ens) and the host loop's k_chain_moments call this in different kernels and must
+// produce the same bits.
+// ---------------------------------------------------------------------------
+template <typename T>
+struct WelfordOps;
+template <>
+struct WelfordOps<float> {
+  static __device__ __forceinline__ float sub(float a, float b) { return __fsub_rn(a, b); }
+  static __device__ __forceinline__ float fma(float a, float b, float c) { return __fmaf_rn(a, b, c); }
+};
+template <>
+struct WelfordOps<double> {
+  static __device__ __forceinline__ double sub(double a, double b) { return __dsub_rn(a, b); }
+  static __device__ __forceinline__ double fma(double a, double b, double c) { return __fma_rn(a, b, c); }
+};
+
+template <typename T>
+__device__ __forceinline__ void chain_moments_update(T* mean, T* m2, T q, long long n, T rn) {
+  typedef WelfordOps<T> W;
+  if (n <= 1) {
+    *mean = q;
+    *m2 = T(0);
+    return;
+  }
+  const T m0 = *mean;
+  const T d = W::sub(q, m0);
+  const T m1 = W::fma(d, rn, m0);
+  *mean = m1;
+  *m2 = W::fma(d, W::sub(q, m1), *m2);
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -976,10 +976,36 @@ extern "C" int ehmc_hmc_run(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* 
 // ---------------------------------------------------------------------------
 // the adaptive ensemble run in one launch
 // ---------------------------------------------------------------------------
+// 1/n of the chain moments' update, rounded to T: the one value both the fused run and k_chain_moments multiply by.
+template <typename T>
+static T chain_rcp(long long n) {
+  return T(1) / T(n);
+}
+
+// The chain moments' accumulators: [D,P] device tensors of the call's dtype with one row stride between them.
+static int check_chain_buffers(const CallViews& v, DLTensor* mean, DLTensor* m2, View* vm, View* v2, const char* fn) {
+  TRY(parse_float(mean, "mean", 2, v.bits, vm));
+  TRY(parse_float(m2, "m2", 2, v.bits, v2));
+  if (vm->host || v2->host) return fail(EHMC_ERR_INVALID, "%s: mean and m2 must be device tensors", fn);
+  if (vm->shape[0] != v.D || vm->shape[1] != v.P || v2->shape[0] != v.D || v2->shape[1] != v.P)
+    return fail(EHMC_ERR_INVALID, "%s: mean and m2 must be [D, P] = [%lld, %lld] like q", fn, v.D, v.P);
+  if (vm->ld != v2->ld) return fail(EHMC_ERR_INVALID, "%s: mean and m2 must have the same row stride", fn);
+  return EHMC_OK;
+}
+
 extern "C" int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
                                      const ehmc_hmc_args* a, int numIterations, const ehmc_adapt_args* ad,
                                      ehmc_comm* comm, DLTensor* state, DLTensor* history, DLTensor* moments,
                                      DLTensor* trace, int64_t traceParticles, int64_t traceOffset, void* stream) {
+  return ehmc_hmc_run_ensemble_chains(ctx, pot, q, mass, a, numIterations, ad, comm, state, history, moments, trace,
+                                      traceParticles, traceOffset, nullptr, stream);
+}
+
+extern "C" int ehmc_hmc_run_ensemble_chains(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
+                                            const ehmc_hmc_args* a, int numIterations, const ehmc_adapt_args* ad,
+                                            ehmc_comm* comm, DLTensor* state, DLTensor* history, DLTensor* moments,
+                                            DLTensor* trace, int64_t traceParticles, int64_t traceOffset,
+                                            const ehmc_chain_args* chains, void* stream) {
   if (ctx) ctx->ep_valid = false;
   NvtxRange nvtx_range("ehmc_hmc_run_ensemble");
   const char* fn = "ehmc_hmc_run_ensemble";
@@ -1013,6 +1039,12 @@ extern "C" int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, D
       return fail(EHMC_ERR_INVALID, "%s: trace must be a contiguous device [D*traceParticles, S] view with room for the iterations", fn);
     S = vt.shape[1];
   }
+  View vcm, vc2;
+  if (chains) {
+    if (chains->struct_size < sizeof(ehmc_chain_args)) return fail(EHMC_ERR_INVALID, "%s: chains.struct_size too small", fn);
+    TRY(check_chain_buffers(v, chains->mean, chains->m2, &vcm, &vc2, fn));
+    if (chains->windowStart < 0) return fail(EHMC_ERR_INVALID, "%s: chains.windowStart < 0", fn);
+  }
   TRY(enter_device(ctx));
   if (numIterations == 0 || v.P == 0) return EHMC_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1044,6 +1076,16 @@ extern "C" int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, D
     R.ntrace = traceParticles;
     R.S = S;
     R.s0 = traceOffset;
+    // (a window that starts after the last iteration updates nothing: off, as with chains == NULL)
+    const bool cm = chains && chains->windowStart < numIterations;
+    std::vector<T> crcp;
+    for (long long k = cm ? chains->windowStart : numIterations; k < numIterations; ++k)
+      crcp.push_back(chain_rcp<T>(k - chains->windowStart + 1));
+    R.cmean = cm ? reinterpret_cast<T*>(vcm.data) : nullptr;
+    R.cm2 = cm ? reinterpret_cast<T*>(vc2.data) : nullptr;
+    R.c_ld = cm ? vcm.ld : 0;
+    R.windowStart = cm ? (int)chains->windowStart : 0;
+    R.crcp = crcp.data();  // host array; the launcher uploads it
     R.rank = comm ? comm->rank : 0;
     R.world = comm ? comm->world : 1;
     R.peers = comm ? comm->peers_dev : nullptr;
@@ -1053,6 +1095,40 @@ extern "C" int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, D
   const int rc = v.bits == 32 ? run(float()) : run(double());
   if (rc == EHMC_OK && comm) comm->seq += (unsigned long long)numIterations;
   return rc;
+}
+
+// ---------------------------------------------------------------------------
+// per-chain moments of the host loop
+// ---------------------------------------------------------------------------
+extern "C" int ehmc_chain_moments_update(ehmc_ctx* ctx, const DLTensor* q, DLTensor* mean, DLTensor* m2, int64_t n,
+                                         void* stream) {
+  NvtxRange nvtx_range("ehmc_chain_moments_update");
+  const char* fn = "ehmc_chain_moments_update";
+  if (!ctx) return fail(EHMC_ERR_INVALID, "%s: NULL context", fn);
+  CallViews v;
+  TRY(parse_float(q, "q", 2, 0, &v.q));
+  if (v.q.host) return fail(EHMC_ERR_INVALID, "%s: q must be a device tensor", fn);
+  v.bits = v.q.bits;
+  v.D = v.q.shape[0];
+  v.P = v.q.shape[1];
+  View vm, v2;
+  TRY(check_chain_buffers(v, mean, m2, &vm, &v2, fn));
+  if (n < 1) return fail(EHMC_ERR_INVALID, "%s: n must be >= 1 (the number of the draw), got %lld", fn, (long long)n);
+  TRY(enter_device(ctx));
+  if (v.D == 0 || v.P == 0) return EHMC_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const dim3 grid((unsigned)std::min<long long>((v.P + 255) / 256, 1 << 16), (unsigned)std::min<long long>(v.D, 65535));
+  if (v.bits == 32)
+    k_chain_moments<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(v.q.data), v.q.ld, v.P, (int)v.D,
+                                                 reinterpret_cast<float*>(vm.data), reinterpret_cast<float*>(v2.data),
+                                                 vm.ld, (long long)n, chain_rcp<float>(n));
+  else
+    k_chain_moments<double><<<grid, 256, 0, st>>>(reinterpret_cast<const double*>(v.q.data), v.q.ld, v.P, (int)v.D,
+                                                  reinterpret_cast<double*>(vm.data), reinterpret_cast<double*>(v2.data),
+                                                  vm.ld, (long long)n, chain_rcp<double>(n));
+  ctx->launches++;
+  CUDA_TRY(cudaGetLastError());
+  return EHMC_OK;
 }
 
 // ---------------------------------------------------------------------------

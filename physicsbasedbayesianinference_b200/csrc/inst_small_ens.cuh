@@ -52,7 +52,8 @@ static int ens_launch(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, EnsRunA
   const unsigned V = R.nvirt, ngroups = (V + ENS_GROUP - 1) / ENS_GROUP;
   // control block (every section on a 128-byte line): hsched [nIter + 1 + lag] | published replicas | ticket [ENS_RING]
   // lines, cursor | group tickets [ENS_RING][ngroups] | done [V], arrived [V] | rows [ENS_RING][V][NS] | group rows
-  // [ENS_RING][ngroups][NS] | gains [adaptIters] | batch rows [nbatch][2 DT + 3] (state precision)
+  // [ENS_RING][ngroups][NS] | gains [adaptIters] | batch rows [nbatch][2 DT + 3] (state precision) | 1/n of the chain
+  // moments' window [nIter - windowStart] (state precision)
   auto up = [](size_t n) { return (n + 15) / 16 * 16; };
   const size_t n_h = up((size_t)R.nIter + 1 + ENS_MAX_LAG);
   const size_t n_pub = (size_t)ENS_PUB_COPIES * 16;
@@ -63,7 +64,9 @@ static int ens_launch(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, EnsRunA
   const size_t n_grows = up((size_t)ENS_RING * ngroups * NS);
   const size_t n_gains = up((size_t)std::max(1, R.adaptIters));
   const size_t n_brows = up(((size_t)nrows * (2 * DT + 3) * sizeof(T) + 7) / 8);
-  const size_t bytes = sizeof(double) * (n_h + n_pub + n_tk + n_gt + n_done + n_rows + n_grows + n_gains + n_brows) + 128;
+  const size_t n_crcp = R.cmean != nullptr ? up(((size_t)(R.nIter - R.windowStart) * sizeof(T) + 7) / 8) : 0;
+  const size_t bytes =
+      sizeof(double) * (n_h + n_pub + n_tk + n_gt + n_done + n_rows + n_grows + n_gains + n_brows + n_crcp) + 128;
   TRY(c->ens_ctl.ensure(bytes));
   double* base = reinterpret_cast<double*>(((uintptr_t)c->ens_ctl.ptr + 127) & ~(uintptr_t)127);
   R.hsched = base;
@@ -82,6 +85,11 @@ static int ens_launch(ehmc_ctx* c, const IterArgs<T>& A, const Pot& pot, EnsRunA
   if (R.adaptIters > 0)  // R.gains arrives as a HOST array
     CUDA_TRY(cudaMemcpyAsync(gains, R.gains, sizeof(double) * R.adaptIters, cudaMemcpyHostToDevice, st));
   R.gains = gains;
+  if (R.cmean != nullptr) {  // R.crcp arrives as a HOST array
+    T* crcp = reinterpret_cast<T*>(static_cast<double*>(R.brows) + n_brows);
+    CUDA_TRY(cudaMemcpyAsync(crcp, R.crcp, sizeof(T) * (size_t)(R.nIter - R.windowStart), cudaMemcpyHostToDevice, st));
+    R.crcp = crcp;
+  }
   R.dbg = nullptr;
   R.dbg_iters = 0;
   if (c->ens_debug > 0) {

@@ -134,6 +134,16 @@ __global__ void k_philox_fill(T* out, long long ld, long long P, int D, T* u, co
   if (u != nullptr) u[i] = NormalBlock<T>::uniform(K, offset + (u64)i, out != nullptr ? D : 0);
 }
 
+// Per-chain moments of the host loop (HMC.run outside the fused launch): the n-th draw q[D, P] of every chain enters its
+// running mean / m2 (chain_moments_update, the same bits as the fused run's epilogue).  One pass, coalesced along P.
+template <typename T>
+__global__ void __launch_bounds__(256) k_chain_moments(const T* __restrict__ q, long long q_ld, long long P, int D,
+                                                      T* mean, T* m2, long long ld, long long n, T rn) {
+  for (int d = blockIdx.y; d < D; d += gridDim.y)
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < P; i += (long long)gridDim.x * blockDim.x)
+      chain_moments_update(&mean[d * ld + i], &m2[d * ld + i], q[d * q_ld + i], n, rn);
+}
+
 // Register-only FFMA chain: 8 independent accumulators x ITER FMAs per thread.
 static __global__ void k_fma_peak(float* out, int iters, float a, float b) {
   float x0 = threadIdx.x, x1 = x0 + 1, x2 = x0 + 2, x3 = x0 + 3, x4 = x0 + 4, x5 = x0 + 5, x6 = x0 + 6, x7 = x0 + 7;

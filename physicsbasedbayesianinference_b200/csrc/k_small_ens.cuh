@@ -88,6 +88,11 @@ struct EnsRunArgs {
   double* moments;     // [2D] += sum q_d, sum q_d^2 of every iteration, or null
   T* trace;            // [D][ntrace][S] kept positions of the first ntrace local particles, or null
   long long ntrace, S, s0;
+  T* cmean;            // [D][c_ld] per-chain running mean over iterations windowStart .. (chain_moments_update), or null
+  T* cm2;              // [D][c_ld] per-chain sum of squared deviations from that mean
+  long long c_ld;
+  int windowStart;     // first iteration of this launch whose positions enter the chain moments
+  const T* crcp;       // [nIter - windowStart] 1/n of draw n of the window, rounded to T (host-computed)
   int rank, world;
   double* const* peers;   // [world] every rank's mailbox [2][world][ENS_MB_STRIDE] (peers[rank] = the local one)
   unsigned long long seq0;  // iterations this communicator has reduced before this launch
@@ -286,7 +291,22 @@ __global__ void __launch_bounds__(K1_THREADS, 8) k_small_ens(const IterArgs<T> A
             for (int d = 0; d < Dn; ++d) R.trace[((long long)d * R.ntrace + i) * R.S + R.s0 + it] = Ain.q[d * Ain.q_ld + i];
         }
       }
-      __syncwarp();  // positions and the batch row are written (memory ordering among the warp's lanes)
+      if (R.cmean != nullptr && it >= R.windowStart) {
+        // per-chain moments of the window (nested R-hat), from the positions each thread just wrote; the next
+        // iteration of these particles reads the accumulators behind the same release / acquire as their positions
+        const long long n = (long long)(it - R.windowStart) + 1;
+        const T rn = R.crcp[n - 1];
+        // (kept rolled: a handful of registers at this point, next to the trajectory's 64)
+#pragma unroll 1
+        for (int sb = 0; sb < (1 << R.sshift); ++sb) {
+          const long long i = ((((long long)b << R.sshift) + sb) * 32) + lane;
+          if (i < Ain.P)
+#pragma unroll 1
+            for (int d = 0; d < Dn; ++d)
+              chain_moments_update(&R.cmean[d * R.c_ld + i], &R.cm2[d * R.c_ld + i], Ain.q[d * Ain.q_ld + i], n, rn);
+        }
+      }
+      __syncwarp();  // positions, chain moments and the batch row are written (memory ordering among the warp's lanes)
       const unsigned grp = b >> R.bshift;
       const unsigned b0 = grp << R.bshift;
       const unsigned cnt = min(1u << R.bshift, NB - b0);  // batches of this group

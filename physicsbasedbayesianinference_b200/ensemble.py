@@ -74,23 +74,38 @@ class Ensemble:
     def _ctx(self):
         return _lib.Context.get(self.device.index if self.onDevice and self.device.index is not None else None)
 
-    def setPosition(self, qStd):
+    def setPosition(self, qStd, superchainSize=1):
         """Distribute positions with a normal distribution of standard deviation qStd
-        (src/ensemble.py:63-76).  Rebinds and returns ``self.q``."""
+        (src/ensemble.py:63-76).  Rebinds and returns ``self.q``.
+
+        superchainSize M > 1 starts superchains for nested R-hat (diagnostics.py): every particle takes the draw of
+        the first particle of its superchain, global particle id // M.  M must divide numParticles and
+        particleOffset, so that no superchain straddles two shards.  M = 1 draws exactly as before."""
+        M = int(superchainSize)
+        if M < 1 or self.numParticles % M or self.particleOffset % M:
+            raise ValueError(f"superchainSize {superchainSize} must be >= 1 and divide numParticles "
+                             f"({self.numParticles}) and particleOffset ({self.particleOffset})")
+        D, P = self.numDimensions, self.numParticles
         if not self.onDevice:
             from scipy.stats import norm
 
-            self.q = norm.rvs(scale=qStd, size=(self.numDimensions, self.numParticles)).astype(self.dtype, copy=False)
+            if M == 1:
+                self.q = norm.rvs(scale=qStd, size=(D, P)).astype(self.dtype, copy=False)
+            else:
+                self.q = np.repeat(norm.rvs(scale=qStd, size=(D, P // M)), M, axis=1).astype(self.dtype, copy=False)
             return self.q
         import torch
 
-        self.q = torch.empty((self.numDimensions, self.numParticles), dtype=self.dtype, device=self.device)
+        self.q = torch.empty((D, P), dtype=self.dtype, device=self.device)
         # fresh positions on every call, like the reference's norm.rvs: call k > 0 draws from the Philox key
         # seed XOR k * 0x9E3779B97F4A7C15 (call 0: the seed itself, the stream documented in ehmc.h)
         seed = (self.seed ^ ((self._posCount * 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF)) & 0xFFFFFFFFFFFFFFFF
         self._posCount += 1
         _lib.set_position(self._ctx(), self.q, qStd, seed, self.particleOffset,
                           _lib.current_stream_ptr(self.q))
+        if M > 1:
+            # the first chain's draw of every superchain (whose global id, a multiple of M, does not depend on sharding)
+            self.q.copy_(self.q.view(D, P // M, M)[:, :, :1].expand(D, P // M, M).reshape(D, P))
         return self.q
 
     def setMomentum(self, temperature):
