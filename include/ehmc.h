@@ -47,6 +47,9 @@
  *  just drawn the momentum needs no further Philox block (D = 10: 3 blocks instead of 4); every other case: word x
  *  (float64: x, y) of block 0xFFFFFFFF.  Version 1 (library versions < 110) always used block 0xFFFFFFFF.
  *  oracle/hmc_oracle.py::philox_stream is the bit-level specification used by the tests.
+ *  Replica-exchange uniform of ehmc_hmc_run_tempered (a new block; no earlier draw changes): block 0xFFFFFFFE with
+ *  the counter of the pair's LOWER particle (its global id, the iteration of the swap), float32 (x >> 8) 2^-24,
+ *  float64 ((x >> 6) << 27 | y >> 5) 2^-53.  tests/tempering_reference.py::swap_uniform specifies it bit for bit.
  */
 #ifndef EHMC_H_
 #define EHMC_H_
@@ -119,7 +122,14 @@ typedef enum {
    *   non-centred:  + 0.5 sum_j thetaTilde_j^2
    * params: y[J], sigma[J] [, scale[D]]: with scale, the same potential in rescaled coordinates, U'(q) = U(scale q)
    * (diagonal mass matrix, HMC.run(adaptMass=True)).  scalars: {muLoc, muScale, tauScale, centered}. */
-  EHMC_FAMILY_HIERARCHICAL_NORMAL = 7
+  EHMC_FAMILY_HIERARCHICAL_NORMAL = 7,
+  /* Mixture of K Gaussians with diagonal covariances, a multimodal target:
+   *   U = -log sum_k w_k prod_d N(q_d; mu_kd, sigma_kd^2)
+   * with the constants (D/2) log 2 pi and log sum_k w_k dropped; the per-component -sum_d log sigma_kd terms are
+   * kept (they weigh the components against each other).  Evaluated as a max-shifted log-sum-exp, so U and grad U
+   * stay finite far from every mode.  params: weights[K] (> 0, need not sum to 1), means[K,D], stds[K,D] (> 0).
+   * scalars: none.  1 <= K <= 8, D <= 32 (larger: EHMC_ERR_UNSUPPORTED). */
+  EHMC_FAMILY_GAUSSIAN_MIXTURE = 8
 } ehmc_family;
 
 typedef enum {
@@ -283,11 +293,41 @@ EHMC_API int ehmc_hmc_iter(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q
  *   momenta_out  [D*P, S] optional
  *   accepted_out [P] int32 optional: accepted proposals per particle
  * Device tensors and the small-D families only (diagonal / small dense Gaussian, funnel, coin toss, hierarchical
- * normal);
+ * normal, Gaussian mixture);
  * EHMC_ERR_UNSUPPORTED otherwise -- call ehmc_hmc_iter per iteration then. */
 EHMC_API int ehmc_hmc_run(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
                  const ehmc_hmc_args* args, int numIterations, DLTensor* samples_out, DLTensor* momenta_out,
                  int64_t sampleOffset, DLTensor* accepted_out, void* stream);
+
+/* ---- getSamples' loop with parallel tempering (replica exchange), in ONE launch -------------------------------- */
+/* Systems of R adjacent particles: particle i is replica r = i mod R of system i / R.  Slot r samples at inverse
+ * temperature betas[r]: momentum std sqrt((mass * boltzmann) * temperature) / sqrt(beta_r), Metropolis test on
+ * beta_r (oldH - newH) -- with boltzmann * temperature = 1 slot r targets exp(-beta_r U).  After every iteration's
+ * Metropolis step the deterministic even-odd schedule proposes swaps: at Philox iteration k the pairs are
+ * (r, r + 1) with r = k (mod 2); the lower particle draws u (block 0xFFFFFFFE, see "RNG stream") and the two exchange
+ * their states iff u < min(1, exp((beta_r - beta_r+1)(U_r - U_r+1))) (a NaN exponent rejects).  The schedule follows
+ * the global iteration, so splitting a run into several calls does not change its results.  At R = 1 (betas = {1})
+ * this is ehmc_hmc_run bit for bit. */
+typedef struct {
+  uint32_t struct_size;   /* sizeof(ehmc_temper_args) */
+  int32_t R;              /* replicas per system: 1, 2, 4, 8, 16 or 32 */
+  const DLTensor* betas;  /* float64[R] device: 1 = betas[0] > betas[1] > ... > betas[R-1] > 0 (read back once) */
+  DLTensor* swaps_out;    /* int32[P] device, optional: accepted swaps of slot r with slot r + 1, per particle */
+  DLTensor* roundtrips_out; /* int32[P/R] device, optional: round trips per system -- a state that visited the
+                               hottest slot and then reached slot 0 (labels start at the call's first iteration) */
+} ehmc_temper_args;
+
+/* numIterations tempered iterations (Philox iterations args.iteration ..), as ehmc_hmc_run:
+ *   q            [D,P] in/out (device); P and args.particleOffset multiples of R
+ *   samples_out  [D*P, S] optional: slot sampleOffset + k holds the positions after iteration k's swap, so slot r of
+ *                a system always holds its beta_r state (slot 0: the target itself)
+ *   accepted_out [P] int32 optional: accepted HMC proposals per particle
+ * Small-D families, device tensors only, Philox draws only (there is no fed z / u); counts are this call's.
+ * EHMC_ERR_INVALID for a bad R, ladder or shard (P or particleOffset not a multiple of R) and for host tensors,
+ * EHMC_ERR_UNSUPPORTED for families without a small-D kernel and for args.dynamic. */
+EHMC_API int ehmc_hmc_run_tempered(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
+                                   const ehmc_hmc_args* args, int numIterations, const ehmc_temper_args* temper,
+                                   DLTensor* samples_out, int64_t sampleOffset, DLTensor* accepted_out, void* stream);
 
 /* ---- the adaptive ensemble run in ONE launch, with the statistics all-reduce inside the kernel -------------- */
 /* Peer-memory mailboxes: one process per GPU creates a communicator, the caller exchanges the opaque handles of
@@ -325,7 +365,8 @@ typedef struct {
  *   moments  float64[2D] device, optional, accumulated: sum q_d, sum q_d^2 over particles and iterations
  *   trace    [D*traceParticles, S] device, optional: kept positions of the first traceParticles local particles,
  *            iteration k in slot traceOffset + k
- * Small-D families (diagonal / small dense Gaussian, funnel, coin toss, hierarchical normal), device tensors,
+ * Small-D families (diagonal / small dense Gaussian, funnel, coin toss, hierarchical normal, Gaussian mixture), device
+ * tensors,
  * leapfrog; every rank of `comm` (NULL: single GPU) must make the same call. */
 EHMC_API int ehmc_hmc_run_ensemble(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
                           const ehmc_hmc_args* args, int numIterations, const ehmc_adapt_args* adapt, ehmc_comm* comm,

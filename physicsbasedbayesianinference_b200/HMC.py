@@ -214,11 +214,68 @@ class HMC:
         return samples_hmc, momentum_hmc
 
 
+    def getSamplesTempered(self, numSamples, temperature, qStd, betas):
+        """getSamples with parallel tempering (replica exchange), for multimodal targets (build-defined).
+
+        The ensemble is cut into P / R systems of R = len(betas) adjacent particles (R in 1, 2, 4, ..., 32; P and
+        particleOffset multiples of R).  Slot r of a system samples at inverse temperature betas[r]
+        (1 = betas[0] > betas[1] > ... > 0): its momentum std is the usual one over sqrt(beta_r) and its Metropolis
+        test uses beta_r (oldH - newH), so with boltzmannConst * temperature = 1 (temperature = 1 / boltzmannConst, as
+        for getSamples) slot r targets exp(-beta_r U).  After every iteration neighbouring slots propose to exchange
+        their states (deterministic even-odd schedule), so states found at high temperature reach slot 0.  The whole
+        loop is one launch (ehmc_hmc_run_tempered): the pairs are R adjacent lanes of a warp and a swap is a few
+        register shuffles.  betas = [1] reproduces getSamples bit for bit.
+
+        qStd: positions drawn as in getSamples (Ensemble.setPosition), or None to continue from the ensemble's
+        current positions (two calls of n iterations then give the bits of one call of 2 n).
+        Device ensembles with Philox draws and small-D families only.
+
+        Returns dict(samples (D, P, S) in level order, coldSamples (D, P / R, S): the view of slot 0, the target's
+        samples; acceptRate[R], swapRate[R - 1] (float64 arrays: accepted HMC proposals per slot, accepted swaps of
+        slot r with slot r + 1 per attempt); roundTrips (P / R,) int32: per system, the states that went from slot 0
+        to the hottest slot and back within the call)."""
+        import torch
+
+        ens = self.ensemble
+        if not ens.onDevice or self.rng != "philox":
+            raise ValueError("getSamplesTempered needs a device ensemble with rng='philox' (the swap uniforms and the "
+                             "momenta are drawn inside the kernel)")
+        if not self._fused_loop_ok():
+            raise ValueError("getSamplesTempered needs a small-D potential family (diagonal or Gaussian mixture up "
+                             "to D = 32, funnel, coin toss, hierarchical normal; dense Gaussian up to D = 16)")
+        b = np.atleast_1d(np.asarray(betas, dtype=np.float64))
+        R = int(b.shape[0])
+        D, P, S = ens.numDimensions, ens.numParticles, int(numSamples)
+        dev = ens.device
+        samples = torch.zeros((D, P, S), dtype=ens.dtype, device=dev)
+        accepted = torch.zeros(P, dtype=torch.int32, device=dev)
+        swaps = torch.zeros(P, dtype=torch.int32, device=dev)
+        trips = torch.zeros(P // max(R, 1), dtype=torch.int32, device=dev)
+        self.integrator.q = ens.setPosition(qStd) if qStd is not None else ens.q
+        ctx = _lib.Context.get(dev.index)
+        bits = ens.q.element_size() * 8
+        it0 = self.iteration
+        _lib.hmc_run_tempered(ctx, self.potential.handle(bits, ctx), self.integrator.q, self.integrator.mass,
+                              self._args(temperature), S, R, torch.as_tensor(b, device=dev),
+                              samples.view(D * P, S) if S else None, 0, accepted, swaps, trips,
+                              stream=_lib.current_stream_ptr(ens.q))
+        self.iteration += S
+        ens.q = self.integrator.q
+        self.lastAccept = None
+        nsys = P // R
+        # pair (r, r + 1) is proposed at the iterations k = r (mod 2)
+        attempts = np.array([sum(1 for k in range(it0, it0 + S) if k % 2 == r % 2) for r in range(R - 1)], dtype=float)
+        acc = accepted.view(nsys, R).sum(0).double().cpu().numpy()
+        sw = swaps.view(nsys, R).sum(0).double().cpu().numpy()[:R - 1]
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return dict(samples=samples, coldSamples=samples.view(D, nsys, R, S)[:, :, 0, :],
+                        acceptRate=acc / max(S * nsys, 1), swapRate=sw / (attempts * nsys), roundTrips=trips)
+
     def _fused_loop_ok(self):
         """Families whose getSamples loop runs as one launch (ehmc_hmc_run)."""
         pot = self.potential
         return pot.family in (_lib.FAMILY_DIAG_GAUSSIAN, _lib.FAMILY_FUNNEL, _lib.FAMILY_COIN_TOSS,
-                              _lib.FAMILY_HIERARCHICAL_NORMAL) and \
+                              _lib.FAMILY_HIERARCHICAL_NORMAL, _lib.FAMILY_GAUSSIAN_MIXTURE) and \
             pot.numDimensions <= 32 or (pot.family == _lib.FAMILY_DENSE_GAUSSIAN and pot.numDimensions <= 16)
 
     # ------------------------------------------------------------------------------------

@@ -20,6 +20,7 @@ from . import diagnostics, io, numpyro_adapter, parallel  # noqa: F401
 from .potential import (  # noqa: F401
     CoinTossPotential,
     FunnelPotential,
+    GaussianMixturePotential,
     GaussianPotential,
     HarmonicPotential,
     HierarchicalNormalPotential,

@@ -24,6 +24,7 @@ FAMILY_NBODY = 4
 FAMILY_LOGISTIC = 5
 FAMILY_COIN_TOSS = 6
 FAMILY_HIERARCHICAL_NORMAL = 7
+FAMILY_GAUSSIAN_MIXTURE = 8
 LEAPFROG = 0
 STORMER_VERLET = 1
 FLAG_BUGCOMPAT_MOMENTUM = 1
@@ -38,7 +39,7 @@ SYMBOLS = (
     "ehmc_potential_eval", "ehmc_set_position", "ehmc_set_momentum", "ehmc_philox_fill", "ehmc_leapfrog",
     "ehmc_stormer_verlet", "ehmc_integrate_nbody_mode", "ehmc_hmc_iter", "ehmc_hmc_run", "ehmc_adapt_step",
     "ehmc_comm_create", "ehmc_comm_handle", "ehmc_comm_connect", "ehmc_comm_destroy", "ehmc_hmc_run_ensemble",
-    "ehmc_chain_moments_update", "ehmc_hmc_run_ensemble_chains",
+    "ehmc_chain_moments_update", "ehmc_hmc_run_ensemble_chains", "ehmc_hmc_run_tempered",
 )
 COMM_HANDLE_BYTES = 64
 COMM_MAX_RANKS = 16
@@ -110,6 +111,18 @@ class ChainArgs(ctypes.Structure):
     ]
 
 
+class TemperArgs(ctypes.Structure):
+    """struct ehmc_temper_args (include/ehmc.h)."""
+
+    _fields_ = [
+        ("struct_size", ctypes.c_uint32),
+        ("R", ctypes.c_int32),
+        ("betas", ctypes.c_void_p),
+        ("swaps_out", ctypes.c_void_p),
+        ("roundtrips_out", ctypes.c_void_p),
+    ]
+
+
 _lib = None
 _lib_lock = threading.Lock()
 
@@ -159,6 +172,8 @@ def load():
                                              vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int64, ctypes.POINTER(ChainArgs),
                                              vp],
             "ehmc_chain_moments_update": [vp, vp, vp, vp, ctypes.c_int64, vp],
+            "ehmc_hmc_run_tempered": [vp, vp, vp, vp, ctypes.POINTER(HmcArgs), ci, ctypes.POINTER(TemperArgs), vp,
+                                      ctypes.c_int64, vp, vp],
         }
         for name, args in sigs.items():
             fn = getattr(lib, name)
@@ -387,6 +402,17 @@ def hmc_run(ctx, pot, q, mass, args, num_iterations, samples=None, momenta=None,
     vs, vmo, va = dl(samples), dl(momenta), dl(accepted)
     check(ctx.lib.ehmc_hmc_run(ctx.handle, pot.handle, vq.ptr, vm.ptr, ctypes.byref(args), int(num_iterations), _p(vs),
                                _p(vmo), int(sample_offset), _p(va), stream))
+
+
+def hmc_run_tempered(ctx, pot, q, mass, args, num_iterations, R, betas, samples=None, sample_offset=0, accepted=None,
+                     swaps=None, roundtrips=None, stream=None):
+    """numIterations tempered iterations in one launch (ehmc_hmc_run_tempered): systems of R adjacent particles at the
+    inverse temperatures betas (float64[R] device); samples is a [D*P, S] view of a (D, P, S) array."""
+    vq, vm, vb = dl(q), dl(mass), dl(betas)
+    vs, va, vw, vr = dl(samples), dl(accepted), dl(swaps), dl(roundtrips)
+    ta = TemperArgs(ctypes.sizeof(TemperArgs), int(R), vb.ptr, _p(vw), _p(vr))
+    check(ctx.lib.ehmc_hmc_run_tempered(ctx.handle, pot.handle, vq.ptr, vm.ptr, ctypes.byref(args), int(num_iterations),
+                                        ctypes.byref(ta), _p(vs), int(sample_offset), _p(va), stream))
 
 
 class Comm:

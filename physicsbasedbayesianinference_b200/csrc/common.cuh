@@ -83,6 +83,7 @@ __device__ __forceinline__ void philox4x32_10_multi(uint4 (&c)[NW], uint2 k) {
 }
 
 #define EHMC_UNIFORM_BLOCK 0xFFFFFFFFu
+#define EHMC_SWAP_BLOCK 0xFFFFFFFEu  // replica-exchange uniforms of the tempered run (k_small_run_tempered)
 
 struct PhiloxKey {
   uint2 key;
@@ -279,6 +280,17 @@ struct RunArgs {
   long long S;      // samples per particle in the arrays
   long long s0;     // first sample slot written by this launch
   int nIter;
+};
+
+// Replica exchange of the tempered run (k_small_run_tempered, ehmc_hmc_run_tempered): particle i is replica
+// r = i mod R of system i / R, R a power of two <= 32, so a system is R adjacent lanes of one warp and a swap is a
+// few register shuffles.  Slot r always runs at inverse temperature betas[r]; the STATES move between the lanes.
+struct TemperRun {
+  const double* betas;  // [R] device, betas[0] = 1 > betas[1] > ... > 0
+  int R;
+  int* swaps;           // [P] or null: accepted swaps of slot r with slot r + 1
+  int* roundtrips;      // [P / R] or null: states labelled "hottest" that reached slot 0
+  unsigned lanes;       // the warp's lanes that hold a particle (set by the kernel)
 };
 
 constexpr unsigned FLAG_BUGCOMPAT = 1u;

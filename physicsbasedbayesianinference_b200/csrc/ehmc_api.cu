@@ -517,6 +517,38 @@ extern "C" int ehmc_potential_create(ehmc_ctx* ctx, int family, const DLTensor* 
       h.centered = scalars[3] == 1.0;
       break;
     }
+    case EHMC_FAMILY_GAUSSIAN_MIXTURE: {
+      if (nparams != 3 || nscalars != 0) { rc = fail(EHMC_ERR_INVALID, "gaussian mixture: params = {weights[K], means[K,D], stds[K,D]}, no scalars"); break; }
+      MixtureState& s = p->mixture;
+      rc = fetch_param(params[0], "weights", 1, &a, &v);
+      if (rc) break;
+      s.K = (int)a.size();
+      if (s.K < 1) { rc = fail(EHMC_ERR_INVALID, "gaussian mixture: empty weights"); break; }
+      if (s.K > MIX_KMAX) { rc = fail(EHMC_ERR_UNSUPPORTED, "gaussian mixture: 1 <= K <= %d components (got %d)", MIX_KMAX, s.K); break; }
+      rc = fetch_param(params[1], "means", 2, &s.mu, &v);
+      if (rc) break;
+      p->D = (int)v.shape[1];
+      if (v.shape[0] != s.K || p->D < 1) { rc = fail(EHMC_ERR_INVALID, "gaussian mixture: means must be [K, D] with K = %d", s.K); break; }
+      rc = fetch_param(params[2], "stds", 2, &b, &v);
+      if (rc) break;
+      if (v.shape[0] != s.K || v.shape[1] != p->D) { rc = fail(EHMC_ERR_INVALID, "gaussian mixture: stds must be [K, D] like means"); break; }
+      if (p->D > 32) { rc = fail(EHMC_ERR_UNSUPPORTED, "family %d has no small-D kernel for D = %d", family, p->D); break; }
+      s.c.resize(s.K);
+      s.iv.resize(b.size());
+      for (int k = 0; k < s.K && rc == EHMC_OK; ++k) {
+        if (!(a[k] > 0 && std::isfinite(a[k]))) { rc = fail(EHMC_ERR_INVALID, "gaussian mixture: weights must be finite and > 0"); break; }
+        double c = std::log(a[k]);
+        for (int d = 0; d < p->D; ++d) {
+          const double sd = b[(size_t)k * p->D + d];
+          if (!(sd > 0 && std::isfinite(sd))) { rc = fail(EHMC_ERR_INVALID, "gaussian mixture: stds must be finite and > 0"); break; }
+          if (!std::isfinite(s.mu[(size_t)k * p->D + d])) { rc = fail(EHMC_ERR_INVALID, "gaussian mixture: means must be finite"); break; }
+          c -= std::log(sd);
+          s.iv[(size_t)k * p->D + d] = 1.0 / (sd * sd);
+        }
+        s.c[k] = c;
+      }
+      break;
+    }
     default:
       rc = fail(EHMC_ERR_UNSUPPORTED, "potential family %d is not built into this library", family);
   }
@@ -971,6 +1003,83 @@ extern "C" int ehmc_hmc_run(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* 
                                 sampleOffset, S, accepted, st);
   return hmc_run_typed<double>(ctx, pot, v, a, numIterations, samples_out ? &vs : nullptr, momenta_out ? &vm : nullptr,
                                sampleOffset, S, accepted, st);
+}
+
+// ---------------------------------------------------------------------------
+// getSamples' loop with replica exchange in one launch
+// ---------------------------------------------------------------------------
+// an optional device int32 counter vector of n entries
+static int parse_counts(const DLTensor* t, const char* name, long long n, int** out, const char* fn) {
+  *out = nullptr;
+  if (!t) return EHMC_OK;
+  View w;
+  TRY(parse(t, name, 1, &w));
+  if (w.host || w.bits != 32 || w.shape[0] != n) return fail(EHMC_ERR_INVALID, "%s: %s must be device int32[%lld]", fn, name, n);
+  *out = reinterpret_cast<int*>(w.data);
+  return EHMC_OK;
+}
+
+extern "C" int ehmc_hmc_run_tempered(ehmc_ctx* ctx, const ehmc_potential* pot, DLTensor* q, const DLTensor* mass,
+                                     const ehmc_hmc_args* a, int numIterations, const ehmc_temper_args* tp,
+                                     DLTensor* samples_out, int64_t sampleOffset, DLTensor* accepted_out, void* stream) {
+  if (ctx) ctx->ep_valid = false;  // q is about to change outside ehmc_hmc_iter
+  NvtxRange nvtx_range("ehmc_hmc_run_tempered");
+  const char* fn = "ehmc_hmc_run_tempered";
+  CallViews v;
+  TRY(common_checks(ctx, pot, q, mass, &v, fn));
+  TRY(check_hmc_args(HmcEntry::run, fn, a, nullptr, numIterations < 0 || sampleOffset < 0));
+  if (!tp || tp->struct_size < sizeof(ehmc_temper_args) || !tp->betas)
+    return fail(EHMC_ERR_INVALID, "%s: temper args (struct_size, betas) are required", fn);
+  const int R = tp->R;
+  if (R < 1 || R > 32 || (R & (R - 1)) != 0) return fail(EHMC_ERR_INVALID, "%s: R = %d must be 1, 2, 4, 8, 16 or 32", fn, R);
+  if (v.P % R != 0 || a->particleOffset % (uint64_t)R != 0)
+    return fail(EHMC_ERR_INVALID, "%s: P = %lld and particleOffset = %llu must be multiples of R = %d (a system never "
+                "straddles two shards)", fn, v.P, (unsigned long long)a->particleOffset, R);
+  View vb;
+  TRY(parse_float(tp->betas, "betas", 1, 64, &vb));
+  if (v.q.host || v.mass.host || vb.host) return fail(EHMC_ERR_INVALID, "%s: q, mass and betas must be device tensors", fn);
+  if (vb.shape[0] != R) return fail(EHMC_ERR_INVALID, "%s: betas must have R = %d entries", fn, R);
+  if (!has_small_kernel(pot)) return fail(EHMC_ERR_UNSUPPORTED, "family %d has no tempered multi-iteration kernel for D = %d", pot->family, pot->D);
+  View vs;
+  long long S = 0;
+  if (samples_out) {
+    TRY(parse_float(samples_out, "samples_out", 2, v.bits, &vs));
+    if (vs.host || vs.shape[0] != v.D * v.P || vs.ld != vs.shape[1])
+      return fail(EHMC_ERR_INVALID, "%s: samples_out must be a contiguous device [D*P, S] view of (D, P, S)", fn);
+    S = vs.shape[1];
+    if (sampleOffset + numIterations > S) return fail(EHMC_ERR_INVALID, "%s: sampleOffset + numIterations exceeds S = %lld", fn, S);
+  }
+  int* accepted = nullptr;
+  TemperRun X = {};
+  X.R = R;
+  X.betas = reinterpret_cast<const double*>(vb.data);
+  TRY(parse_counts(accepted_out, "accepted_out", v.P, &accepted, fn));
+  TRY(parse_counts(tp->swaps_out, "swaps_out", v.P, &X.swaps, fn));
+  TRY(parse_counts(tp->roundtrips_out, "roundtrips_out", v.P / R, &X.roundtrips, fn));
+  TRY(enter_device(ctx));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // the ladder, read back once: 1 = beta_0 > beta_1 > ... > beta_R-1 > 0
+  double hb[32];
+  CUDA_TRY(cudaMemcpyAsync(hb, vb.data, sizeof(double) * R, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  for (int r = 0; r < R; ++r)
+    if (!(r == 0 ? hb[0] == 1.0 : (hb[r] > 0.0 && hb[r] < hb[r - 1])))
+      return fail(EHMC_ERR_INVALID, "%s: betas must decrease strictly from betas[0] = 1 and stay > 0", fn);
+  if (v.P == 0 || numIterations == 0) return EHMC_OK;
+  auto run = [&](auto tag) -> int {
+    typedef decltype(tag) T;
+    IterArgs<T> A = hmc_args<T>(v, a);
+    A.p = nullptr;
+    RunArgs<T> Ra;
+    Ra.samples = samples_out ? reinterpret_cast<T*>(vs.data) : nullptr;
+    Ra.momenta = nullptr;
+    Ra.accepted = accepted;
+    Ra.S = S;
+    Ra.s0 = sampleOffset;
+    Ra.nIter = numIterations;
+    return run_small_tempered<T>(ctx, pot, A, a->integrator, Ra, X, st);
+  };
+  return v.bits == 32 ? run(float()) : run(double());
 }
 
 // ---------------------------------------------------------------------------

@@ -137,6 +137,13 @@ struct HierarchicalState {          // hierarchical normal model (make_hier), fl
   bool centered = false;
 };
 
+struct MixtureState {               // Gaussian mixture with diagonal covariances (make_mixture), float64 host tables
+  int K = 0;                        // components, 1 .. 8
+  std::vector<double> c;            // log w_k - sum_d log sigma_kd [K]
+  std::vector<double> mu;           // means [K][D]
+  std::vector<double> iv;           // 1 / sigma_kd^2 [K][D]
+};
+
 struct ehmc_potential {
   ehmc_ctx* ctx = nullptr;
   int family = 0;
@@ -149,6 +156,7 @@ struct ehmc_potential {
   LogisticState logistic;
   NBodyState nbody;
   HierarchicalState hier;
+  MixtureState mixture;
 };
 
 // peer-memory mailboxes of the fused ensemble run (comm.cu)
@@ -199,6 +207,10 @@ int launch_small(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int
 // getSamples' whole loop in one launch (small-D families, Philox draws)
 template <typename T>
 int run_small(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, const RunArgs<T>& R, cudaStream_t st);
+// the same loop with replica exchange between the R adjacent particles of each system (k_small_run_tempered)
+template <typename T>
+int run_small_tempered(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, const RunArgs<T>& R,
+                       const TemperRun& X, cudaStream_t st);
 // the adaptive ensemble run as one persistent launch (k_small_ens.cuh)
 template <typename T>
 struct EnsRunArgs;

@@ -85,6 +85,22 @@ static HierPot<T, DT, CENTERED> make_hier(const ehmc_potential* p) {
   return f;
 }
 
+template <typename T, int DT>
+static MixturePot<T, DT> make_mixture(const ehmc_potential* p) {
+  const MixtureState& s = p->mixture;
+  MixturePot<T, DT> f;
+  f.K = s.K;
+  for (int k = 0; k < MIX_KMAX; ++k) {
+    f.c[k] = k < s.K ? (T)s.c[k] : T(0);
+    for (int d = 0; d < DT; ++d) {
+      const bool on = k < s.K && d < p->D;
+      f.mu[k][d] = on ? (T)s.mu[(size_t)k * p->D + d] : T(0);
+      f.iv[k][d] = on ? (T)s.iv[(size_t)k * p->D + d] : T(0);
+    }
+  }
+  return f;
+}
+
 // The register-resident functor of p at its kernel width DT, the least of 2, 4, 8, 10, 16, 32 that holds p->D, handed
 // to f(std::integral_constant<int, DT>(), pot).  The dense family has one up to DT = 16 (above, k_dense), the
 // hierarchical model from DT = 4 (D = J + 2 >= 3).  Without one: EHMC_ERR_UNSUPPORTED, with the message "family F has
@@ -106,6 +122,7 @@ static int with_small_pot(const ehmc_potential* p, const char* what, F&& f) {
       case EHMC_FAMILY_HIERARCHICAL_NORMAL:
         if constexpr (DT >= 4) return p->hier.centered ? f(dt, make_hier<T, DT, true>(p)) : f(dt, make_hier<T, DT, false>(p));
         break;
+      case EHMC_FAMILY_GAUSSIAN_MIXTURE: return f(dt, make_mixture<T, DT>(p));
       default: break;
     }
     return none();
@@ -160,9 +177,27 @@ int run_small(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int in
     using Pot = std::decay_t<decltype(pot)>;
     const unsigned grid = (unsigned)std::max<long long>(1, (A.P + K1_THREADS - 1) / K1_THREADS);
     if (integ == INTEG_LEAPFROG)
-      k_small_run<T, DT, Pot, INTEG_LEAPFROG><<<grid, K1_THREADS, 0, st>>>(A, pot, R);
+      k_small_run<T, DT, Pot, INTEG_LEAPFROG><<<grid, K1_THREADS, 0, st>>>(A, pot, R, TemperRun());
     else
-      k_small_run<T, DT, Pot, INTEG_STORMER><<<grid, K1_THREADS, 0, st>>>(A, pot, R);
+      k_small_run<T, DT, Pot, INTEG_STORMER><<<grid, K1_THREADS, 0, st>>>(A, pot, R, TemperRun());
+    c->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return EHMC_OK;
+  });
+}
+
+template <typename T>
+int run_small_tempered(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<T>& A, int integ, const RunArgs<T>& R,
+                       const TemperRun& X, cudaStream_t st) {
+  return with_small_pot<T>(p, "tempered multi-iteration kernel", [&](auto dt, const auto& pot) -> int {
+    constexpr int DT = decltype(dt)::value;
+    using Pot = std::decay_t<decltype(pot)>;
+    // one thread per particle: the kernel's lane mask covers exactly the warp's particles
+    const unsigned grid = (unsigned)std::max<long long>(1, (A.P + K1_THREADS - 1) / K1_THREADS);
+    if (integ == INTEG_LEAPFROG)
+      k_small_run<T, DT, Pot, INTEG_LEAPFROG, true><<<grid, K1_THREADS, 0, st>>>(A, pot, R, X);
+    else
+      k_small_run<T, DT, Pot, INTEG_STORMER, true><<<grid, K1_THREADS, 0, st>>>(A, pot, R, X);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return EHMC_OK;

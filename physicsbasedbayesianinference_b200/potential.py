@@ -284,6 +284,43 @@ class HierarchicalNormalPotential(Potential):
         return dict(mu=mu, tau=tau, theta=theta)
 
 
+class GaussianMixturePotential(Potential):
+    """A mixture of K Gaussians with diagonal covariances -- a multimodal target:
+
+        U(q) = -log sum_k w_k prod_d N(q_d; means[k, d], stds[k, d]^2)
+
+    up to the constant (D/2) log 2 pi + log sum_k w_k (the weights need not sum to 1).  1 <= K <= 8, D <= 32.  An HMC
+    chain started in one mode of a well-separated mixture stays there; HMC.getSamplesTempered samples all of them."""
+
+    family = _lib.FAMILY_GAUSSIAN_MIXTURE
+
+    def __init__(self, weights, means, stds):
+        self.weights = np.atleast_1d(np.asarray(weights, dtype=np.float64)).copy()
+        self.means = np.atleast_2d(np.asarray(means, dtype=np.float64)).copy()
+        self.stds = np.atleast_2d(np.asarray(stds, dtype=np.float64)).copy()
+        K = self.weights.shape[0]
+        if self.weights.ndim != 1 or self.means.ndim != 2 or self.means.shape[0] != K or self.stds.shape != self.means.shape:
+            raise ValueError("weights must be (K,), means and stds (K, D)")
+        if not 1 <= K <= 8:
+            raise ValueError(f"the mixture kernels take 1 <= K <= 8 components (got {K})")
+        if not np.all((self.weights > 0) & np.isfinite(self.weights)):
+            raise ValueError("weights must be finite and > 0")
+        if not np.all((self.stds > 0) & np.isfinite(self.stds)):
+            raise ValueError("stds must be finite and > 0")
+        if not np.all(np.isfinite(self.means)):
+            raise ValueError("means must be finite")
+        super().__init__(self.means.shape[1])
+
+    def _params(self):
+        return [self.weights, self.means, self.stds]
+
+    def rescaled(self, scales):
+        # U'(q') = U(s q') - sum_d log s_d: the component densities at q' with means / s, stds / s are those at s q'
+        # times prod_d s_d, the same factor for every component (exact, so mass adaptation works)
+        s = np.asarray(scales, dtype=np.float64)
+        return GaussianMixturePotential(self.weights, self.means / s, self.stds / s)
+
+
 class NBodyPotential(Potential):
     """Every ensemble particle is a whole B-body system; coordinates are flattened
     component-major, d = c*B + b (the reference's own convention, src/potential.py:83-84).
