@@ -20,6 +20,8 @@ stores the old momentum instead.
 """
 from __future__ import annotations
 
+from types import SimpleNamespace
+
 import numpy as np
 
 from . import _lib
@@ -307,7 +309,7 @@ class HMC:
         fused=True runs the WHOLE call as one persistent cooperative launch (ehmc_hmc_run_ensemble, small-D
         families, Leapfrog, fixed numSteps): trajectory kernel, per-iteration statistics, their all-reduce across the
         ranks of `group` (stores into the peers' mailboxes over NVLink, inside the kernel) and the step-size update,
-        with the same one-iteration-stale schedule as the loop below -- no launch, no NCCL call and no host work per
+        with the same one-iteration-stale schedule as the host loop -- no launch, no NCCL call and no host work per
         iteration.  fused=None (default) picks it whenever it applies (statistics wanted, numSteps fixed: adapt=False
         or keepNumSteps=True); it needs CUDA IPC / peer access between the GPUs of `group`.
 
@@ -341,177 +343,139 @@ class HMC:
         (W^) as float64 CPU tensors, chainMean and chainVar (D, P local) device tensors in the ensemble's dtype (the
         original coordinates) and rhatDraws (N, the window's length) -- all None when the window is empty.
         """
+        o = SimpleNamespace(**locals())  # the options, handed on to the engines as given
+        del o.self
         if adaptLag not in (1, 2, 3, 4):
             raise ValueError("adaptLag must be 1, 2, 3 or 4")
-        if chainDiagnostics and not self._inRun:
-            phased = adaptMass or getattr(self, "massScale", None) is not None
-            self._check_chain_diagnostics(numIterations, adapt, adaptIterations, adaptLag, phased, deviceAdapt, group,
-                                          superchainSize)
-        if not self._inRun:
-            # everything below runs with _inRun set: non-finite acceptance ratios are rejected unless the driver was
-            # built with an explicit rejectNonFinite=False (see __init__)
-            self._inRun = True
-            try:
-                return self.run(numIterations, temperature, adapt=adapt, targetAccept=targetAccept,
-                                adaptIterations=adaptIterations, traceParticles=traceParticles, group=group,
-                                collectStats=collectStats, keepNumSteps=keepNumSteps, deviceAdapt=deviceAdapt,
-                                graph=graph, fused=fused, adaptLag=adaptLag, adaptMass=adaptMass,
-                                massWindows=massWindows, chainDiagnostics=chainDiagnostics,
-                                superchainSize=superchainSize)
-            finally:
-                self._inRun = False
-        if adaptMass or getattr(self, "massScale", None) is not None:
-            if adaptMass and not adapt:
-                raise ValueError("adaptMass=True needs adapt=True (the step size must follow the mass)")
-            return self._run_mass_adapt(numIterations, temperature, adaptMass=adaptMass, massWindows=massWindows,
-                                        adapt=adapt, targetAccept=targetAccept, adaptIterations=adaptIterations,
-                                        traceParticles=traceParticles, group=group, collectStats=collectStats,
-                                        keepNumSteps=keepNumSteps, deviceAdapt=deviceAdapt, graph=graph, fused=fused,
-                                        adaptLag=adaptLag, chainDiagnostics=chainDiagnostics,
-                                        superchainSize=superchainSize)
+        n = int(numIterations)
+        # the iterations whose statistics adapt the step size
+        nAdapt = 0 if not adapt else (n if adaptIterations is None else min(n, int(adaptIterations)))
+        phased = adaptMass or self.massScale is not None
+        if chainDiagnostics:
+            self._check_chain_diagnostics(o, n, nAdapt, phased)
+        if adaptMass and not adapt:
+            raise ValueError("adaptMass=True needs adapt=True (the step size must follow the mass)")
         if deviceAdapt and adaptLag != 1:
             raise ValueError("deviceAdapt=True implements adaptLag=1 only")
-        if fused is None:
-            fused = (collectStats and not deviceAdapt and self.ensemble.onDevice and self.method == "Leapfrog"
-                     and self._fused_loop_ok() and (keepNumSteps or not adapt) and numIterations > 0)
-        if fused:
-            return self._run_fused(numIterations, temperature, adapt, targetAccept, adaptIterations, traceParticles,
-                                   group, adaptLag, chainDiagnostics, superchainSize)
-        if deviceAdapt:
-            return self._run_device_adapt(numIterations, temperature, adapt, targetAccept, adaptIterations,
-                                          traceParticles, group, graph)
+        if not self.ensemble.onDevice:
+            raise TypeError("HMC.run needs a device-backed Ensemble (device='cuda'); use getSamples for host arrays")
+        if fused and (self.method != "Leapfrog" or not self._fused_loop_ok()):
+            raise ValueError("fused=True needs method='Leapfrog' and a small-D potential family (D <= 32)")
+        if deviceAdapt and not fused and graph and traceParticles:
+            raise ValueError("traceParticles needs graph=False (the trace slot changes every iteration)")
+        # everything below runs with _inRun set: non-finite acceptance ratios are rejected unless the driver was
+        # built with an explicit rejectNonFinite=False (see __init__)
+        self._inRun = True
+        try:
+            if phased:
+                return self._run_mass_adapt(o, n, nAdapt)
+            return self._run_engine(o, n, adapt, nAdapt, chainDiagnostics)
+        finally:
+            self._inRun = False
+
+    def _run_engine(self, o, n, adapt, nAdapt, chainDiagnostics):
+        """n iterations, the first nAdapt of them adapting the step size, on the engine that applies: a whole run()
+        call, or one phase of _run_mass_adapt.  n, adapt, nAdapt and chainDiagnostics are the call's or the phase's;
+        the other options come from o, run()'s arguments."""
         import torch
 
-        from .parallel import StatsReducer, StepSizeAdapter, unpack_stats
-
+        fused = o.fused
+        if fused is None:
+            fused = (o.collectStats and not o.deviceAdapt and self.method == "Leapfrog" and self._fused_loop_ok()
+                     and (o.keepNumSteps or not adapt) and n > 0)
         ens = self.ensemble
-        if not ens.onDevice:
-            raise TypeError("HMC.run needs a device-backed Ensemble (device='cuda'); use getSamples for host arrays")
-        D, P = ens.numDimensions, ens.numParticles
-        dev = ens.device
-        reducer = StatsReducer(group)
-        world = reducer.dist.get_world_size(group) if reducer.enabled else 1
-        Ptot = float(P)
-        if reducer.enabled:
-            t = torch.tensor([P], dtype=torch.float64, device=dev)
-            reducer.dist.all_reduce(t, group=group)
-            Ptot = float(t.item())
-        # without keepNumSteps the trajectory length is fixed and numSteps follows the step size: a step size above
-        # simulTime would mean numSteps = 0 (nothing moves, acceptance 1, the adapter runs away), so it is capped
-        adapter = (StepSizeAdapter(self.stepSize, targetAccept, maxStep=1e3 if keepNumSteps else min(1e3, self.simulTime))
-                   if adapt else None)
-        adaptIterations = numIterations if adaptIterations is None else adaptIterations
-        # adaptLag + 1 statistics slots (device vector + pinned host copy + "copy done" event).  Iteration k
-        # writes slot k % nslot; a side stream all-reduces it and copies it to the host behind an event,
-        # so the host only ever waits for iteration k - adaptLag while iteration k is already running:
-        # the GPU never idles on the statistics (they are consumed adaptLag iterations late).
-        nslot = adaptLag + 1
-        stats = [torch.zeros(2 * D + 3, dtype=torch.float64, device=dev) for _ in range(nslot)]
-        hosts = [torch.zeros(2 * D + 3, dtype=torch.float64).pin_memory() for _ in range(nslot)]
-        hosts_np = [h.numpy() for h in hosts]
-        done = [torch.cuda.Event() for _ in range(nslot)]
-        main = torch.cuda.current_stream(dev)
-        side = torch.cuda.Stream(dev)
-        out = dict(acceptRate=[], meanAcceptProb=[], meanH=[], stepSize=[], numSteps=[])
-        sum1 = np.zeros(D)
-        sum2 = np.zeros(D)
-        nstat = 0
-        trace = (torch.empty((D, traceParticles, numIterations), dtype=ens.dtype, device=dev)
-                 if traceParticles else None)
-        w0 = self._chain_window(numIterations, adapt, adaptIterations, adaptLag) if chainDiagnostics else numIterations
-        chains = self._chain_buffers(numIterations - w0)
-        ctx = _lib.Context.get(dev.index)
-        self.integrator.q = ens.q
-        pending = []  # slots whose statistics are in flight, oldest first (at most adaptLag of them)
-
-        def consume(slot, it):
-            nonlocal nstat
-            done[slot].synchronize()  # host wait: kernel `it` + all-reduce + D2H of 2D+3 doubles
-            h = hosts_np[slot]
-            acc_prob = float(h[1]) / Ptot
-            out["acceptRate"].append(float(h[0]) / Ptot)
-            out["meanAcceptProb"].append(acc_prob)
-            out["meanH"].append(float(h[2]) / Ptot)
-            sum1[:] += h[3:3 + D]
-            sum2[:] += h[3 + D:3 + 2 * D]
-            nstat += 1
-            if adapter is not None and it < adaptIterations:
-                self.stepSize = adapter.update(acc_prob)
-                self.integrator.stepSize = self.stepSize
-                if keepNumSteps:
-                    self.simulTime = self.integrator.finalTime = self.integrator.numSteps * self.stepSize
-                else:
-                    self.integrator.numSteps = max(1, int(self.simulTime / self.stepSize))  # src/integrator.py:51
-
-        for it in range(numIterations):
-            slot = it % nslot
-            out["stepSize"].append(self.stepSize)
-            out["numSteps"].append(self.integrator.numSteps)
-            self.step(temperature, stats=stats[slot] if collectStats else None, reuseEndpoint=it > 0)
-            if trace is not None:
-                trace[:, :, it] = ens.q[:, :traceParticles]
-            if chains is not None and it >= w0:
-                _lib.chain_moments_update(ctx, ens.q, chains[0], chains[1], it - w0 + 1, _lib.current_stream_ptr(ens.q))
-            if collectStats:
-                side.wait_stream(main)
-                with torch.cuda.stream(side):
-                    reducer.reduce(stats[slot])
-                    hosts[slot].copy_(stats[slot], non_blocking=True)
-                    done[slot].record(side)
-                if len(pending) >= adaptLag:
-                    consume(*pending.pop(0))  # statistics of iteration it - adaptLag
-                pending.append((slot, it))
-        for pd in pending:
-            consume(*pd)
-        main.wait_stream(side)
-        sum1 = torch.from_numpy(sum1)
-        sum2 = torch.from_numpy(sum2)
-        n = max(nstat, 1) * Ptot
-        mean = sum1 / n
-        out.update(mean=mean, var=sum2 / n - mean * mean, trace=trace, worldSize=world)
+        D = ens.numDimensions
+        world, Ptot, ranks = self._ensemble_size(o.group)
+        trace = (torch.empty((D, o.traceParticles, n), dtype=ens.dtype, device=ens.device)
+                 if o.traceParticles else None)
+        w0 = self._chain_window(n, nAdapt, o.adaptLag) if chainDiagnostics else n
+        chains = self._chain_buffers(n, w0)
+        # every engine fills hist (n, 4): acceptance rate, mean acceptance probability and mean H of the iterations
+        # whose statistics it collected (the first nstat), step size of every iteration; and mom: the sums of q_d and
+        # q_d^2 over those nstat iterations
+        if fused:
+            hist, numSteps, mom, nstat = self._run_fused(o, n, nAdapt, Ptot, trace, chains)
+        elif o.deviceAdapt:
+            hist, numSteps, mom, nstat = self._run_device_adapt(o, n, nAdapt, Ptot, trace)
+        else:
+            hist, numSteps, mom, nstat = self._run_host_loop(o, n, nAdapt, Ptot, trace, chains)
+        h, m = hist.cpu().numpy(), mom.cpu().numpy()
+        cnt = float(max(nstat, 1)) * Ptot
+        mean = torch.from_numpy(m[:D] / cnt)
+        out = dict(acceptRate=list(h[:nstat, 0]), meanAcceptProb=list(h[:nstat, 1]), meanH=list(h[:nstat, 2]),
+                   stepSize=list(h[:, 3]), numSteps=numSteps, mean=mean, var=torch.from_numpy(m[D:] / cnt) - mean * mean,
+                   trace=trace, worldSize=world)
+        if fused:
+            out["fused"] = True
         if chainDiagnostics:
-            out.update(self._chain_result(chains, numIterations - w0, superchainSize,
-                                          (group if group is not None else reducer.dist.group.WORLD)
-                                          if reducer.enabled else None))
+            out.update(self._chain_result(chains, n - w0, o.superchainSize, ranks))
         return out
 
+    def _ensemble_size(self, group):
+        """(world size, particles of all ranks, the ranks that combine the chain diagnostics or None) for `group`.
+        The total costs one NCCL all-reduce and a host read-back, so it is taken ONCE per (group, shard size) --
+        repeated in every call it put ~2 ms of collective + synchronisation in front of a fused launch that runs 200
+        iterations in 7 ms at 8 GPUs."""
+        import torch.distributed as dist
+
+        P = self.ensemble.numParticles
+        if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+            return 1, float(P), None
+        key = (id(group), P)
+        cache = self.__dict__.setdefault("_ptotCache", {})
+        if key not in cache:
+            import torch
+
+            t = torch.tensor([P], dtype=torch.float64, device=self.ensemble.device)
+            dist.all_reduce(t, group=group)
+            cache[key] = float(t.item())
+        return dist.get_world_size(group), cache[key], group if group is not None else dist.group.WORLD
+
+    def _keep_step_size(self, stepSize):
+        """Takes over the step size an engine with a fixed number of leapfrog steps ended with."""
+        self.stepSize = float(stepSize)
+        self.integrator.stepSize = self.stepSize
+        self.simulTime = self.integrator.finalTime = self.integrator.numSteps * self.stepSize
+
     # ------------------------------------------------------------------------------------
-    def _chain_window(self, n, adapt, adaptIterations, adaptLag, phased=False):
-        """First iteration of a run() call whose positions enter the chain diagnostics: the first one whose step size
-        is final (the statistics of iteration k set the step size of iteration k + 1 + adaptLag); with mass
-        adaptation (phased) the first one after the warm-up phases."""
-        nAdapt = 0 if not adapt else (n if adaptIterations is None else min(n, int(adaptIterations)))
+    def _chain_window(self, n, nAdapt, adaptLag, phased=False):
+        """First iteration of a run() call of n iterations, nAdapt of them adapting the step size, whose positions
+        enter the chain diagnostics: the first one whose step size is final (the statistics of iteration k set the
+        step size of iteration k + 1 + adaptLag); with mass adaptation (phased) the first one after the warm-up
+        phases."""
         if nAdapt == 0:
             return 0
         return nAdapt if phased else min(n, nAdapt + adaptLag)
 
-    def _check_chain_diagnostics(self, n, adapt, adaptIterations, adaptLag, phased, deviceAdapt, group, M):
+    def _check_chain_diagnostics(self, o, n, nAdapt, phased):
         """run(chainDiagnostics=True)'s refusals, raised before any device work."""
-        if deviceAdapt:
+        if o.deviceAdapt:
             raise ValueError("chainDiagnostics=True needs deviceAdapt=False (a graph replay would bake in the draw count)")
         ens = self.ensemble
-        M = int(M)
+        M = int(o.superchainSize)
         if M < 1 or ens.numParticles % M or ens.particleOffset % M:
             raise ValueError(f"superchainSize {M} must be >= 1 and divide numParticles ({ens.numParticles}) and "
                              f"particleOffset ({ens.particleOffset}): a superchain must not straddle two shards")
-        N = int(n) - self._chain_window(int(n), adapt, adaptIterations, adaptLag, phased)
+        N = n - self._chain_window(n, nAdapt, o.adaptLag, phased)
         if N == 1 and M == 1:
             raise ValueError("nested R-hat needs superchainSize > 1 or a window of more than one iteration")
         import torch.distributed as dist
 
-        single = not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1
+        single = not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(o.group) == 1
         if single and ens.numParticles // M < 2:
             raise ValueError(f"nested R-hat needs at least 2 superchains, got {ens.numParticles // M}")
 
-    def _chain_buffers(self, N):
-        """(mean, m2) accumulators [D, P] of the chain diagnostics (no initialisation: draw 1 writes them), or None."""
-        if N <= 0:
+    def _chain_buffers(self, n, w0):
+        """(mean, m2, w0): the accumulators [D, P] of the chain diagnostics over iterations w0 .. n - 1 of a call (no
+        initialisation: draw 1 writes them), or None when that window is empty."""
+        if w0 >= n:
             return None
         import torch
 
         ens = self.ensemble
-        return tuple(torch.empty((ens.numDimensions, ens.numParticles), dtype=ens.dtype, device=ens.device)
-                     for _ in range(2))
+        mean, m2 = (torch.empty((ens.numDimensions, ens.numParticles), dtype=ens.dtype, device=ens.device)
+                    for _ in range(2))
+        return mean, m2, w0
 
     def _chain_result(self, chains, N, M, group):
         """The result keys of run(chainDiagnostics=True) from the accumulators of N draws (group: combine the ranks)."""
@@ -519,40 +483,34 @@ class HMC:
             return dict(rhat=None, rhatBetween=None, rhatWithin=None, chainMean=None, chainVar=None, rhatDraws=None)
         from .diagnostics import nested_rhat_from_moments
 
-        mean, m2 = chains
+        mean, m2, _ = chains
         var = m2 / (N - 1) if N > 1 else m2.zero_()
         rhat, between, within = nested_rhat_from_moments(mean, var, N, M, group=group)
         return dict(rhat=rhat.cpu(), rhatBetween=between.cpu(), rhatWithin=within.cpu(), chainMean=mean, chainVar=var,
                     rhatDraws=N)
 
 
-    def _run_mass_adapt(self, numIterations, temperature, *, adaptMass, massWindows, adapt, adaptIterations,
-                        traceParticles, chainDiagnostics=False, superchainSize=1, **kw):
+    def _run_mass_adapt(self, o, n, nAdapt):
         """run() in rescaled coordinates (see run(adaptMass=True)).
 
         The call is cut into phases -- parallel.mass_windows during the warm-up, one phase for the rest -- and every
-        phase is an ordinary run() (one fused launch where that applies) on the ensemble in the coordinates
-        q' = q / massScale with the potential Potential.rescaled(massScale).  A window's var (returned by its run(),
-        all-reduced over ranks, pooled over the window's iterations) is the variance in the CURRENT coordinates, so
-        the scales compose multiplicatively.  Step-size adaptation restarts its gain sequence in every phase (each
-        run() call starts at k = 1), which lets the step size follow a new mass quickly, as Stan does."""
+        phase runs on its engine (one fused launch where that applies) on the ensemble in the coordinates
+        q' = q / massScale with the potential Potential.rescaled(massScale).  A window's var (all-reduced over ranks,
+        pooled over the window's iterations) is the variance in the CURRENT coordinates, so the scales compose
+        multiplicatively.  Step-size adaptation restarts its gain sequence in every phase (each phase starts at
+        k = 1), which lets the step size follow a new mass quickly, as Stan does."""
         import torch
 
         from .parallel import MassAdapter, mass_windows
 
         ens = self.ensemble
-        if not ens.onDevice:
-            raise TypeError("HMC.run needs a device-backed Ensemble (device='cuda')")
         D = ens.numDimensions
-        n = int(numIterations)
-        nAdapt = 0 if not adapt else (n if adaptIterations is None else min(n, int(adaptIterations)))
-        phases = mass_windows(nAdapt, massWindows) if adaptMass else ([(nAdapt, False)] if nAdapt else [])
+        phases = mass_windows(nAdapt, o.massWindows) if o.adaptMass else ([(nAdapt, False)] if nAdapt else [])
         phases = [(k, upd, True) for k, upd in phases]
         if n - nAdapt > 0:
             phases.append((n - nAdapt, False, False))
         base = self.potential
-        scale = np.ones(D) if getattr(self, "massScale", None) is None else np.asarray(self.massScale, dtype=np.float64)
-        self.massScale = None  # (the phases below are plain run() calls)
+        scale = np.ones(D) if self.massScale is None else np.asarray(self.massScale, dtype=np.float64)
         adapter = MassAdapter(D)
 
         def enter(s):
@@ -568,9 +526,7 @@ class HMC:
         try:
             for k, updateMass, adaptive in phases:
                 # the chain diagnostics' window is the phase after the warm-up (its step size and mass are final)
-                r = self.run(k, temperature, adapt=adaptive, adaptIterations=k if adaptive else 0,
-                             traceParticles=traceParticles, chainDiagnostics=chainDiagnostics and not adaptive,
-                             superchainSize=superchainSize, **kw)
+                r = self._run_engine(o, k, adaptive, k if adaptive else 0, o.chainDiagnostics and not adaptive)
                 for key in ("acceptRate", "meanAcceptProb", "meanH", "stepSize", "numSteps"):
                     out[key].extend(r[key])
                 out["massScale"].extend([scale.copy()] * k)
@@ -582,7 +538,8 @@ class HMC:
                                     chainMean=r["chainMean"] * st, chainVar=r["chainVar"] * (st * st),
                                     rhatDraws=r["rhatDraws"])
                 if updateMass:
-                    cnt = float(k) * float(r.get("numParticlesTotal", ens.numParticles * r.get("worldSize", 1)))
+                    # local particles x world: not the ensemble's size when the shards are uneven
+                    cnt = float(k) * float(ens.numParticles * r["worldSize"])
                     s_new = base.projectScales(adapter.scales(r["mean"].numpy(), r["var"].numpy(), cnt))
                     ens.q.div_(torch.as_tensor(s_new, dtype=ens.q.dtype, device=ens.device)[:, None])
                     scale = scale * s_new
@@ -593,16 +550,92 @@ class HMC:
         self.massScale = None if np.all(scale == 1.0) else scale
         if r is not None:
             sc = torch.from_numpy(scale)
-            out.update(mean=r["mean"] * sc, var=r["var"] * sc * sc, worldSize=r.get("worldSize", 1),
+            out.update(mean=r["mean"] * sc, var=r["var"] * sc * sc, worldSize=r["worldSize"],
                        fused=r.get("fused", False))
         out["trace"] = torch.cat(traces, dim=2) if traces else None
-        if chainDiagnostics:
+        if o.chainDiagnostics:
             out.update(chainOut)
         return out
 
-    def _run_fused(self, numIterations, temperature, adapt, targetAccept, adaptIterations, traceParticles, group,
-                   adaptLag=1, chainDiagnostics=False, superchainSize=1):
-        """HMC.run as ONE launch: see run(fused=True) and csrc/k_small_ens.cuh."""
+    def _run_host_loop(self, o, n, nAdapt, Ptot, trace, chains):
+        """One ehmc_hmc_iter launch per iteration; returns (hist, numSteps, mom, nstat) (see _run_engine)."""
+        import torch
+
+        from .parallel import StatsReducer, StepSizeAdapter
+
+        ens = self.ensemble
+        D, dev = ens.numDimensions, ens.device
+        # the options the loop reads every iteration, as locals
+        temperature, collectStats, keepNumSteps, adaptLag = o.temperature, o.collectStats, o.keepNumSteps, o.adaptLag
+        ntrace = o.traceParticles
+        reducer = StatsReducer(o.group)
+        # without keepNumSteps the trajectory length is fixed and numSteps follows the step size: a step size above
+        # simulTime would mean numSteps = 0 (nothing moves, acceptance 1, the adapter runs away), so it is capped
+        adapter = (StepSizeAdapter(self.stepSize, o.targetAccept, maxStep=1e3 if keepNumSteps else min(1e3, self.simulTime))
+                   if nAdapt else None)
+        # adaptLag + 1 statistics slots (device vector + pinned host copy + "copy done" event).  Iteration k
+        # writes slot k % nslot; a side stream all-reduces it and copies it to the host behind an event,
+        # so the host only ever waits for iteration k - adaptLag while iteration k is already running:
+        # the GPU never idles on the statistics (they are consumed adaptLag iterations late).
+        nslot = adaptLag + 1
+        stats = [torch.zeros(2 * D + 3, dtype=torch.float64, device=dev) for _ in range(nslot)]
+        hosts = [torch.zeros(2 * D + 3, dtype=torch.float64).pin_memory() for _ in range(nslot)]
+        hosts_np = [h.numpy() for h in hosts]
+        done = [torch.cuda.Event() for _ in range(nslot)]
+        main = torch.cuda.current_stream(dev)
+        side = torch.cuda.Stream(dev)
+        hist = torch.zeros((n, 4), dtype=torch.float64)
+        mom = torch.zeros(2 * D, dtype=torch.float64)
+        hist_np, mom_np = hist.numpy(), mom.numpy()
+        stepSizes, numSteps = [], []
+        nstat = 0
+        w0 = n if chains is None else chains[2]
+        ctx = _lib.Context.get(dev.index)
+        self.integrator.q = ens.q
+        pending = []  # slots whose statistics are in flight, oldest first (at most adaptLag of them)
+
+        def consume(slot, it):
+            nonlocal nstat
+            done[slot].synchronize()  # host wait: kernel `it` + all-reduce + D2H of 2D+3 doubles
+            h = hosts_np[slot]
+            hist_np[it, :3] = h[:3] / Ptot
+            mom_np[:] += h[3:]
+            nstat += 1
+            if adapter is not None and it < nAdapt:
+                self.stepSize = adapter.update(float(hist_np[it, 1]))
+                self.integrator.stepSize = self.stepSize
+                if keepNumSteps:
+                    self.simulTime = self.integrator.finalTime = self.integrator.numSteps * self.stepSize
+                else:
+                    self.integrator.numSteps = max(1, int(self.simulTime / self.stepSize))  # src/integrator.py:51
+
+        for it in range(n):
+            slot = it % nslot
+            stepSizes.append(self.stepSize)
+            numSteps.append(self.integrator.numSteps)
+            self.step(temperature, stats=stats[slot] if collectStats else None, reuseEndpoint=it > 0)
+            if trace is not None:
+                trace[:, :, it] = ens.q[:, :ntrace]
+            if it >= w0:
+                _lib.chain_moments_update(ctx, ens.q, chains[0], chains[1], it - w0 + 1, _lib.current_stream_ptr(ens.q))
+            if collectStats:
+                side.wait_stream(main)
+                with torch.cuda.stream(side):
+                    reducer.reduce(stats[slot])
+                    hosts[slot].copy_(stats[slot], non_blocking=True)
+                    done[slot].record(side)
+                if len(pending) >= adaptLag:
+                    consume(*pending.pop(0))  # statistics of iteration it - adaptLag
+                pending.append((slot, it))
+        for pd in pending:
+            consume(*pd)
+        main.wait_stream(side)
+        hist_np[:, 3] = stepSizes
+        return hist, numSteps, mom, nstat
+
+    def _run_fused(self, o, n, nAdapt, Ptot, trace, chains):
+        """HMC.run as ONE launch: see run(fused=True) and csrc/k_small_ens.cuh; returns (hist, numSteps, mom, nstat)
+        (see _run_engine)."""
         import math
 
         import torch
@@ -610,123 +643,66 @@ class HMC:
         from .parallel import ensemble_comm
 
         ens = self.ensemble
-        if not ens.onDevice:
-            raise TypeError("HMC.run needs a device-backed Ensemble (device='cuda')")
-        if self.method != "Leapfrog" or not self._fused_loop_ok():
-            raise ValueError("fused=True needs method='Leapfrog' and a small-D potential family (D <= 32)")
-        D, P, dev = ens.numDimensions, ens.numParticles, ens.device
+        D, dev = ens.numDimensions, ens.device
         ctx = _lib.Context.get(dev.index)
-        comm = ensemble_comm(ctx, group, dev)
-        world, Ptot = 1, float(P)
-        if comm is not None:
-            import torch.distributed as dist
-
-            world = dist.get_world_size(group)
-            # the ensemble size over all ranks: one NCCL all-reduce and a host read-back, ONCE per (group, shard
-            # size) -- repeated in every call it put ~2 ms of collective + synchronisation in front of a launch
-            # that runs 200 iterations in 7 ms at 8 GPUs
-            key = (id(group), P)
-            cache = self.__dict__.setdefault("_ptotCache", {})
-            if key not in cache:
-                t = torch.tensor([P], dtype=torch.float64, device=dev)
-                dist.all_reduce(t, group=group)
-                cache[key] = float(t.item())
-            Ptot = cache[key]
-        n = int(numIterations)
-        adaptRows = 0 if not adapt else (n if adaptIterations is None else min(n, int(adaptIterations)))
         state = torch.tensor([self.stepSize, math.log(self.stepSize), 0.0, 0.0], dtype=torch.float64, device=dev)
         hist = torch.zeros((n, 4), dtype=torch.float64, device=dev)
         mom = torch.zeros(2 * D, dtype=torch.float64, device=dev)
-        ntrace = int(traceParticles)
-        trace = torch.empty((D, ntrace, n), dtype=ens.dtype, device=dev) if ntrace else None
-        w0 = self._chain_window(n, adapt, adaptIterations, adaptLag) if chainDiagnostics else n
-        chains = self._chain_buffers(n - w0)
-        self.integrator.q = ens.q
-        numSteps = self.integrator.numSteps
-        q = ens.q
-        bits = q.element_size() * 8
-        _lib.hmc_run_ensemble(ctx, self.potential.handle(bits, ctx), q, self.integrator.mass, self._args(temperature), n,
-                              _lib.make_adapt_args(Ptot, adaptRows, target=targetAccept, lag=adaptLag), state, comm=comm,
-                              history=hist,
-                              moments=mom, trace=None if trace is None else trace.view(D * ntrace, n),
-                              trace_particles=ntrace, stream=_lib.current_stream_ptr(q),
-                              chains=None if chains is None else (chains[0], chains[1], w0))
+        ntrace = 0 if trace is None else trace.shape[1]
+        self.integrator.q = q = ens.q
+        _lib.hmc_run_ensemble(ctx, self.potential.handle(q.element_size() * 8, ctx), q, self.integrator.mass,
+                              self._args(o.temperature), n,
+                              _lib.make_adapt_args(Ptot, nAdapt, target=o.targetAccept, lag=o.adaptLag), state,
+                              comm=ensemble_comm(ctx, o.group, dev), history=hist, moments=mom,
+                              trace=None if trace is None else trace.view(D * ntrace, n), trace_particles=ntrace,
+                              stream=_lib.current_stream_ptr(q), chains=chains)
         self.iteration += n
-        st = state.cpu().numpy()  # synchronises
-        self.stepSize = float(st[0])
-        self.integrator.stepSize = self.stepSize
-        self.simulTime = self.integrator.finalTime = numSteps * self.stepSize
-        h = hist.cpu().numpy()
-        m = mom.cpu().numpy()
-        cnt = float(max(n, 1)) * Ptot
-        mean = torch.from_numpy(m[:D] / cnt)
-        out = dict(acceptRate=list(h[:, 0]), meanAcceptProb=list(h[:, 1]), meanH=list(h[:, 2]), stepSize=list(h[:, 3]),
-                   numSteps=[numSteps] * n, mean=mean, var=torch.from_numpy(m[D:] / cnt) - mean * mean,
-                   trace=trace, worldSize=world, fused=True)
-        if chainDiagnostics:
-            ranks = None
-            if comm is not None:
-                ranks = group if group is not None else dist.group.WORLD
-            out.update(self._chain_result(chains, n - w0, superchainSize, ranks))
-        return out
+        self._keep_step_size(state[0].item())  # synchronises
+        return hist, [self.integrator.numSteps] * n, mom, n
 
-    def _run_device_adapt(self, numIterations, temperature, adapt, targetAccept, adaptIterations, traceParticles,
-                          group, graph, graphIterations=10):
+    def _run_device_adapt(self, o, n, nAdapt, Ptot, trace, graphIterations=10):
         """Two control blocks used alternately: iteration k runs with block k & 1; on a side stream the
         statistics of iteration k are all-reduced and ehmc_adapt_step writes the block iteration k + 2
         will read, taking the adaptation state from the other block.  Iteration k + 1 therefore only
         waits for the update computed from iteration k - 1 (the one-iteration-stale pipeline of the
-        host-side loop) and the all-reduce overlaps iteration k + 1."""
+        host-side loop) and the all-reduce overlaps iteration k + 1.  Returns (hist, numSteps, mom, nstat)
+        (see _run_engine)."""
         import torch
 
         from .parallel import StatsReducer
 
         ens = self.ensemble
-        if not ens.onDevice:
-            raise TypeError("HMC.run needs a device-backed Ensemble (device='cuda')")
-        if graph and traceParticles:
-            raise ValueError("traceParticles needs graph=False (the trace slot changes every iteration)")
-        D, P, dev = ens.numDimensions, ens.numParticles, ens.device
-        reducer = StatsReducer(group)
-        world = reducer.dist.get_world_size(group) if reducer.enabled else 1
-        Ptot = float(P)
-        if reducer.enabled:
-            t = torch.tensor([P], dtype=torch.float64, device=dev)
-            reducer.dist.all_reduce(t, group=group)
-            Ptot = float(t.item())
+        D, dev = ens.numDimensions, ens.device
+        reducer = StatsReducer(o.group)
         ctx = _lib.Context.get(dev.index)
-        adaptRows = 0 if not adapt else (numIterations if adaptIterations is None else adaptIterations)
         it0 = self.iteration
         blocks = [_lib.dynamic_to_device(self.stepSize, it0 + b, dev, row=b) for b in range(2)]
         stats = [torch.zeros(2 * D + 3, dtype=torch.float64, device=dev) for _ in range(2)]
-        hist = torch.zeros((numIterations, 4), dtype=torch.float64, device=dev)
+        hist = torch.zeros((n, 4), dtype=torch.float64, device=dev)
         mom = torch.zeros(2 * D, dtype=torch.float64, device=dev)
-        trace = (torch.empty((D, traceParticles, numIterations), dtype=ens.dtype, device=dev)
-                 if traceParticles else None)
         self.integrator.q = ens.q
-        numSteps = self.integrator.numSteps
         # high priority: the 1-block update kernel and the small all-reduce must not queue behind the
         # thousands of CTAs of the running trajectory kernel
         side = torch.cuda.Stream(dev, priority=-1)
 
-        def enqueue(k0, n, main):
-            """Iterations k0 .. k0 + n - 1 on `main` + `side`; joins the two streams at the end."""
+        def enqueue(k0, count, main):
+            """Iterations k0 .. k0 + count - 1 on `main` + `side`; joins the two streams at the end."""
             ran = [None, None]      # per parity: event "kernel + statistics of this parity done"
             adapted = [None, None]  # per parity: event "block of this parity rewritten"
-            for k in range(k0, k0 + n):
+            for k in range(k0, k0 + count):
                 b = k & 1
                 if adapted[b] is not None:
                     main.wait_event(adapted[b])  # block b and stats[b] are free / up to date
-                self.step(temperature, stats=stats[b], dynamic=blocks[b].data_ptr())
+                self.step(o.temperature, stats=stats[b], dynamic=blocks[b].data_ptr())
                 if trace is not None:
-                    trace[:, :, k] = ens.q[:, :traceParticles]
+                    trace[:, :, k] = ens.q[:, :o.traceParticles]
                 ran[b] = torch.cuda.Event()
                 ran[b].record(main)
                 with torch.cuda.stream(side):
                     side.wait_event(ran[b])
                     reducer.reduce(stats[b])
-                    _lib.adapt_step(ctx, stats[b], Ptot, blocks[b].data_ptr(), target=targetAccept,
-                                    adapt_rows=adaptRows, state_ptr=blocks[1 - b].data_ptr(), stride=2, history=hist,
+                    _lib.adapt_step(ctx, stats[b], Ptot, blocks[b].data_ptr(), target=o.targetAccept,
+                                    adapt_rows=nAdapt, state_ptr=blocks[1 - b].data_ptr(), stride=2, history=hist,
                                     moments=mom, stream=_lib.current_stream_ptr(stats[b]))
                     adapted[b] = torch.cuda.Event()
                     adapted[b].record(side)
@@ -735,9 +711,9 @@ class HMC:
         main = torch.cuda.current_stream(dev)
         side.wait_stream(main)
         G = int(graphIterations) & ~1
-        if graph and G >= 2 and numIterations >= 2 + G:
+        if o.graph and G >= 2 and n >= 2 + G:
             # eager head: sizes the library's scratch buffers outside the capture and leaves a multiple of G
-            head = 2 + (numIterations - 2) % G
+            head = 2 + (n - 2) % G
             enqueue(0, head, main)
             g = torch.cuda.CUDAGraph()
             cap = torch.cuda.Stream(dev)
@@ -748,22 +724,13 @@ class HMC:
                     enqueue(head, G, cap)
             main.wait_stream(cap)
             self.iteration = it0 + head  # the captured calls advanced the host counter; it is reset below anyway
-            for _ in range((numIterations - head) // G):
+            for _ in range((n - head) // G):
                 g.replay()
         else:
-            enqueue(0, numIterations, main)
-        self.iteration = it0 + numIterations
-        newest = _lib.dynamic_from_device(blocks[(numIterations - 1) & 1 if numIterations else 0])  # synchronises
-        self.stepSize = float(newest.stepSize)
-        self.integrator.stepSize = self.stepSize
-        self.simulTime = self.integrator.finalTime = numSteps * self.stepSize
-        h = hist.cpu().numpy()
-        m = mom.cpu().numpy()
-        n = float(max(numIterations, 1)) * Ptot
-        mean = torch.from_numpy(m[:D] / n)
-        return dict(acceptRate=list(h[:, 0]), meanAcceptProb=list(h[:, 1]), meanH=list(h[:, 2]), stepSize=list(h[:, 3]),
-                    numSteps=[numSteps] * numIterations, mean=mean, var=torch.from_numpy(m[D:] / n) - mean * mean,
-                    trace=trace, worldSize=world)
+            enqueue(0, n, main)
+        self.iteration = it0 + n
+        self._keep_step_size(_lib.dynamic_from_device(blocks[(n - 1) & 1 if n else 0]).stepSize)  # synchronises
+        return hist, [self.integrator.numSteps] * n, mom, n
 
 
 class GaussianDensity:
