@@ -68,6 +68,10 @@ static int launch_tc3_c8(ehmc_ctx* c, const ehmc_potential* p, const IterArgs<fl
     CUDA_TRY(cudaMemsetAsync(c->overflow.ptr, 0, sizeof(unsigned), st));
   }
   pa.overflow = static_cast<unsigned*>(c->overflow.ptr);
+  // h == 0 is the fixed point of both integrators (q, p, H unchanged, accepted); the kernel runs it as Leapfrog with
+  // L = 0 (see k_dense_tc3).  A device-resident step size (A.dyn) is not known here; ehmc_adapt_step keeps it in
+  // [minStep, maxStep] with minStep > 0.
+  if (A.dyn == nullptr && A.h == 0.f) integ = INTEG_LEAPFROG;
   // persistent: one CTA per SM (the CTA takes the whole TMEM), tiles dealt in contiguous ranges
   const long long ntiles = (A.P + TC_M - 1) / TC_M;
   const unsigned grid = (unsigned)std::min<long long>(c->prop.multiProcessorCount, ntiles);

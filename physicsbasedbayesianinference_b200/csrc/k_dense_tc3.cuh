@@ -232,7 +232,10 @@ __global__ void __launch_bounds__(TC3_THREADS, 1) k_dense_tc3(const IterArgs<flo
   const uint32_t mma_d = tmem_base + (uint32_t)(grp * 256);
   const uint32_t mma_hi = mma_d + (uint32_t)S::HI_COL, mma_lo = mma_d + (uint32_t)S::LO_COL;
 
-  // h == 0 is a fixed point (q, p, H unchanged): run it as L = 0 so that 1 / h never appears
+  // h == 0 is a fixed point (q, p, H unchanged, accepted): run it as L = 0 so that 1 / h never appears.  That holds
+  // for Leapfrog only: Stormer-Verlet's start-up evaluation would still kick and drift a full step of the stand-in
+  // h = 1, so launch_tc3_c8 runs Stormer-Verlet at h == 0 as Leapfrog.  (k_dense follows the reference there instead:
+  // q unchanged, p = (q - q) / 0 = NaN, accepted unless EHMC_FLAG_REJECT_NONFINITE.)
   const int L = A.h == 0.f ? 0 : A.L;
   const float h = A.h == 0.f ? 1.f : A.h;
   const long long ntiles = (A.P + TC_M - 1) / TC_M;
